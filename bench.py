@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- candidate-path segment evaluations / s (cost + collision) on an 8192^2 multi-layer raster.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2], SURVEY.md 8d "C3"): synthetic 8192^2 raster with L = 3 float32 cost layers
@@ -38,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (no __pycache__ of the modules it imports)
 
 RASTER = 8192
 WP = 64                 # waypoints per path (N = 62 free + start + goal)
@@ -244,9 +245,13 @@ def run_reference(args):
     Z = host_paths(per_step, 2000, n)                # rank 0's batch of the GPU arm (same seed)
     times = []
     for s in range(args.warmup + args.steps):
-        rate, dt, th, _ = cpu_c_rate(layers, occ, geo, Z, cores)
+        rate, dt, th, res = cpu_c_rate(layers, occ, geo, Z, cores)
         if s >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        c, k, _ = res
+        i = int(np.argmin(c))
+        dump_outputs(args.dump_outputs, torch.from_numpy(c), torch.from_numpy(k), float(c[i]), i)
     T = float(np.sum(times))
     value = per_step * (WP - 1) * args.steps / T
     line = {'impl': 'reference', 'metric': METRIC, 'value': value, 'unit': 'segment-evals/s', 'n_gpus': args.gpus,
@@ -308,6 +313,28 @@ def workload_config(args):
             'raster': args.raster, 'layers': 3, 'waypoints': WP, 'paths_per_gpu_per_step': args.paths,
             'samples_per_cell': SPC, 'sharding': 'paths sharded contiguously over ranks, map replicated',
             'l2': 'inputs larger than L2 (texels 1 GiB, paths 1 KiB each); no explicit flush'}
+
+
+DUMP_MAX_PATHS = 1 << 22         # 2 x 16 MiB of float32 per-path outputs at most; larger batches are sampled
+DUMP_SEED = 20260104
+
+
+def dump_outputs(out_dir, cost, col, best_cost, best_idx):
+    """--dump-outputs: what the caller of the timed step receives (RasterMap.score_paths_best), as .npy files, so that two
+    builds can be compared output for output.  The inputs are seeded, so the same arguments give the same inputs.
+    cost.npy (B,) f32, collide.npy (B,) f32 0 / 1, best_cost.npy / best_index.npy (1,) f64 (the decoded best key).
+    Batches of more than DUMP_MAX_PATHS paths keep a fixed seeded sample of the rows, listed in path_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    c = cost.cpu().numpy().astype(np.float32)
+    k = col.cpu().numpy().astype(np.float32)
+    if c.size > DUMP_MAX_PATHS:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(c.size, DUMP_MAX_PATHS, replace=False))
+        c, k = c[idx], k[idx]
+        np.save(os.path.join(out_dir, 'path_index.npy'), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, 'cost.npy'), c)
+    np.save(os.path.join(out_dir, 'collide.npy'), k)
+    np.save(os.path.join(out_dir, 'best_cost.npy'), np.array([best_cost], dtype=np.float64))
+    np.save(os.path.join(out_dir, 'best_index.npy'), np.array([best_idx], dtype=np.float64))
 
 
 def kernel_profile(kname, B, n):
@@ -415,6 +442,8 @@ def run_ours(args):
     assert int(eng.get_stat('score_kernel_count')) == args.steps
     eng.set_option('time_kernels', 0)
     best_cost, best_idx = udist.decode_key(int(key.item()))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, cost, col, best_cost, best_idx)
     variant = int(os.environ.get('UAM_INT_VARIANT', '-1'))
     combine = int(os.environ.get('UAM_COMBINE_LAYERS', '1'))
     quad = {0: '4', 1: '8', 2: '1'}[combine]         # texel form sampled by the large-batch pipelines (8: sign-packed quads)
@@ -652,7 +681,12 @@ def main():
     ap.add_argument('--c5-queries', type=int, default=16, help='C5: queries per GPU, 1 altitude band')
     ap.add_argument('--c5-queries-bands', type=int, default=4, help='C5: full sweeps per GPU, 8 altitude bands')
     ap.add_argument('--c5-routes', type=int, default=128, help='C5: start/goal queries per GPU (128 x 8 GPUs = the 1024 of BASELINE config 5)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the outputs of the last one (rank 0: per-path cost and collision flag, '
+                         'best cost and index) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     if args.impl == 'reference':
         run_reference(args)

@@ -1,7 +1,7 @@
 """path_generation/gpu_backend.py -- the file a maintainer of nomaporon/uam_path_planning adds to bind libuam_b200.so
 (include/uam_b200.h) from the REFERENCE'S OWN classes with ctypes.  Shown in INTEGRATION.md section 2 and executed by
-tests/test_integration_binding.py (CPU: table extraction from the reference's closures, when /root/reference exists;
-GPU: the raw binding below against the reference's golden costs).
+tests/test_integration_binding.py (CPU: table extraction from closures laid out like the reference's, against the tables
+frozen from the reference's own objects; GPU: the raw binding below against the reference's golden costs).
 
 Nothing here imports uam_path_planning_b200: only ctypes + numpy + the shared library.
 

@@ -246,7 +246,6 @@ def test_c_abi_exports_every_declared_symbol():
     assert b'sm_100a' in lib.uam_version()
 
 
-@pytest.mark.skipif(have_gpu(), reason='checks the behaviour WITHOUT a CUDA device')
 def test_option_and_stat_tables_match_the_header():
     """Engine.OPTIONS / Engine.STATS are the enum values of include/uam_b200.h (UAM_OPT_* / UAM_STAT_*): every enumerator has
     its name in the Python table with the same number, and nothing else is in the tables."""
@@ -263,7 +262,18 @@ def test_option_and_stat_tables_match_the_header():
 
 
 def test_no_cpu_fallback():
-    """Without a GPU the product refuses to work: ctx creation fails and every evaluation raises."""
+    """Without a GPU the product refuses to work: ctx creation fails and every evaluation raises.  On a machine with a GPU
+    the same checks run in a child process that sees no device (CUDA_VISIBLE_DEVICES empty)."""
+    if not have_gpu():
+        _check_no_cpu_fallback()
+        return
+    code = 'import conftest, test_host_logic as t; t._check_no_cpu_fallback(); print("ok")'
+    r = subprocess.run([sys.executable, '-c', code], cwd=os.path.dirname(os.path.abspath(__file__)), capture_output=True,
+                       text=True, timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=''))
+    assert r.returncode == 0 and r.stdout.strip().endswith('ok'), r.stdout[-3000:] + r.stderr[-3000:]
+
+
+def _check_no_cpu_fallback():
     lib = _lib.load()
     h = ctypes.c_void_p()
     assert lib.uam_ctx_create(0, ctypes.byref(h)) == -2 and not h.value

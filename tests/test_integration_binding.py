@@ -1,12 +1,14 @@
 """INTEGRATION.md section 2 executed: integration/gpu_backend.py (the file a maintainer adds to the reference) binds
 libuam_b200.so with plain ctypes from the reference's own classes.
 
-CPU part (needs /root/reference, skipped elsewhere): the tables read out of the reference's closures equal the frozen
-tests/golden/reference_tables.npz and, bit for bit, the tables the product's own constructors build.
+CPU part: the tables gpu_backend.extract_tables reads out of closures laid out like the reference's equal the frozen
+tests/golden/reference_tables.npz (what it read from the reference's own objects, tests/golden/make_reference_tables.py)
+and, bit for bit, the tables the product's own constructors build.
 GPU part: the raw binding, fed with the frozen tables, reproduces the reference's golden costs / constraint vectors.
 """
 import os
 import sys
+from types import SimpleNamespace
 
 import numpy as np
 import pytest
@@ -16,7 +18,6 @@ from conftest import build_product_map, full_paths
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, 'integration'))
 GOLD = os.path.join(ROOT, 'tests', 'golden')
-HAVE_REF = os.path.isdir('/root/reference/geo_simulation_project/path_generation')
 
 
 def _tables():
@@ -24,22 +25,64 @@ def _tables():
     return {k: t[k] for k in t.files}
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='needs the reference tree (authoring container only)')
+# The reference's objects as gpu_backend sees them: a shape has `.inequalities` (`Function`s whose `.f` is a closure over
+# the shape's numbers, with the reference's variable names) and `.center`; a map has `.obstacles`, `.regions[name]['shapes']`
+# and `.region_names()`; a problem has `.map`, `.params`, `.weights`, `.options`.
+def _function(f):
+    return SimpleNamespace(f=f)
+
+
+def _polygon_edge(Pa_F, Pb_F, sgn_F):                          # polygon.py:66-98
+    def line_F(x):
+        return (Pb_F[1, 0] - Pa_F[1, 0]) * (x[0] - Pa_F[0, 0]) - (Pb_F[0, 0] - Pa_F[0, 0]) * (x[1] - Pa_F[1, 0])
+    return _function(lambda x: -sgn_F * line_F(x))
+
+
+def _ellipse(center, r1, r2):                                  # ball.py:33-37
+    def func(x):
+        return ((x[0] - center[0]) / r1) ** 2 + ((x[1] - center[1]) / r2) ** 2 - 1
+    return _function(func)
+
+
+def _square_sides(center, r1, r2):                             # square.py:29-51: right, left, top, bottom
+    return [_function(lambda x: x[0] - center[0] - r1), _function(lambda x: -x[0] + center[0] - r1),
+            _function(lambda x: x[1] - center[1] - r2), _function(lambda x: -x[1] + center[1] - r2)]
+
+
+def _reference_layout_shape(s):
+    """a product shape (vertex order and edge signs of its constructor) -> the same numbers in the reference's closures"""
+    R = s.records()
+    if s.kind == 'polygon':
+        P = [r[1:3].reshape(2, 1) for r in R]                  # hull vertices in edge order: edge k runs P[k] -> P[k + 1]
+        ineq = [_polygon_edge(P[k], P[(k + 1) % len(P)], r[5]) for k, r in enumerate(R)]
+    else:
+        assert s.kind == 'ball'
+        ineq = [_ellipse(R[0, 1:3].copy(), R[0, 3], R[0, 4])]
+    return SimpleNamespace(inequalities=ineq, center=s.center)
+
+
+def _reference_layout_problem(spec, N=80):
+    m = build_product_map(spec)
+    names = [name for name, _ in spec['regions']]
+    regions = {n: {'shapes': [_reference_layout_shape(s) for s in shapes]} for n, shapes in zip(names, m._region_lists())}
+    rm = SimpleNamespace(obstacles=[_reference_layout_shape(s) for s in m.obstacles], regions=regions,
+                         region_names=lambda: list(regions), x_start=spec['x_start'], x_goal=spec['x_goal'])
+    return SimpleNamespace(map=rm, N=N, options=dict(spec['options']), weights=dict(zip(names, spec['weights'])),
+                           params={'maxratio': spec['maxratio'], 'maxalpha': spec['maxalpha'], 'enlargement': spec['enlargement']})
+
+
 def test_tables_from_reference_closures(fixture_spec):
-    import subprocess
-    # in a subprocess: the reference's modules and the casadi stand-in must not leak into this interpreter
-    code = ('import sys, numpy as np; sys.path.insert(0, %r); sys.path.insert(0, %r);'
-            'import make_reference_tables as mt, gpu_backend as gb;'
-            'spec, m, pr = mt.reference_map_and_problem();'
-            't = gb.extract_tables(m); g = gb.GpuProblem.__new__(gb.GpuProblem); g.p = pr;'
-            'np.savez(sys.argv[1], p=g.parameter_vector(), flags=g.flags(), **t)') % (GOLD, os.path.join(ROOT, 'integration'))
-    import tempfile
-    out = os.path.join(tempfile.mkdtemp(), 't.npz')
-    subprocess.run([sys.executable, '-W', 'ignore', '-c', code, out], check=True, cwd=GOLD)
-    got, frozen = np.load(out), _tables()
+    import gpu_backend as gb
+    pr = _reference_layout_problem(fixture_spec)
+    g = gb.GpuProblem.__new__(gb.GpuProblem)                    # no device context: only the host-side packing
+    g.p = pr
+    got, frozen = gb.extract_tables(pr.map), _tables()
     for k in ('edges', 'off', 'region', 'center'):
         assert np.array_equal(got[k], frozen[k]), k
     assert int(got['n_regions']) == int(frozen['n_regions']) == 3
+    sq = np.array([gb.inequality_record(f) for f in _square_sides(np.array([1.0, 1.0]), 0.5, 0.25)])
+    assert np.array_equal(sq, frozen['square_records'])          # the box sides are told apart by probing f
+    got = dict(got, p=g.parameter_vector(), flags=g.flags())
     # ... and they are the tables the product's constructors build from the same numbers
     from uam_path_planning_b200.shapes import flatten_shapes
     m = build_product_map(fixture_spec)
