@@ -221,6 +221,22 @@ int uam_score_paths_raster_host(uam_ctx* ctx, const double* h_z, int64_t B, int 
                                 int n_p, int flags, double samples_per_cell, float* h_cost,
                                 uint8_t* h_collide);
 
+/* Gradient of the raster cost with respect to every waypoint: d_grad (B, 2(N+2)) float64, same layout as d_z (columns
+ * 2 .. 2N+1 are the solver's variables z_1..z_N).  d_cost / d_collide (nullable) receive the same bits as
+ * uam_score_paths_raster for the same inputs and options, so the gradient is that of the function being scored:
+ *   - the sample counts S_k are held fixed: S_k is piecewise constant in z and the cost jumps where it changes; the
+ *     gradient is that of the piece the path is on;
+ *   - dP/du on the cell the scorer samples, at its fp32 fractions: sum_l w_l ((1-fy)(t01-t00) + fy(t11-t10)) (dP/dv
+ *     likewise), 0 in a coordinate whose clamp to [0, W-1] / [0, H-1] is active; du/dx = 1/dx, dv/dy = 1/dy;
+ *   - sample s of segment k moves with weight 1 - s/S_k with z_k and s/S_k with z_{k+1}; the goal sample with z_{N+1};
+ *   - the length part is uam_grad_paths_analytic's (fp64, pairs (m_s, z_0) unless UAM_OWN_START, last segment absent;
+ *     2 d with UAM_LENGTH_SMOOTH, else d / |d| with the zero subgradient at |d| = 0), times N+1.
+ * Penalty slopes are summed in fp32 like the cost, in an order fixed per path: a path's gradient has the same bits
+ * whatever else the batch holds.  Same kernel choice as the scorer (waypoint kernel; integral mode: variant -1 / 0 / 2,
+ * quad texels where the scorer uses them); a forced integral variant 1 or 3 gives UAM_ERR_UNSUPPORTED. */
+int uam_grad_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
+                          double samples_per_cell, float* d_cost, uint8_t* d_collide, double* d_grad, void* stream);
+
 /* Scoring + best candidate in one call: as uam_score_paths_raster, and *d_key receives the best key (see uam_best) of the
  * batch -- of ALL ranks' batches when a peer group is attached (uam_peer_attach): the last kernel of the step finds the
  * local min, pushes it into every peer's symmetric block over NVLink and waits for theirs (no separate collective).

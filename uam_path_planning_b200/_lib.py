@@ -50,6 +50,7 @@ SIGNATURES = {
     'uam_analytic_g_len': (_i, [_vp, _i, C.POINTER(_i64)]),
     'uam_score_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _vp, _vp, _vp, _vp]),
     'uam_score_paths_raster_host': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _vp, _vp]),
+    'uam_grad_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _vp, _vp, _vp, _vp]),
     'uam_eval_points': (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     'uam_eval_points_host': (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp]),
     'uam_eval_inequalities_host': (_i, [_vp, _vp, _i, _vp, _i64, _vp]),

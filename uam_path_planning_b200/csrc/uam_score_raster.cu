@@ -193,6 +193,39 @@ __device__ __forceinline__ void uam_tap_eval(const UamRasterParams& rp, const Ua
     }
 }
 
+// Slopes of one layer's bilinear interpolant on the sampled cell, at the fp32 fractions of the tap.
+__device__ __forceinline__ void uam_lerp2_grad(float t00, float t01, float t10, float t11, float fx, float fy, float& du, float& dv) {
+    du = (1.0f - fy) * (t01 - t00) + fy * (t11 - t10);
+    dv = (1.0f - fx) * (t10 - t00) + fx * (t11 - t01);
+}
+
+// uam_tap_eval (same pen / occ bits) + the slopes dP/du, dP/dv of the weighted penalty on the sampled cell.  The caller
+// zeroes a slope whose clamp is active (the clamped coordinate does not move with the waypoint).
+template <int TF>
+__device__ __forceinline__ void uam_tap_grad(const UamRasterParams& rp, const UamTap<TF>& t, float& pen, bool& occ, float& du, float& dv) {
+    uam_tap_eval<TF>(rp, t, pen, occ);
+    if constexpr (TF == 8) {
+        uam_lerp2_grad(fabsf(t.q.x), fabsf(t.q.y), fabsf(t.q.z), fabsf(t.q.w), t.fx, t.fy, du, dv);
+        du *= rp.w0; dv *= rp.w0;
+    } else if constexpr (TF == 1) {
+        uam_lerp2_grad(t.q.x, t.q.y, t.q.z, t.q.w, t.fx, t.fy, du, dv);
+        du *= rp.w0; dv *= rp.w0;
+    } else {
+        uam_lerp2_grad(t.a.x, t.b.x, t.c.x, t.d.x, t.fx, t.fy, du, dv);
+        du *= rp.w0; dv *= rp.w0;
+        if constexpr (TF == 4) {
+            float u1, v1, u2, v2;
+            uam_lerp2_grad(t.a.y, t.b.y, t.c.y, t.d.y, t.fx, t.fy, u1, v1);
+            uam_lerp2_grad(t.a.z, t.b.z, t.c.z, t.d.z, t.fx, t.fy, u2, v2);
+            du += rp.w1 * u1 + rp.w2 * u2;
+            dv += rp.w1 * v1 + rp.w2 * v2;
+        }
+    }
+}
+
+// true where the clamp of a pixel coordinate to [0, n-1] is inactive (the sample moves with its waypoint)
+__device__ __forceinline__ bool uam_free_coord(double u, int n) { return u >= 0.0 && u <= (double)(n - 1); }
+
 // Weighted bilinear penalty + nearest-cell occupancy at pixel coordinates (u, v): one lane fetches all 4 texels.
 template <int TF, int LAYOUT>
 __device__ __forceinline__ void uam_sample(const typename UamTexel<TF>::T* __restrict__ tex, const UamRasterParams& rp,
@@ -282,6 +315,42 @@ __device__ __forceinline__ double uam_len_term(const double2* __restrict__ zp, i
     return acc;
 }
 
+// d(length term)/d z_j in fp64, the expressions of uam_k_grad_analytic: pairs (m_s, z_0) (unless UAM_OWN_START),
+// (z_0, z_1), ..., (z_{N-1}, z_N); 2 d with UAM_LENGTH_SMOOTH, else d / |d| (zero subgradient at |d| = 0)
+__device__ __forceinline__ double2 uam_len_grad(const double2* __restrict__ zp, int j, int N, const double2 p,
+                                                const UamRasterParams& rp) {
+    const bool len_smooth = (rp.flags & UAM_LENGTH_SMOOTH) != 0;
+    double Lx = 0.0, Ly = 0.0;
+    if (j <= N) {
+        if (j >= 1 || !(rp.flags & UAM_OWN_START)) {
+            const double2 a = j >= 1 ? zp[j - 1] : make_double2(rp.ms_x, rp.ms_y);
+            const double dx = p.x - a.x, dy = p.y - a.y;
+            if (len_smooth) { Lx += 2.0 * dx; Ly += 2.0 * dy; }
+            else { const double n = sqrt(dx * dx + dy * dy); if (n > 0.0) { Lx += dx / n; Ly += dy / n; } }
+        }
+        if (j <= N - 1) {
+            const double2 q = zp[j + 1];
+            const double dx = q.x - p.x, dy = q.y - p.y;
+            if (len_smooth) { Lx -= 2.0 * dx; Ly -= 2.0 * dy; }
+            else { const double n = sqrt(dx * dx + dy * dy); if (n > 0.0) { Lx -= dx / n; Ly -= dy / n; } }
+        }
+    }
+    return make_double2(Lx, Ly);
+}
+
+// Per-segment gradient sums -> the segment's share of its two waypoints' penalty gradient (pixel units, fp32).
+// In: su = {sum dP/du, sum s dP/du, sum dP/dv, sum s dP/dv} over the segment's samples s = 0..S-1, is = 1/S.  Sample s
+// sits at (1 - s/S) z_k + (s/S) z_{k+1} and carries weight 1/S: out = {z_k: du, dv, z_{k+1}: du, dv}.
+__device__ __forceinline__ float4 uam_seg_grad(float4 su, float is) {
+    return make_float4(is * (su.x - is * su.y), is * (su.z - is * su.w), is * (is * su.y), is * (is * su.w));
+}
+
+// Gradient of waypoint j: (N+1) d(length)/dz_j + (1/N) dP/dz_j, with (pu, pv) the penalty part in pixel units
+__device__ __forceinline__ double2 uam_grad_point(double2 lg, float pu, float pv, int N, const UamRasterParams& rp) {
+    const double dN1 = (double)(N + 1), dN = (double)N;
+    return make_double2(dN1 * lg.x + (double)pu / rp.dx / dN, dN1 * lg.y + (double)pv / rp.dy / dN);
+}
+
 // sample count of a segment with pixel-space extent (dU, dV)
 __device__ __forceinline__ double uam_seg_samples(double dU, double dV, double spc) {
     double Sd = fmax(1.0, ceil(__dmul_rn(uam_norm2r(dU, dV), spc)));
@@ -314,11 +383,13 @@ __device__ __forceinline__ UamSegTable uam_seg_table(unsigned char* base, int n)
 }
 
 // ---- waypoint mode ----------------------------------------------------------------------------------------
-template <int TF, int LAYOUT>
+// GRAD: also the gradient (uam_grad_paths_raster): every waypoint is its own segment's only sample (weight 1), so
+// waypoint j's gradient is its own tap's slopes + its length part, written by the lane that holds it.
+template <int TF, int LAYOUT, bool GRAD = false>
 __global__ void __launch_bounds__(UAM_CTA_THREADS)
 uam_k_score_raster_wp(const double2* __restrict__ z, long long B, int Wp, UamRasterParams rp,
                       const typename UamTexel<TF>::T* __restrict__ tex, float* __restrict__ cost,
-                      uint8_t* __restrict__ collide, long long* __restrict__ nsamp) {
+                      uint8_t* __restrict__ collide, long long* __restrict__ nsamp, double2* __restrict__ grad) {
     const int lane = threadIdx.x & 31;
     const long long warp0 = (long long)blockIdx.x * UAM_WARPS_PER_CTA + (threadIdx.x >> 5);
     const long long nwarps = (long long)gridDim.x * UAM_WARPS_PER_CTA;
@@ -341,13 +412,31 @@ uam_k_score_raster_wp(const double2* __restrict__ z, long long B, int Wp, UamRas
             if (two) len_sum += uam_len_term(zp, j2, N, q, rp);
             float pen;
             bool occ;
-            uam_tap_eval<TF>(rp, ta, pen, occ);
-            pen_sum += pen;
-            col = col || occ;
-            uam_tap_eval<TF>(rp, tb, pen, occ);
-            if (two) {
+            if constexpr (GRAD) {
+                float du, dv;
+                uam_tap_grad<TF>(rp, ta, pen, occ, du, dv);
                 pen_sum += pen;
                 col = col || occ;
+                const double pu = uam_pix(p.x, rp.x0, rp.dx), pv = uam_pix(p.y, rp.y0, rp.dy);
+                grad[path * Wp + j] = uam_grad_point(uam_len_grad(zp, j, N, p, rp), uam_free_coord(pu, rp.W) ? du : 0.0f,
+                                                     uam_free_coord(pv, rp.H) ? dv : 0.0f, N, rp);
+                uam_tap_grad<TF>(rp, tb, pen, occ, du, dv);
+                if (two) {
+                    pen_sum += pen;
+                    col = col || occ;
+                    const double qu = uam_pix(q.x, rp.x0, rp.dx), qv = uam_pix(q.y, rp.y0, rp.dy);
+                    grad[path * Wp + j2] = uam_grad_point(uam_len_grad(zp, j2, N, q, rp), uam_free_coord(qu, rp.W) ? du : 0.0f,
+                                                          uam_free_coord(qv, rp.H) ? dv : 0.0f, N, rp);
+                }
+            } else {
+                uam_tap_eval<TF>(rp, ta, pen, occ);
+                pen_sum += pen;
+                col = col || occ;
+                uam_tap_eval<TF>(rp, tb, pen, occ);
+                if (two) {
+                    pen_sum += pen;
+                    col = col || occ;
+                }
             }
         }
         pen_sum = uam_warp_sum(pen_sum);
@@ -365,16 +454,23 @@ uam_k_score_raster_wp(const double2* __restrict__ z, long long B, int Wp, UamRas
 // The path's samples are flattened (segment k owns flat indices [P_k, P_{k+1})), lanes stride the flat index, so 32
 // consecutive samples of one polyline -- a compact footprint in the raster -- are fetched together and no lane
 // idles on short segments.  Total samples per path are capped at 2^31 - 1 by the host-side S_k cap.
-template <int TF, int LAYOUT, int PAIR>
+// GRAD (PAIR = 0 only): also the gradient.  One sample per lane per trip and all lanes run every trip; per window of 32
+// consecutive samples the lanes of each segment's run combine their {dP/du, s dP/du, dP/dv, s dP/dv} with a segmented
+// shuffle sum keyed by the segment, and the run's last lane adds the result to the segment's sums in shared memory (one
+// writer per segment and window, windows in order: the bits depend on the path alone).  The per-lane penalty sums see
+// the same samples in the same order as the scorer's two-per-trip loop, so cost and collide are the scorer's bits.
+template <int TF, int LAYOUT, int PAIR, bool GRAD = false>
 __global__ void __launch_bounds__(UAM_CTA_THREADS)
 uam_k_score_raster_int(const double2* __restrict__ z, long long B, int Wp, UamRasterParams rp,
                        const typename UamTexel<TF>::T* __restrict__ tex, float* __restrict__ cost,
-                       uint8_t* __restrict__ collide, long long* __restrict__ nsamp) {
+                       uint8_t* __restrict__ collide, long long* __restrict__ nsamp, double2* __restrict__ grad) {
     extern __shared__ __align__(128) unsigned char uam_smem[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int wpc = blockDim.x >> 5;
-    const UamSegTable tb = uam_seg_table(uam_smem + (size_t)warp * uam_seg_table_bytes(Wp), Wp);
+    unsigned char* const wbase = uam_smem + (size_t)warp * (uam_seg_table_bytes(Wp) + (GRAD ? (size_t)Wp * sizeof(float4) : 0));
+    const UamSegTable tb = uam_seg_table(wbase, Wp);
+    float4* const gs = reinterpret_cast<float4*>(wbase + uam_seg_table_bytes(Wp));     // GRAD: per-segment sums
     const long long warp0 = (long long)blockIdx.x * wpc + warp;
     const long long nwarps = (long long)gridDim.x * wpc;
     const int N = Wp - 2;
@@ -426,7 +522,62 @@ uam_k_score_raster_int(const double2* __restrict__ z, long long B, int Wp, UamRa
         int k = 0, p1 = tb.P[1];
         double kU = tb.U[0], kV = tb.V[0], kSU = tb.SU[0], kSV = tb.SV[0];
         float kIS = tb.IS[0];
-        if (PAIR) {
+        if constexpr (GRAD) {
+            for (int j = lane; j < Wp; j += 32) gs[j] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+            __syncwarp();
+            double sd = (double)lane;
+            for (int t0 = 0; t0 < T; t0 += 32) {
+                const int t = t0 + lane;
+                float4 g = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                int kk = Wp;                      // lanes past the end: a key no segment has
+                if (t < T) {
+                    if (t >= p1) {
+                        do { ++k; p1 = tb.P[k + 1]; } while (t >= p1);
+                        sd = (double)(t - tb.P[k]);
+                        kU = tb.U[k]; kV = tb.V[k]; kSU = tb.SU[k]; kSV = tb.SV[k]; kIS = tb.IS[k];
+                    }
+                    const double u = __dadd_rn(kU, __dmul_rn(sd, kSU));
+                    const double v = __dadd_rn(kV, __dmul_rn(sd, kSV));
+                    const float s = (float)sd;
+                    sd += 32.0;
+                    UamTap<TF> a;
+                    uam_tap_load<TF, LAYOUT>(tex, rp, u, v, a);
+                    float pen, du, dv;
+                    bool occ;
+                    uam_tap_grad<TF>(rp, a, pen, occ, du, dv);
+                    acc += pen * kIS;
+                    col = col || occ;
+                    if (!uam_free_coord(u, rp.W)) du = 0.0f;
+                    if (!uam_free_coord(v, rp.H)) dv = 0.0f;
+                    g = make_float4(du, s * du, dv, s * dv);
+                    kk = k;
+                }
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const int ko = __shfl_up_sync(0xffffffffu, kk, o);
+                    const float x = __shfl_up_sync(0xffffffffu, g.x, o), y = __shfl_up_sync(0xffffffffu, g.y, o);
+                    const float zz = __shfl_up_sync(0xffffffffu, g.z, o), w = __shfl_up_sync(0xffffffffu, g.w, o);
+                    if (lane >= o && ko == kk) { g.x += x; g.y += y; g.z += zz; g.w += w; }
+                }
+                const int kn = __shfl_down_sync(0xffffffffu, kk, 1);
+                if (kk < Wp && (lane == 31 || kn != kk)) {
+                    float4 c = gs[kk];
+                    c.x += g.x; c.y += g.y; c.z += g.z; c.w += g.w;
+                    gs[kk] = c;
+                }
+                __syncwarp();
+            }
+            for (int j = lane; j < Wp; j += 32) {
+                const float4 a = uam_seg_grad(gs[j], tb.IS[j]);
+                float pu = a.x, pv = a.y;
+                if (j >= 1) {
+                    const float4 b = uam_seg_grad(gs[j - 1], tb.IS[j - 1]);
+                    pu += b.z;
+                    pv += b.w;
+                }
+                grad[path * Wp + j] = uam_grad_point(uam_len_grad(zp, j, N, zp[j], rp), pu, pv, N, rp);
+            }
+        } else if (PAIR) {
             const int side = lane & 1;
             double sd = (double)(lane >> 1);
             for (int tb0 = 0; tb0 < T; tb0 += 16) {
@@ -797,14 +948,19 @@ template <int TF> struct UamTapsPerTrip { static const int N = 2; };
 template <> struct UamTapsPerTrip<1> { static const int N = 4; };
 template <> struct UamTapsPerTrip<8> { static const int N = 4; };
 
+// GRAD: four more 32 x 33 partial matrices behind the group's shared memory, for the per-record sums of dP/du, s dP/du,
+// dP/dv and s dP/dv (s = the sample's number in its record); flushed and reduced exactly like the penalty partials.
+#define UAM_GROUP_GPART (32 * 33)
+#define UAM_GROUP_SMEM_GRAD (UAM_GROUP_SMEM + 4 * UAM_GROUP_GPART * 4)     // 22832
+
 // The sample loop of uam_group_score.  CLAMP = false: the caller guarantees that every sample of the group lies
 // strictly inside the raster.
-template <int TF, int LAYOUT, int TILE, bool CLAMP>
+template <int TF, int LAYOUT, int TILE, bool CLAMP, bool GRAD = false>
 __device__ __forceinline__ void uam_group_samples(const UamRasterParams& rp, const typename UamTexel<TF>::T* __restrict__ tex,
                                                   const unsigned char* s_tile, int ti0, int tj0, const UamGroupRec* s_rec,
                                                   const int2* s_PQ, float* part, uint2* s_tab, unsigned* s_bits, const int lane,
                                                   const int P, const int S, const int T, float& acc, unsigned& colmask, int& kcur,
-                                                  int& pcur) {
+                                                  int& pcur, float* gpart, float4& gacc) {
     constexpr int TAPS = UamTapsPerTrip<TF>::N;
     const unsigned le_mask = 0xffffffffu >> (31 - lane);
     // record parameters of this lane's current record (re-read only when the record changes)
@@ -849,6 +1005,8 @@ __device__ __forceinline__ void uam_group_samples(const UamRasterParams& rp, con
         for (int t0 = f0; t0 < t_end; t0 += 32 * TAPS) {
             UamTap<TF> tap[TAPS];
             int kk[TAPS], pp[TAPS];
+            float ss[TAPS];                 // GRAD: sample number in the record, slopes kept per coordinate
+            bool fu[TAPS], fv[TAPS];
             const uint2* tab = s_tab + ((t0 - f0) >> 5);
 #pragma unroll
             for (int j = 0; j < TAPS; ++j) {
@@ -872,21 +1030,42 @@ __device__ __forceinline__ void uam_group_samples(const UamRasterParams& rp, con
                 const double u = __dadd_rn(ca.x, __dmul_rn(sd, ca.y)), v = __dadd_rn(cb.x, __dmul_rn(sd, cb.y));
                 if constexpr (TILE) uam_tap_load_tile<TF>(s_tile, ti0, tj0, rp, u, v, tap[j]);
                 else uam_tap_load<TF, LAYOUT, CLAMP>(tex, rp, u, v, tap[j]);
+                if constexpr (GRAD) {
+                    ss[j] = (float)(wb + lane - qc);
+                    fu[j] = !CLAMP || uam_free_coord(u, rp.W);
+                    fv[j] = !CLAMP || uam_free_coord(v, rp.H);
+                }
             }
 #pragma unroll
             for (int j = 0; j < TAPS; ++j) {
-                float pen;
+                float pen, du, dv;
                 bool occ;
-                uam_tap_eval<TF>(rp, tap[j], pen, occ);
+                if constexpr (GRAD) uam_tap_grad<TF>(rp, tap[j], pen, occ, du, dv);
+                else uam_tap_eval<TF>(rp, tap[j], pen, occ);
                 const int k = kk[j];
                 if (k != kcur) {
                     const int row = (lane - pcur) & 31;          // record-local residue class of this lane's samples
                     part[row * 33 + kcur] = acc;
                     acc = 0.0f;
+                    if constexpr (GRAD) {
+                        gpart[row * 33 + kcur] = gacc.x;
+                        gpart[UAM_GROUP_GPART + row * 33 + kcur] = gacc.y;
+                        gpart[2 * UAM_GROUP_GPART + row * 33 + kcur] = gacc.z;
+                        gpart[3 * UAM_GROUP_GPART + row * 33 + kcur] = gacc.w;
+                        gacc = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                    }
                     kcur = k;
                     pcur = pp[j];
                 }
                 acc += pen;
+                if constexpr (GRAD) {
+                    if (!fu[j]) du = 0.0f;
+                    if (!fv[j]) dv = 0.0f;
+                    gacc.x += du;
+                    gacc.y += ss[j] * du;
+                    gacc.z += dv;
+                    gacc.w += ss[j] * dv;
+                }
                 colmask |= uam_shl_clamp(occ ? 1u : 0u, (unsigned)k);    // (k = 32, the dummy of a full group: shifted out)
             }
         }
@@ -903,11 +1082,32 @@ __device__ __forceinline__ void uam_group_samples(const UamRasterParams& rp, con
 // parameters only when its record changes; (3) a lane's partial for record k goes to the row of its record-local
 // residue class (lane - P_k) mod 32, so the final per-record sums are one 32 x 32 transpose-reduce (31 shuffles)
 // instead of 32 warp sums (160 shuffles) -- same pairing tree, same bits.
-template <int TF, int LAYOUT, int TILE>
+// per-record sums of a 32 x 33 partial matrix: v[s] = this lane's residue class of record s; 32 x 32 transpose-reduce,
+// pairing tree (l, l^16), (.., ^8), (.., ^4), (.., ^2), (.., ^1) like uam_warp_sum; lane s ends with the sum of record s
+__device__ __forceinline__ float uam_part_reduce(const float* part, const int lane) {
+    float v[32];
+#pragma unroll
+    for (int s = 0; s < 32; ++s) v[s] = part[lane * 33 + s];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const bool hi = (lane & o) != 0;
+#pragma unroll
+        for (int i = 0; i < o; ++i) {
+            const float send = hi ? v[i] : v[i + o];
+            const float keep = hi ? v[i + o] : v[i];
+            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+        }
+    }
+    return v[0];
+}
+
+// GRAD: gmine = the record's {sum dP/du, sum s dP/du, sum dP/dv, sum s dP/dv} (slopes of clamped coordinates are 0).
+template <int TF, int LAYOUT, int TILE, bool GRAD = false>
 __device__ __forceinline__ void uam_group_score(const UamRasterParams& rp, const typename UamTexel<TF>::T* __restrict__ tex,
                                                 const unsigned char* s_tile, int ti0, int tj0, unsigned char* warp_smem,
                                                 const int lane, const double U, const double V, const double SU,
-                                                const double SV, const int S, const int s0, float& mine, bool& collide) {
+                                                const double SV, const int S, const int s0, float& mine, bool& collide,
+                                                float4* gmine = nullptr) {
     UamGroupRec* s_rec = reinterpret_cast<UamGroupRec*>(warp_smem + UAM_GROUP_REC_OFF);
     int2* s_PQ = reinterpret_cast<int2*>(warp_smem + UAM_GROUP_PQ_OFF);       // {P_k, Q_k = P_k - s0_k}: flat index -> sample number
     float* part = reinterpret_cast<float*>(warp_smem + UAM_GROUP_PART_OFF);
@@ -938,6 +1138,11 @@ __device__ __forceinline__ void uam_group_score(const UamRasterParams& rp, const
 #pragma unroll
     for (int q = 0; q < 9; ++q)
         if (q * 32 + lane < 32 * 33 / 4) reinterpret_cast<float4*>(part)[q * 32 + lane] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    float* const gpart = reinterpret_cast<float*>(warp_smem + UAM_GROUP_SMEM);
+    if constexpr (GRAD) {
+#pragma unroll
+        for (int q = 0; q < 33; ++q) reinterpret_cast<float4*>(gpart)[q * 32 + lane] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    }
     __syncwarp();
     // Fast path: when every record of the group lies strictly inside the raster (first and last sample in
     // [0, W-1) x [0, H-1); the samples in between are monotone), the clamps and the saturation of the cell / fraction
@@ -952,44 +1157,44 @@ __device__ __forceinline__ void uam_group_score(const UamRasterParams& rp, const
     float acc = 0.0f;
     unsigned colmask = 0;
     int kcur = 0, pcur = 0;     // the record `acc` belongs to and its first flat index
-    if (all_inside) uam_group_samples<TF, LAYOUT, TILE, false>(rp, tex, s_tile, ti0, tj0, s_rec, s_PQ, part, s_tab, s_bits, lane, P, S, T, acc, colmask, kcur, pcur);
-    else uam_group_samples<TF, LAYOUT, TILE, true>(rp, tex, s_tile, ti0, tj0, s_rec, s_PQ, part, s_tab, s_bits, lane, P, S, T, acc, colmask, kcur, pcur);
+    float4 gacc = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    if (all_inside) uam_group_samples<TF, LAYOUT, TILE, false, GRAD>(rp, tex, s_tile, ti0, tj0, s_rec, s_PQ, part, s_tab, s_bits, lane, P, S, T, acc, colmask, kcur, pcur, gpart, gacc);
+    else uam_group_samples<TF, LAYOUT, TILE, true, GRAD>(rp, tex, s_tile, ti0, tj0, s_rec, s_PQ, part, s_tab, s_bits, lane, P, S, T, acc, colmask, kcur, pcur, gpart, gacc);
     {
         const int row = (lane - pcur) & 31;
         part[row * 33 + kcur] = acc;             // (kcur = 32, the dummy of a full group, is the padding column)
-    }
-    __syncwarp();
-    // per-record sums: v[s] = this lane's residue class of record s; 32 x 32 transpose-reduce, pairing tree
-    // (l, l^16), (.., ^8), (.., ^4), (.., ^2), (.., ^1) like uam_warp_sum; lane s ends with the sum of record s
-    float v[32];
-#pragma unroll
-    for (int s = 0; s < 32; ++s) v[s] = part[lane * 33 + s];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const bool hi = (lane & o) != 0;
-#pragma unroll
-        for (int i = 0; i < o; ++i) {
-            const float send = hi ? v[i] : v[i + o];
-            const float keep = hi ? v[i + o] : v[i];
-            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+        if constexpr (GRAD) {
+            gpart[row * 33 + kcur] = gacc.x;
+            gpart[UAM_GROUP_GPART + row * 33 + kcur] = gacc.y;
+            gpart[2 * UAM_GROUP_GPART + row * 33 + kcur] = gacc.z;
+            gpart[3 * UAM_GROUP_GPART + row * 33 + kcur] = gacc.w;
         }
     }
-    mine = v[0];
+    __syncwarp();
+    mine = uam_part_reduce(part, lane);
+    if constexpr (GRAD) {
+        gmine->x = uam_part_reduce(gpart, lane);
+        gmine->y = uam_part_reduce(gpart + UAM_GROUP_GPART, lane);
+        gmine->z = uam_part_reduce(gpart + 2 * UAM_GROUP_GPART, lane);
+        gmine->w = uam_part_reduce(gpart + 3 * UAM_GROUP_GPART, lane);
+    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) colmask |= __shfl_xor_sync(0xffffffffu, colmask, o);
     collide = ((colmask >> lane) & 1u) != 0u;
     __syncwarp();
 }
 
-template <int TF, int LAYOUT>
-__global__ void __launch_bounds__(UAM_CTA_THREADS, 4)
+// GRAD: also part_grad[id] = the segment's share of its two waypoints' penalty gradient (uam_seg_grad); 22.8 KB of shared
+// memory per warp, so one CTA of 8 warps per SM.
+template <int TF, int LAYOUT, bool GRAD = false>
+__global__ void __launch_bounds__(UAM_CTA_THREADS, GRAD ? 1 : 4)
 uam_k_score_groups(unsigned long long n_seg, int Wp, UamRasterParams rp, const typename UamTexel<TF>::T* __restrict__ tex,
                    const double2* __restrict__ z, const unsigned* __restrict__ sorted_id, float* __restrict__ part_pen,
-                   uint8_t* __restrict__ part_col, unsigned* __restrict__ next_group) {
+                   uint8_t* __restrict__ part_col, unsigned* __restrict__ next_group, float4* __restrict__ part_grad) {
     extern __shared__ __align__(128) unsigned char uam_smem[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
-    unsigned char* base = uam_smem + (size_t)warp * UAM_GROUP_SMEM;
+    unsigned char* base = uam_smem + (size_t)warp * (GRAD ? UAM_GROUP_SMEM_GRAD : UAM_GROUP_SMEM);
     const unsigned long long n_groups = (n_seg + 31) >> 5;
     // The groups are handed out through a counter, in sorted order: a warp that finishes early takes the next group instead of
     // idling behind a fixed share (ncu r02 with a fixed round-robin share per warp: the SMs were busy 91 % of the kernel's
@@ -1009,7 +1214,11 @@ uam_k_score_groups(unsigned long long n_seg, int Wp, UamRasterParams rp, const t
         if (have) r = uam_make_segment(z, (unsigned long long)__ldg(sorted_id + ridx), Wp, rp);
         float mine;
         bool col;
-        uam_group_score<TF, LAYOUT, 0>(rp, tex, nullptr, 0, 0, base, lane, r.U, r.V, r.SU, r.SV, r.S, 0, mine, col);
+        float4 gmine;
+        uam_group_score<TF, LAYOUT, 0, GRAD>(rp, tex, nullptr, 0, 0, base, lane, r.U, r.V, r.SU, r.SV, r.S, 0, mine, col, &gmine);
+        if constexpr (GRAD) {
+            if (have) part_grad[r.id] = uam_seg_grad(gmine, r.IS);
+        }
         if (have) {
             if (TF == 8 && rp.w0 >= 0.0f) {
                 // sign-packed quads with a weight >= 0: every tap is >= 0, so the partial is >= 0 (or NaN) and its sign bit is
@@ -1028,12 +1237,15 @@ uam_k_score_groups(unsigned long long n_seg, int Wp, UamRasterParams rp, const t
 // BEST: the launch also finds the best candidate (and exchanges it with the peer ranks): uam_best_tail_cta
 // PACKED: the collision flag is the sign bit of the partial (uam_k_score_groups<8>), part_col is not read.
 // len_path: the paths' length terms from uam_k_bin_hist (the waypoints are then read only when nsamp is asked for).
-template <int BEST, int PACKED>
+// GRAD: also grad: waypoint j = segment j's start share + segment j-1's end share (part_grad, fp32, in that order) + the
+// fp64 length part.
+template <int BEST, int PACKED, bool GRAD = false>
 __global__ void __launch_bounds__(UAM_CTA_THREADS)
 uam_k_reduce_paths(const double2* __restrict__ z, long long B, int Wp, UamRasterParams rp,
                    const float* __restrict__ part_pen, const uint8_t* __restrict__ part_col,
                    const double* __restrict__ len_path, float* __restrict__ cost,
-                   uint8_t* __restrict__ collide, long long* __restrict__ nsamp, UamBestTail tl) {
+                   uint8_t* __restrict__ collide, long long* __restrict__ nsamp, UamBestTail tl,
+                   const float4* __restrict__ part_grad, double2* __restrict__ grad) {
     const int lane = threadIdx.x & 31;
     const long long warp0 = (long long)blockIdx.x * UAM_WARPS_PER_CTA + (threadIdx.x >> 5);
     const long long nwarps = (long long)gridDim.x * UAM_WARPS_PER_CTA;
@@ -1064,6 +1276,19 @@ uam_k_reduce_paths(const double2* __restrict__ z, long long B, int Wp, UamRaster
                 } else {
                     acc[t] += pv[t];
                     col[t] = col[t] || cv[t];
+                }
+                if constexpr (GRAD) {
+                    if (pb + t < B) {
+                        const long long row = (pb + t) * Wp;
+                        const float4 a = part_grad[row + j];
+                        float pu = a.x, pvv = a.y;
+                        if (j >= 1) {
+                            const float4 e = part_grad[row + j - 1];
+                            pu += e.z;
+                            pvv += e.w;
+                        }
+                        grad[row + j] = uam_grad_point(uam_len_grad(z + row, j, N, z[row + j], rp), pu, pvv, N, rp);
+                    }
                 }
                 if (nsamp && pb + t < B) {
                     long long S = 1;
@@ -1531,10 +1756,11 @@ int uam_raster_prepare(uam_ctx* ctx, int64_t B, int N, const double* h_p, int n_
     return UAM_OK;
 }
 
+// d_grad != NULL: the gradient forms of the last two kernels (uam_grad_paths_raster; best must be NULL then)
 template <int TF, int LAYOUT>
 int uam_raster_launch_binned(uam_ctx* ctx, const void* texv, const double2* z, int64_t B, int Wp, const UamRasterParams& rp,
                              float* d_cost, uint8_t* d_collide, long long* d_nsamp, cudaStream_t st, int slot,
-                             const UamBestTail* best, bool* best_done) {
+                             const UamBestTail* best, bool* best_done, double2* d_grad = nullptr) {
     typedef typename UamTexel<TF>::T T;
     const unsigned long long n_seg = (unsigned long long)B * Wp;
     UamBinGeo bg;
@@ -1547,7 +1773,9 @@ int uam_raster_launch_binned(uam_ctx* ctx, const void* texv, const double2* z, i
     bg.hx = (float)(0.5 / rp.dx); bg.hy = (float)(0.5 / rp.dy);
     bg.ox = (float)(-rp.x0 / rp.dx - 0.5); bg.oy = (float)(-rp.y0 / rp.dy - 0.5);
     // scratch: sorted ids (u32) | part_pen (f32) | hist (u32) | cursor (u32) | len_path (f64) | seg_bin (u16) | part_col (u8)
-    const size_t need = n_seg * (4 + 4 + 2 + 1) + (size_t)bg.nbins * 8 + 16 + (size_t)B * 8 + 256;
+    // (+ gradient: part_grad (float4) behind part_col, 16-byte aligned)
+    const size_t need_score = n_seg * (4 + 4 + 2 + 1) + (size_t)bg.nbins * 8 + 16 + (size_t)B * 8 + 256;
+    const size_t need = need_score + (d_grad ? n_seg * 16 + 16 : 0);
     UAM_TRY(uam_reserve(ctx, &ctx->d_bin_scratch[slot], &ctx->bin_scratch_bytes[slot], need));
     unsigned* sorted_id = (unsigned*)ctx->d_bin_scratch[slot];
     float* part_pen = (float*)(sorted_id + n_seg);
@@ -1557,6 +1785,7 @@ int uam_raster_launch_binned(uam_ctx* ctx, const void* texv, const double2* z, i
     double* len_path = (double*)(cursor + bg.nbins);          // (8-byte aligned: n_seg * 8 + nbins * 8 + 16 bytes in)
     unsigned short* seg_bin = (unsigned short*)(len_path + B);
     uint8_t* part_col = (uint8_t*)(seg_bin + n_seg);
+    float4* part_grad = (float4*)(((uintptr_t)(part_col + n_seg) + 15) & ~(uintptr_t)15);
     UAM_NVTX("uam.raster.binned");
     UAM_CUDA(ctx, cudaMemsetAsync(hist, 0, (size_t)(bg.nbins + 4) * 4, st));
     // a CTA of the histogram / scatter kernels owns whole paths: ppc paths = about UAM_BIN_CHUNK segments
@@ -1583,24 +1812,34 @@ int uam_raster_launch_binned(uam_ctx* ctx, const void* texv, const double2* z, i
     const size_t gsmem = (size_t)UAM_GROUP_SMEM * UAM_WARPS_PER_CTA;
     const unsigned long long n_groups = (n_seg + 31) >> 5;        // (< 2^27: segment ids are 32-bit)
     const long long sctas = std::min<long long>((long long)((n_groups + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA), (long long)ctx->sm_count * 16);
-    if (ctx->time_kernels && slot == 0) {
+    const bool timed = ctx->time_kernels && slot == 0 && !d_grad;
+    if (timed) {
         UAM_TRY(uam_time_begin(ctx, st));
     }
     nvtxRangePushA("uam.raster.score");
-    uam_k_score_groups<TF, LAYOUT><<<(unsigned)sctas, UAM_CTA_THREADS, gsmem, st>>>(n_seg, Wp, rp, (const T*)texv, z, sorted_id, part_pen, part_col, next_group);
+    if (d_grad) {
+        const size_t gsmem_g = (size_t)UAM_GROUP_SMEM_GRAD * UAM_WARPS_PER_CTA;
+        UAM_CUDA(ctx, cudaFuncSetAttribute(uam_k_score_groups<TF, LAYOUT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsmem_g));
+        uam_k_score_groups<TF, LAYOUT, true><<<(unsigned)sctas, UAM_CTA_THREADS, gsmem_g, st>>>(n_seg, Wp, rp, (const T*)texv, z, sorted_id, part_pen, part_col,
+                                                                                             next_group, part_grad);
+    } else {
+        uam_k_score_groups<TF, LAYOUT><<<(unsigned)sctas, UAM_CTA_THREADS, gsmem, st>>>(n_seg, Wp, rp, (const T*)texv, z, sorted_id, part_pen, part_col, next_group, nullptr);
+    }
     nvtxRangePop();
     UAM_CHECK_LAUNCH(ctx, "uam_k_score_groups");
-    if (ctx->time_kernels && slot == 0) {
+    if (timed) {
         UAM_TRY(uam_time_end(ctx, st));
     }
     const long long rctas = std::min<long long>((B + 4 * UAM_WARPS_PER_CTA - 1) / (4 * UAM_WARPS_PER_CTA), (long long)ctx->sm_count * 16);   // 4 paths per warp and trip
     UAM_NVTX("uam.raster.reduce+best");
     const bool packed = TF == 8 && rp.w0 >= 0.0f;       // the condition uam_k_score_groups tests
     const UamBestTail tl = best ? *best : UamBestTail{};
-    if (best && packed) uam_k_reduce_paths<1, 1><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl);
-    else if (best) uam_k_reduce_paths<1, 0><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl);
-    else if (packed) uam_k_reduce_paths<0, 1><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl);
-    else uam_k_reduce_paths<0, 0><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl);
+    if (d_grad && packed) uam_k_reduce_paths<0, 1, true><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, part_grad, d_grad);
+    else if (d_grad) uam_k_reduce_paths<0, 0, true><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, part_grad, d_grad);
+    else if (best && packed) uam_k_reduce_paths<1, 1><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, nullptr, nullptr);
+    else if (best) uam_k_reduce_paths<1, 0><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, nullptr, nullptr);
+    else if (packed) uam_k_reduce_paths<0, 1><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, nullptr, nullptr);
+    else uam_k_reduce_paths<0, 0><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, nullptr, nullptr);
     if (best) *best_done = true;
     UAM_CHECK_LAUNCH(ctx, "uam_k_reduce_paths");
     return UAM_OK;
@@ -1706,7 +1945,7 @@ int uam_raster_launch_t(uam_ctx* ctx, const void* texv, uint64_t tex_key, const 
     if (rp.spc == 0.0) {
       {
         const long long ctas = std::min<long long>((B + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA, (long long)ctx->sm_count * 16);
-        uam_k_score_raster_wp<TF, LAYOUT><<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp);
+        uam_k_score_raster_wp<TF, LAYOUT><<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp, nullptr);
         UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_wp");
         if (timed) {
             UAM_TRY(uam_time_end(ctx, st));
@@ -1731,10 +1970,10 @@ int uam_raster_launch_t(uam_ctx* ctx, const void* texv, uint64_t tex_key, const 
     const long long ctas = std::min<long long>((B + wpc - 1) / wpc, (long long)ctx->sm_count * 16);
     if (rp.variant == 1) {
         if (smem > 48 * 1024) UAM_CUDA(ctx, cudaFuncSetAttribute(uam_k_score_raster_int<TF, LAYOUT, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        uam_k_score_raster_int<TF, LAYOUT, 1><<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp);
+        uam_k_score_raster_int<TF, LAYOUT, 1><<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp, nullptr);
     } else {
         if (smem > 48 * 1024) UAM_CUDA(ctx, cudaFuncSetAttribute(uam_k_score_raster_int<TF, LAYOUT, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        uam_k_score_raster_int<TF, LAYOUT, 0><<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp);
+        uam_k_score_raster_int<TF, LAYOUT, 0><<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp, nullptr);
     }
     UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_int");
     if (timed) {
@@ -1914,7 +2153,72 @@ int uam_raster_precompute(uam_ctx* ctx, UamRasterParams* rp, int64_t B, int N, c
     return UAM_OK;
 }
 
+// The gradient forms of the kernels uam_raster_launch_t would run for the same call (variants 1 and 3 are refused by
+// the caller): waypoint kernel, warp-per-path integral kernel, or the binned pipeline.
+template <int TF, int LAYOUT>
+int uam_raster_grad_launch_t(uam_ctx* ctx, const void* texv, const double2* z, int64_t B, int Wp, const UamRasterParams& rp,
+                             float* d_cost, uint8_t* d_collide, double2* d_grad, cudaStream_t st) {
+    typedef typename UamTexel<TF>::T T;
+    const T* tex = (const T*)texv;
+    if (rp.spc == 0.0) {
+        const long long ctas = std::min<long long>((B + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA, (long long)ctx->sm_count * 16);
+        uam_k_score_raster_wp<TF, LAYOUT, true><<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, nullptr, d_grad);
+        UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_wp");
+        return UAM_OK;
+    }
+    if (rp.variant >= 2 && (unsigned long long)B * Wp < 0xffffffffull) {
+        bool unused = false;
+        return uam_raster_launch_binned<TF, LAYOUT>(ctx, texv, z, B, Wp, rp, d_cost, d_collide, nullptr, st, 0, nullptr, &unused, d_grad);
+    }
+    if constexpr (UamIsQuad<TF>::v) {
+        return uam_fail(ctx, UAM_ERR_STATE, "quad texels are not sampled by the warp-per-path integral kernels");
+    } else {
+        const size_t per_warp = uam_seg_table_bytes(Wp) + (size_t)Wp * sizeof(float4);
+        const size_t budget = 200 * 1024;
+        if (per_warp > budget) return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "N = %d waypoints per path is too many for integral mode", Wp - 2);
+        const int wpc = (int)std::max<size_t>(1, std::min<size_t>(UAM_WARPS_PER_CTA, budget / per_warp));
+        const size_t smem = per_warp * wpc;
+        const long long ctas = std::min<long long>((B + wpc - 1) / wpc, (long long)ctx->sm_count * 16);
+        if (smem > 48 * 1024) UAM_CUDA(ctx, cudaFuncSetAttribute(uam_k_score_raster_int<TF, LAYOUT, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        uam_k_score_raster_int<TF, LAYOUT, 0, true><<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, nullptr, d_grad);
+        UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_int");
+        return UAM_OK;
+    }
+}
+
 }  // namespace
+
+extern "C" int uam_grad_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
+                                     double samples_per_cell, float* d_cost, uint8_t* d_collide, double* d_grad, void* stream) {
+    if (!ctx) return UAM_ERR_INVALID;
+    UamRasterParams rp;
+    UAM_TRY(uam_raster_prepare(ctx, B, N, h_p, n_p, flags, samples_per_cell, &rp));
+    if (B == 0) return UAM_OK;
+    if (!d_z || !d_grad) return uam_fail(ctx, UAM_ERR_INVALID, "paths or gradient pointer is NULL");
+    if (rp.spc > 0.0 && (rp.variant == 1 || rp.variant == 3))
+        return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "integral variant %d has no gradient form (use -1, 0 or 2)", rp.variant);
+    UAM_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = uam_pick_stream(ctx, stream);
+    UAM_TRY(uam_raster_precompute(ctx, &rp, B, N, st));
+    const int Wp = N + 2, lay = ctx->geo.layout;
+    const double2* z = reinterpret_cast<const double2*>(d_z);
+    double2* g = reinterpret_cast<double2*>(d_grad);
+    if (rp.combined) {
+        UamRasterParams rc2 = rp;          // as uam_raster_launch: the weights of an L = 2..3 raster are inside the quads
+        if (ctx->geo.texel_floats == 4) { rc2.w0 = 1.0f; rc2.w1 = 0.0f; rc2.w2 = 0.0f; }
+        rc2.row_stride = rp.row_stride2;
+        if (rp.combined == 2)
+            return lay ? uam_raster_grad_launch_t<8, 1>(ctx, ctx->d_tex_comb, z, B, Wp, rc2, d_cost, d_collide, g, st)
+                       : uam_raster_grad_launch_t<8, 0>(ctx, ctx->d_tex_comb, z, B, Wp, rc2, d_cost, d_collide, g, st);
+        return lay ? uam_raster_grad_launch_t<1, 1>(ctx, ctx->d_tex_comb, z, B, Wp, rc2, d_cost, d_collide, g, st)
+                   : uam_raster_grad_launch_t<1, 0>(ctx, ctx->d_tex_comb, z, B, Wp, rc2, d_cost, d_collide, g, st);
+    }
+    if (ctx->geo.texel_floats == 2)
+        return lay ? uam_raster_grad_launch_t<2, 1>(ctx, ctx->d_tex, z, B, Wp, rp, d_cost, d_collide, g, st)
+                   : uam_raster_grad_launch_t<2, 0>(ctx, ctx->d_tex, z, B, Wp, rp, d_cost, d_collide, g, st);
+    return lay ? uam_raster_grad_launch_t<4, 1>(ctx, ctx->d_tex, z, B, Wp, rp, d_cost, d_collide, g, st)
+               : uam_raster_grad_launch_t<4, 0>(ctx, ctx->d_tex, z, B, Wp, rp, d_cost, d_collide, g, st);
+}
 
 static int uam_score_paths_raster_impl(uam_ctx* ctx, const double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
                                        double samples_per_cell, float* d_cost, uint8_t* d_collide, int64_t* d_nsamples,

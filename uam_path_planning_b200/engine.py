@@ -215,6 +215,30 @@ class Engine:
                                                           float(samples_per_cell), _np_ptr(cost), _np_ptr(col)))
         return cost, col
 
+    def grad_raster(self, Z, N: int, p, flags: int, samples_per_cell: float = 0.0):
+        """Z (B, 2(N+2)) float64 -> (cost f32 (B,), collide u8 (B,), grad f64 (B, 2(N+2))) of the raster cost
+        (uam_grad_paths_raster: cost / collide are score_raster's bits); numpy in -> numpy out, CUDA tensor in -> CUDA
+        tensors out."""
+        import torch
+        p = _f64c(p)
+        N = int(N)
+        host = not _is_tensor(Z)
+        if host:
+            Z = _f64c(Z)
+            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
+                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
+            Z = torch.from_numpy(Z).to(f'cuda:{self.device}')
+        assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+        st = self._tensor_args(Z)
+        B = Z.shape[0]
+        cost = torch.empty(B, dtype=torch.float32, device=Z.device)
+        col = torch.empty(B, dtype=torch.uint8, device=Z.device)
+        grad = torch.empty_like(Z)
+        self._check(self._lib.uam_grad_paths_raster(self._h, C.c_void_p(Z.data_ptr()), B, N, _np_ptr(p), p.size, flags,
+                                                    float(samples_per_cell), C.c_void_p(cost.data_ptr()),
+                                                    C.c_void_p(col.data_ptr()), C.c_void_p(grad.data_ptr()), st))
+        return (cost.cpu().numpy(), col.cpu().numpy(), grad.cpu().numpy()) if host else (cost, col, grad)
+
     def score_raster_best(self, Z, N: int, p, flags: int, samples_per_cell: float, global_offset: int = 0, out=None, key=None):
         """score_raster on a CUDA tensor + the best key of the batch -- of every rank's batch when a peer group is attached
         (attach_peers): the exchange over NVLink peer memory rides in the last kernel of the step.

@@ -88,6 +88,15 @@ class RasterMap:
         p = self.parameter_vector(weights, x_start)
         return self.engine.score_raster(Z, N, p, flags, samples_per_cell, want_nsamples, out)
 
+    def cost_gradient(self, Z, weights: Sequence[float], samples_per_cell: float = 0.0, length_smooth: bool = True,
+                      x_start=None):
+        """(cost, collide, grad) of score_paths' cost for Z (B, 2(N+2)) float64 (numpy or CUDA tensor), arguments as in
+        score_paths.  cost / collide are score_paths' bits; grad (B, 2(N+2)) float64 is d cost / d Z with the per-segment
+        sample counts held fixed (columns 2 .. 2N+1 are the free waypoints; include/uam_b200.h has the definition)."""
+        N = Z.shape[1] // 2 - 2
+        flags = (_lib.UAM_LENGTH_SMOOTH if length_smooth else 0) | (_lib.UAM_OWN_START if x_start is None else 0)
+        return self.engine.grad_raster(Z, N, self.parameter_vector(weights, x_start), flags, samples_per_cell)
+
     def score_paths_best(self, Z, weights: Sequence[float], samples_per_cell: float = 0.0, length_smooth: bool = True,
                          x_start=None, global_offset: int = 0, out=None, key=None):
         """score_paths on a CUDA tensor + the best candidate's key (distributed.decode_key) in the same call; with a peer
