@@ -68,6 +68,15 @@ __device__ __forceinline__ unsigned uam_tex_col(unsigned j) {
     return ((j >> 2) << 4) + ((j & 2u) << 1) + (j & 1u);
 }
 
+// Quad-texel address of cell (i, j): uam_tex_row<4, LAYOUT>(i, rs) + uam_tex_col<4, LAYOUT>(j), the same 32-bit value.  Tiled:
+// 2i = 4 (i >> 1) + 2 (i & 1), so (i >> 1) rs + 2 (i & 1) + 2j - (j & 1) = (i >> 1)(rs - 4) + 2 (i + j) - (j & 1), which the
+// compiler issues in 6 instructions (shift, and, add, shift-add, multiply-add, wide multiply-add) instead of 8.
+template <int LAYOUT>
+__device__ __forceinline__ unsigned uam_quad_index(unsigned i, unsigned j, unsigned rs) {
+    if (LAYOUT == 0) return i * rs + j;
+    return (i >> 1) * (rs - 4u) + ((i + j) << 1) - (j & 1u);
+}
+
 // pixel coordinate of a world coordinate: (x - x0)/dx - 1/2 with a true division (oracle: pixel_coords)
 __device__ __forceinline__ double uam_pix(double x, double x0, double dx) {
     return __dsub_rn(__ddiv_rn(__dsub_rn(x, x0), dx), 0.5);
@@ -152,9 +161,9 @@ __device__ __forceinline__ void uam_tap_load(const typename UamTexel<TF>::T* __r
         uam_cell_frac1_inside(v, i0, t.fy);
     }
     if constexpr (TF == 8) {
-        t.q = __ldg(tex + (uam_tex_row<4, LAYOUT>(i0, rp.row_stride) + uam_tex_col<4, LAYOUT>(j0)));
+        t.q = __ldg(tex + uam_quad_index<LAYOUT>(i0, j0, rp.row_stride));
     } else if constexpr (TF == 1) {
-        t.q = __ldg(tex + (uam_tex_row<4, LAYOUT>(i0, rp.row_stride) + uam_tex_col<4, LAYOUT>(j0)));
+        t.q = __ldg(tex + uam_quad_index<LAYOUT>(i0, j0, rp.row_stride));
         const unsigned ni = (unsigned)i0 + (t.fy >= 0.5f ? 1u : 0u), nj = (unsigned)j0 + (t.fx >= 0.5f ? 1u : 0u);
         t.ow = __ldg(rp.occ_bits + uam_occ_word(ni, nj, rp.occ_blocks_x));
         t.ob = uam_occ_bit(ni, nj);
@@ -1186,8 +1195,12 @@ __device__ __forceinline__ void uam_group_score(const UamRasterParams& rp, const
 
 // GRAD: also part_grad[id] = the segment's share of its two waypoints' penalty gradient (uam_seg_grad); 22.8 KB of shared
 // memory per warp, so one CTA of 8 warps per SM.
+// Scoring form on quad texels: 3 CTAs (24 warps) per SM, up to 80 registers.  At 4 CTAs the 64-register cap made the sample
+// loop spill and re-derive the lane, the shared-memory base and constants inside it (259 instructions per 4 taps against 235);
+// on the C3 shard (B200 at 1000 W) the kernel takes 1.455 ms at 3 CTAs, 1.531 ms at 4 and 1.604 ms at 2
+// (profiles/r03_ab_group_occupancy.txt).
 template <int TF, int LAYOUT, bool GRAD = false>
-__global__ void __launch_bounds__(UAM_CTA_THREADS, GRAD ? 1 : 4)
+__global__ void __launch_bounds__(UAM_CTA_THREADS, GRAD ? 1 : (UamIsQuad<TF>::v ? 3 : 4))
 uam_k_score_groups(unsigned long long n_seg, int Wp, UamRasterParams rp, const typename UamTexel<TF>::T* __restrict__ tex,
                    const double2* __restrict__ z, const unsigned* __restrict__ sorted_id, float* __restrict__ part_pen,
                    uint8_t* __restrict__ part_col, unsigned* __restrict__ next_group, float4* __restrict__ part_grad) {
