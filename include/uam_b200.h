@@ -237,6 +237,33 @@ int uam_score_paths_raster_host(uam_ctx* ctx, const double* h_z, int64_t B, int 
 int uam_grad_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
                           double samples_per_cell, float* d_cost, uint8_t* d_collide, double* d_grad, void* stream);
 
+/* Refine every path of d_z in place by monotone descent on the raster cost of uam_grad_paths_raster (same p, flags and
+ * samples_per_cell), each path with its own step.  "Evaluate Z" below is one gradient launch on the whole batch:
+ * (c f32, k u8, g f64), c / k being uam_score_paths_raster's bits.  Per path, with h = min(|dx|, |dy|) of the raster:
+ *   start: tau = step_cells, accepted = 0, (c, k, g) = evaluate(Z);
+ *   each of the `iterations` trips:
+ *     1. m = max |g| over the free columns 2 .. 2N+1; the path is active iff tau >= min_step_cells, every free g is
+ *        finite, m > 0 and c is finite;
+ *     2. trial Zt: free columns Z - r g with r = (tau h) / m (fp64, rounded multiply, divide, subtract: no waypoint
+ *        moves more than tau cells) for an active path, Zt = Z otherwise; columns 0, 1, 2N+2, 2N+3 are never written;
+ *     3. (ct, kt, gt) = evaluate(Zt) for the whole batch;
+ *     4. accept iff active and kt <= k and ct < c (float32; a NaN ct rejects): Z, c, k, g <- Zt, ct, kt, gt,
+ *        tau <- min(2 tau, max_step_cells), accepted += 1; an active path that is not accepted halves tau.
+ * On return d_z, d_cost and d_collide hold the final Z, c and k (c / k = uam_score_paths_raster's bits for the returned
+ * paths), d_accepted (int32, nullable) the accepted trips.  So a path's (collide, cost) never gets worse, a path that did
+ * not collide never starts to, and a row with NaN or inf in its gradient is left as it was.  The penalty layers carry no
+ * obstacle term: refinement does not steer a colliding path out of an obstacle.  S_k may change along the way (the cost
+ * is piecewise smooth); the accept test uses the scored cost.  Everything after the quad texels are built (see
+ * uam_raster_precompute: the first call for a raster / weights may synchronise) is ordered on `stream`: iterations + 1
+ * gradient launches and as many uam_k_refine_step launches, no host read-back.  Scratch: 48 (N + 2) + 18 bytes per path,
+ * kept by the ctx.  B = 0 is a no-op; iterations < 0, step sizes that are not finite or break
+ * 0 < min_step_cells <= step_cells <= max_step_cells, or a NULL pointer (d_accepted excepted) give UAM_ERR_INVALID; no
+ * raster UAM_ERR_STATE; a forced integral variant 1 or 3 UAM_ERR_UNSUPPORTED, as for the gradient. */
+int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
+                            double samples_per_cell, int iterations, double step_cells, double max_step_cells,
+                            double min_step_cells, float* d_cost, uint8_t* d_collide, int32_t* d_accepted,
+                            void* stream);
+
 /* Scoring + best candidate in one call: as uam_score_paths_raster, and *d_key receives the best key (see uam_best) of the
  * batch -- of ALL ranks' batches when a peer group is attached (uam_peer_attach): the last kernel of the step finds the
  * local min, pushes it into every peer's symmetric block over NVLink and waits for theirs (no separate collective).

@@ -60,6 +60,23 @@ struct UamRasterGeo {
     int tiles_y;
 };
 
+// What the raster kernels of one API call read (uam_score_raster.cu): made by uam_raster_prepare from the call's
+// arguments, completed by uam_raster_precompute.
+struct UamRasterParams {
+    double x0, dx, y0, dy;
+    double ms_x, ms_y;
+    double spc;
+    int H, W;
+    unsigned row_stride;  // tiled layout: texels per tile-row (tiles_x * texels per tile); row-major: W
+    float w0, w1, w2;
+    int flags;
+    int variant;          // integral-mode kernel, decided once per API call from the call's whole batch
+    int combined;         // score on the quad texels (ctx->d_tex_comb, row stride row_stride2): 1 = + bit-plane, 2 = sign-packed
+    unsigned row_stride2;
+    const unsigned* occ_bits;   // quad mode: occupancy bit-plane (uam_occ_word / uam_occ_bit)
+    unsigned occ_blocks_x;      // 32 x 32-cell blocks per block-row of the bit-plane
+};
+
 // ---- best-candidate exchange between the ranks of one box (uam_best.cu) -------------------------------------------
 // One-sided min-reduce of the 8-byte best key over NVLink peer memory: every rank owns a small "symmetric block"
 // (cudaMalloc + CUDA IPC, mapped into every peer process); the tail of the scoring step stores this rank's key into its
@@ -194,6 +211,9 @@ struct uam_ctx {
     void* d_ring_cand[UAM_HOST_PIPE_DEPTH] = {};
     size_t ring_cand_bytes[UAM_HOST_PIPE_DEPTH] = {};
     unsigned long long* d_ring_key[UAM_HOST_PIPE_DEPTH] = {};
+    // raster refinement (uam_refine.cu): trial paths, both gradients and the per-path step state
+    void* d_refine_scratch = nullptr;
+    size_t refine_scratch_bytes = 0;
 };
 
 int uam_fail(uam_ctx* ctx, int code, const char* fmt, ...);
@@ -217,6 +237,14 @@ int uam_best_tail(uam_ctx* ctx, int slot, unsigned long long offset, unsigned lo
 int uam_best_launch(uam_ctx* ctx, const void* d_cost, int cost_is_f64, int64_t B, const UamBestTail& tail, cudaStream_t st);
 int uam_make_candidates_launch(uam_ctx* ctx, const double* d_cand, const double* h_ends, const double* d_disp, int N, int64_t B,
                                double jitter_sigma, uint64_t seed, uint64_t index0, double* d_z, cudaStream_t st);
+// Raster scorer (uam_score_raster.cu), in the three steps of a call: uam_raster_prepare checks the arguments and fills
+// the parameters; uam_raster_precompute builds the quad texels when a batch of this B and N samples them (may
+// synchronise); uam_raster_grad_enqueue then enqueues one gradient launch (uam_grad_paths_raster's kernels) of a batch of
+// the same B and N on `st`, without host synchronisation.  d_cost / d_collide are nullable, d_z and d_grad are not.
+int uam_raster_prepare(uam_ctx* ctx, int64_t B, int N, const double* h_p, int n_p, int flags, double spc, UamRasterParams* rp);
+int uam_raster_precompute(uam_ctx* ctx, UamRasterParams* rp, int64_t B, int N, cudaStream_t st);
+int uam_raster_grad_enqueue(uam_ctx* ctx, const UamRasterParams& rp, const double* d_z, int64_t B, int N, float* d_cost,
+                            uint8_t* d_collide, double* d_grad, cudaStream_t st);
 
 // NVTX range over the rest of the enclosing scope (host side; a no-op costing a few ns when no profiler is attached):
 // upload / bin / score / reduce / exchange phases show up by name on an Nsight Systems timeline

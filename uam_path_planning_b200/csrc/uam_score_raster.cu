@@ -27,21 +27,6 @@
 
 namespace {
 
-struct UamRasterParams {
-    double x0, dx, y0, dy;
-    double ms_x, ms_y;
-    double spc;
-    int H, W;
-    unsigned row_stride;  // tiled layout: texels per tile-row (tiles_x * texels per tile); row-major: W
-    float w0, w1, w2;
-    int flags;
-    int variant;          // integral-mode kernel, decided once per API call from the call's whole batch
-    int combined;         // score on the quad texels (ctx->d_tex_comb, row stride row_stride2): 1 = + bit-plane, 2 = sign-packed
-    unsigned row_stride2;
-    const unsigned* occ_bits;   // quad mode: occupancy bit-plane (uam_occ_word / uam_occ_bit)
-    unsigned occ_blocks_x;      // 32 x 32-cell blocks per block-row of the bit-plane
-};
-
 template <int TF> struct UamTexel;
 template <> struct UamTexel<2> { typedef float2 T; };
 template <> struct UamTexel<4> { typedef float4 T; };
@@ -1739,6 +1724,8 @@ __global__ void uam_k_build_tiles(const typename UamTexel<TF>::T* __restrict__ t
     }
 }
 
+}  // namespace
+
 // ---- host side ---------------------------------------------------------------------------------------------------
 int uam_raster_prepare(uam_ctx* ctx, int64_t B, int N, const double* h_p, int n_p, int flags, double spc,
                        UamRasterParams* rp) {
@@ -1768,6 +1755,8 @@ int uam_raster_prepare(uam_ctx* ctx, int64_t B, int N, const double* h_p, int n_
     rp->row_stride2 = 0;
     return UAM_OK;
 }
+
+namespace {
 
 // d_grad != NULL: the gradient forms of the last two kernels (uam_grad_paths_raster; best must be NULL then)
 template <int TF, int LAYOUT>
@@ -2156,6 +2145,8 @@ int uam_raster_launch(uam_ctx* ctx, const double* d_z, int64_t B, int N, const U
     return UAM_OK;
 }
 
+}  // namespace
+
 // Once per API call, before any chunk is launched: make the quad texels if this call will use them.
 int uam_raster_precompute(uam_ctx* ctx, UamRasterParams* rp, int64_t B, int N, cudaStream_t st) {
     // large batches: integral mode through the binned pipelines, waypoint mode when the batch is worth the one-off build
@@ -2165,6 +2156,8 @@ int uam_raster_precompute(uam_ctx* ctx, UamRasterParams* rp, int64_t B, int N, c
     }
     return UAM_OK;
 }
+
+namespace {
 
 // The gradient forms of the kernels uam_raster_launch_t would run for the same call (variants 1 and 3 are refused by
 // the caller): waypoint kernel, warp-per-path integral kernel, or the binned pipeline.
@@ -2213,6 +2206,11 @@ extern "C" int uam_grad_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B,
     UAM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = uam_pick_stream(ctx, stream);
     UAM_TRY(uam_raster_precompute(ctx, &rp, B, N, st));
+    return uam_raster_grad_enqueue(ctx, rp, d_z, B, N, d_cost, d_collide, d_grad, st);
+}
+
+int uam_raster_grad_enqueue(uam_ctx* ctx, const UamRasterParams& rp, const double* d_z, int64_t B, int N, float* d_cost,
+                            uint8_t* d_collide, double* d_grad, cudaStream_t st) {
     const int Wp = N + 2, lay = ctx->geo.layout;
     const double2* z = reinterpret_cast<const double2*>(d_z);
     double2* g = reinterpret_cast<double2*>(d_grad);

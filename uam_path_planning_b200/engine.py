@@ -239,6 +239,36 @@ class Engine:
                                                     C.c_void_p(col.data_ptr()), C.c_void_p(grad.data_ptr()), st))
         return (cost.cpu().numpy(), col.cpu().numpy(), grad.cpu().numpy()) if host else (cost, col, grad)
 
+    def refine_raster(self, Z, N: int, p, flags: int, samples_per_cell: float, iterations: int, step_cells: float,
+                      max_step_cells: float, min_step_cells: float):
+        """Z (B, 2(N+2)) float64 -> (Z_out f64, cost f32 (B,), collide u8 (B,), accepted i32 (B,)) of
+        uam_refine_paths_raster; numpy in -> numpy out, CUDA tensor in -> new CUDA tensors out (Z is not modified)."""
+        import torch
+        p = _f64c(p)
+        N = int(N)
+        host = not _is_tensor(Z)
+        if host:
+            Z = _f64c(Z)
+            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
+                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
+            Zo = torch.from_numpy(Z).to(f'cuda:{self.device}')
+        else:
+            assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+            self._tensor_args(Z)
+            Zo = Z.clone()
+        st = self._tensor_args(Zo)
+        B = Zo.shape[0]
+        cost = torch.empty(B, dtype=torch.float32, device=Zo.device)
+        col = torch.empty(B, dtype=torch.uint8, device=Zo.device)
+        acc = torch.empty(B, dtype=torch.int32, device=Zo.device)
+        self._check(self._lib.uam_refine_paths_raster(
+            self._h, C.c_void_p(Zo.data_ptr()), B, N, _np_ptr(p), p.size, flags, float(samples_per_cell), int(iterations),
+            float(step_cells), float(max_step_cells), float(min_step_cells), C.c_void_p(cost.data_ptr()),
+            C.c_void_p(col.data_ptr()), C.c_void_p(acc.data_ptr()), st))
+        if host:
+            return Zo.cpu().numpy(), cost.cpu().numpy(), col.cpu().numpy(), acc.cpu().numpy()
+        return Zo, cost, col, acc
+
     def score_raster_best(self, Z, N: int, p, flags: int, samples_per_cell: float, global_offset: int = 0, out=None, key=None):
         """score_raster on a CUDA tensor + the best key of the batch -- of every rank's batch when a peer group is attached
         (attach_peers): the exchange over NVLink peer memory rides in the last kernel of the step.
