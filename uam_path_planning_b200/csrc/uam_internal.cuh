@@ -67,12 +67,11 @@ struct UamRasterParams {
     double ms_x, ms_y;
     double spc;
     int H, W;
-    unsigned row_stride;  // tiled layout: texels per tile-row (tiles_x * texels per tile); row-major: W
-    float w0, w1, w2;
+    unsigned row_stride;  // tiled layout: texels per tile-row (tiles_x * texels per tile); row-major: W (of the quads if combined)
+    float w0, w1, w2;     // combined with L = 2..3: {1, 0, 0}, the weights are inside the quads
     int flags;
     int variant;          // integral-mode kernel, decided once per API call from the call's whole batch
-    int combined;         // score on the quad texels (ctx->d_tex_comb, row stride row_stride2): 1 = + bit-plane, 2 = sign-packed
-    unsigned row_stride2;
+    int combined;         // score on the quad texels (ctx->d_tex_comb): 1 = + bit-plane, 2 = sign-packed
     const unsigned* occ_bits;   // quad mode: occupancy bit-plane (uam_occ_word / uam_occ_bit)
     unsigned occ_blocks_x;      // 32 x 32-cell blocks per block-row of the bit-plane
 };
@@ -241,7 +240,10 @@ int uam_make_candidates_launch(uam_ctx* ctx, const double* d_cand, const double*
 // the parameters; uam_raster_precompute builds the quad texels when a batch of this B and N samples them (may
 // synchronise); uam_raster_grad_enqueue then enqueues one gradient launch (uam_grad_paths_raster's kernels) of a batch of
 // the same B and N on `st`, without host synchronisation.  d_cost / d_collide are nullable, d_z and d_grad are not.
+// uam_raster_grad_supported refuses the integral variants without a gradient form (1 and 3); a gradient call checks it
+// before uam_raster_precompute.
 int uam_raster_prepare(uam_ctx* ctx, int64_t B, int N, const double* h_p, int n_p, int flags, double spc, UamRasterParams* rp);
+int uam_raster_grad_supported(uam_ctx* ctx, const UamRasterParams& rp);
 int uam_raster_precompute(uam_ctx* ctx, UamRasterParams* rp, int64_t B, int N, cudaStream_t st);
 int uam_raster_grad_enqueue(uam_ctx* ctx, const UamRasterParams& rp, const double* d_z, int64_t B, int N, float* d_cost,
                             uint8_t* d_collide, double* d_grad, cudaStream_t st);

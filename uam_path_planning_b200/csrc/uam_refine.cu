@@ -134,8 +134,7 @@ extern "C" int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int
     UAM_TRY(uam_raster_prepare(ctx, B, N, h_p, n_p, flags, samples_per_cell, &rp));
     if (B == 0) return UAM_OK;
     if (!d_z || !d_cost || !d_collide) return uam_fail(ctx, UAM_ERR_INVALID, "paths, cost or collide pointer is NULL");
-    if (rp.spc > 0.0 && (rp.variant == 1 || rp.variant == 3))
-        return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "integral variant %d has no gradient form (use -1, 0 or 2)", rp.variant);
+    UAM_TRY(uam_raster_grad_supported(ctx, rp));
     UAM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = uam_pick_stream(ctx, stream);
     UAM_NVTX("uam.raster.refine");

@@ -20,10 +20,14 @@
 // penalty sums are fp32; the length term is fp64.  Sums finish with warp-shuffle reductions in a fixed order
 // (bit-reproducible; no floating-point atomics).
 #include <algorithm>
+#include <type_traits>
 
 #include "uam_internal.cuh"
 
 #define UAM_MAX_SAMPLES_PER_SEGMENT 1048576.0   // cap on S_k (a segment never spans more cells than this)
+// B * (N + 2) from which a batch is large: the auto integral variant is the binned pipeline, and waypoint mode is worth
+// the one-off build of the quad texels
+#define UAM_LARGE_BATCH_SEGMENTS 262144ull
 
 namespace {
 
@@ -219,33 +223,6 @@ __device__ __forceinline__ void uam_tap_grad(const UamRasterParams& rp, const Ua
 
 // true where the clamp of a pixel coordinate to [0, n-1] is inactive (the sample moves with its waypoint)
 __device__ __forceinline__ bool uam_free_coord(double u, int n) { return u >= 0.0 && u <= (double)(n - 1); }
-
-// Weighted bilinear penalty + nearest-cell occupancy at pixel coordinates (u, v): one lane fetches all 4 texels.
-template <int TF, int LAYOUT>
-__device__ __forceinline__ void uam_sample(const typename UamTexel<TF>::T* __restrict__ tex, const UamRasterParams& rp,
-                                           double u, double v, float& pen, bool& occ) {
-    int i0, j0;
-    float fx, fy;
-    uam_cell_frac1(u, rp.W, j0, fx);
-    uam_cell_frac1(v, rp.H, i0, fy);
-    const bool right = fx >= 0.5f, down = fy >= 0.5f;
-    const unsigned r0 = uam_tex_row<TF, LAYOUT>(i0, rp.row_stride), r1 = uam_tex_row<TF, LAYOUT>(i0 + 1, rp.row_stride);
-    const unsigned c0 = uam_tex_col<TF, LAYOUT>(j0), c1 = uam_tex_col<TF, LAYOUT>(j0 + 1);
-    if constexpr (TF == 2) {
-        const float2* t2 = reinterpret_cast<const float2*>(tex);
-        const float2 a = __ldg(t2 + r0 + c0), b = __ldg(t2 + r0 + c1), c = __ldg(t2 + r1 + c0), d = __ldg(t2 + r1 + c1);
-        pen = rp.w0 * uam_lerp2(a.x, b.x, c.x, d.x, fx, fy);
-        const float o = down ? (right ? d.y : c.y) : (right ? b.y : a.y);
-        occ = o != 0.0f;
-    } else {
-        const float4* t4 = reinterpret_cast<const float4*>(tex);
-        const float4 a = __ldg(t4 + r0 + c0), b = __ldg(t4 + r0 + c1), c = __ldg(t4 + r1 + c0), d = __ldg(t4 + r1 + c1);
-        pen = rp.w0 * uam_lerp2(a.x, b.x, c.x, d.x, fx, fy) + rp.w1 * uam_lerp2(a.y, b.y, c.y, d.y, fx, fy) +
-              rp.w2 * uam_lerp2(a.z, b.z, c.z, d.z, fx, fy);
-        const float o = down ? (right ? d.w : c.w) : (right ? b.w : a.w);
-        occ = o != 0.0f;
-    }
-}
 
 // Lane-pair form: the two lanes of a pair work on the SAME sample; lane `side` (0 = left, 1 = right) fetches the
 // texel column j0 + side (rows i0 and i0 + 1), lerps it in y, and the pair exchanges the column results with one
@@ -1750,9 +1727,8 @@ int uam_raster_prepare(uam_ctx* ctx, int64_t B, int N, const double* h_p, int n_
     rp->flags = flags;
     // auto (-1): the binned pipeline pays off once the batch has enough segments to fill the raster bins.  Decided
     // from the whole call (not per pipeline chunk), so host-buffer and device-buffer calls run the same kernels.
-    rp->variant = ctx->int_variant >= 0 ? ctx->int_variant : ((unsigned long long)B * (N + 2) >= 262144ull ? 2 : 0);
+    rp->variant = ctx->int_variant >= 0 ? ctx->int_variant : ((unsigned long long)B * (N + 2) >= UAM_LARGE_BATCH_SEGMENTS ? 2 : 0);
     rp->combined = 0;
-    rp->row_stride2 = 0;
     return UAM_OK;
 }
 
@@ -1836,12 +1812,11 @@ int uam_raster_launch_binned(uam_ctx* ctx, const void* texv, const double2* z, i
     UAM_NVTX("uam.raster.reduce+best");
     const bool packed = TF == 8 && rp.w0 >= 0.0f;       // the condition uam_k_score_groups tests
     const UamBestTail tl = best ? *best : UamBestTail{};
-    if (d_grad && packed) uam_k_reduce_paths<0, 1, true><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, part_grad, d_grad);
-    else if (d_grad) uam_k_reduce_paths<0, 0, true><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, part_grad, d_grad);
-    else if (best && packed) uam_k_reduce_paths<1, 1><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, nullptr, nullptr);
-    else if (best) uam_k_reduce_paths<1, 0><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, nullptr, nullptr);
-    else if (packed) uam_k_reduce_paths<0, 1><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, nullptr, nullptr);
-    else uam_k_reduce_paths<0, 0><<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl, nullptr, nullptr);
+    const auto reduce = d_grad ? (packed ? uam_k_reduce_paths<0, 1, true> : uam_k_reduce_paths<0, 0, true>)
+                      : best   ? (packed ? uam_k_reduce_paths<1, 1> : uam_k_reduce_paths<1, 0>)
+                               : (packed ? uam_k_reduce_paths<0, 1> : uam_k_reduce_paths<0, 0>);
+    reduce<<<(unsigned)rctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, part_pen, part_col, len_path, d_cost, d_collide, d_nsamp, tl,
+                                                        d_grad ? part_grad : nullptr, d_grad);
     if (best) *best_done = true;
     UAM_CHECK_LAUNCH(ctx, "uam_k_reduce_paths");
     return UAM_OK;
@@ -1931,58 +1906,54 @@ int uam_raster_launch_tiles(uam_ctx* ctx, const void* texv, uint64_t tex_key, co
     return UAM_OK;
 }
 
-template <int TF, int LAYOUT>
+// One launch of the scorer (GRAD = false) or of its gradient (GRAD = true, uam_grad_paths_raster) on texels of form TF:
+// the waypoint kernel, the warp-per-path integral kernel or the binned pipeline.  Integral variants 1 and 3 have no
+// gradient form (uam_raster_grad_supported refuses them first).  The scorer's dominant kernel is timed for slot 0.
+template <int TF, int LAYOUT, bool GRAD>
 int uam_raster_launch_t(uam_ctx* ctx, const void* texv, uint64_t tex_key, const double2* z, int64_t B, int Wp,
-                        const UamRasterParams& rp, float* d_cost, uint8_t* d_collide, long long* d_nsamp, cudaStream_t st, int slot,
-                        const UamBestTail* best, bool* best_done) {
+                        const UamRasterParams& rp, float* d_cost, uint8_t* d_collide, long long* d_nsamp, double2* d_grad,
+                        cudaStream_t st, int slot, const UamBestTail* best, bool* best_done) {
     typedef typename UamTexel<TF>::T T;
     const T* tex = (const T*)texv;
-    const bool timed = ctx->time_kernels && slot == 0 && !(rp.spc > 0.0 && rp.variant >= 2);
-    if (timed) {
-        UAM_TRY(uam_time_begin(ctx, st));
-    }
-    if constexpr (UamIsQuad<TF>::v) {
-        if (rp.spc > 0.0 && rp.variant < 2) return uam_fail(ctx, UAM_ERR_STATE, "quad texels are not sampled by the warp-per-path integral kernels");
-    }
+    const bool timed = !GRAD && ctx->time_kernels && slot == 0;
     if (rp.spc == 0.0) {
-      {
         const long long ctas = std::min<long long>((B + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA, (long long)ctx->sm_count * 16);
-        uam_k_score_raster_wp<TF, LAYOUT><<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp, nullptr);
+        if (timed) UAM_TRY(uam_time_begin(ctx, st));
+        uam_k_score_raster_wp<TF, LAYOUT, GRAD><<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp, d_grad);
         UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_wp");
-        if (timed) {
-            UAM_TRY(uam_time_end(ctx, st));
-        }
-      }
+        if (timed) UAM_TRY(uam_time_end(ctx, st));
         return UAM_OK;
     }
     if (rp.variant >= 2 && (unsigned long long)B * Wp < 0xffffffffull) {
-        if (rp.variant == 3 && (rp.W + UAM_TS - 1) / UAM_TS + (rp.H + UAM_TS - 1) / UAM_TS < 65535) {
-            bool fell_back = false;
-            UAM_TRY((uam_raster_launch_tiles<TF, LAYOUT>(ctx, texv, tex_key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, &fell_back)));
-            if (!fell_back) return UAM_OK;
+        if constexpr (!GRAD) {
+            if (rp.variant == 3 && (rp.W + UAM_TS - 1) / UAM_TS + (rp.H + UAM_TS - 1) / UAM_TS < 65535) {
+                bool fell_back = false;
+                UAM_TRY((uam_raster_launch_tiles<TF, LAYOUT>(ctx, texv, tex_key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, &fell_back)));
+                if (!fell_back) return UAM_OK;
+            }
         }
-        return uam_raster_launch_binned<TF, LAYOUT>(ctx, texv, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, best, best_done);
+        return uam_raster_launch_binned<TF, LAYOUT>(ctx, texv, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, best, best_done, d_grad);
     }
-  if constexpr (!UamIsQuad<TF>::v) {
-    const size_t per_warp = uam_seg_table_bytes(Wp);
-    const size_t budget = 200 * 1024;
-    if (per_warp > budget) return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "N = %d waypoints per path is too many for integral mode", Wp - 2);
-    const int wpc = (int)std::max<size_t>(1, std::min<size_t>(UAM_WARPS_PER_CTA, budget / per_warp));
-    const size_t smem = per_warp * wpc;
-    const long long ctas = std::min<long long>((B + wpc - 1) / wpc, (long long)ctx->sm_count * 16);
-    if (rp.variant == 1) {
-        if (smem > 48 * 1024) UAM_CUDA(ctx, cudaFuncSetAttribute(uam_k_score_raster_int<TF, LAYOUT, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        uam_k_score_raster_int<TF, LAYOUT, 1><<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp, nullptr);
+    if constexpr (UamIsQuad<TF>::v) {
+        return uam_fail(ctx, UAM_ERR_STATE, "quad texels are not sampled by the warp-per-path integral kernels");
     } else {
-        if (smem > 48 * 1024) UAM_CUDA(ctx, cudaFuncSetAttribute(uam_k_score_raster_int<TF, LAYOUT, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        uam_k_score_raster_int<TF, LAYOUT, 0><<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp, nullptr);
+        const size_t per_warp = uam_seg_table_bytes(Wp) + (GRAD ? (size_t)Wp * sizeof(float4) : 0);
+        const size_t budget = 200 * 1024;
+        if (per_warp > budget) return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "N = %d waypoints per path is too many for integral mode", Wp - 2);
+        const int wpc = (int)std::max<size_t>(1, std::min<size_t>(UAM_WARPS_PER_CTA, budget / per_warp));
+        const size_t smem = per_warp * wpc;
+        const long long ctas = std::min<long long>((B + wpc - 1) / wpc, (long long)ctx->sm_count * 16);
+        auto kernel = uam_k_score_raster_int<TF, LAYOUT, 0, GRAD>;
+        if constexpr (!GRAD) {
+            if (rp.variant == 1) kernel = uam_k_score_raster_int<TF, LAYOUT, 1>;
+        }
+        if (smem > 48 * 1024) UAM_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (timed) UAM_TRY(uam_time_begin(ctx, st));
+        kernel<<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, d_nsamp, d_grad);
+        UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_int");
+        if (timed) UAM_TRY(uam_time_end(ctx, st));
+        return UAM_OK;
     }
-    UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_int");
-    if (timed) {
-        UAM_TRY(uam_time_end(ctx, st));
-    }
-  }
-    return UAM_OK;
 }
 
 // Quad texels for the large-batch integral pipelines (variants 2 and 3), whose gather is bound by the number of load
@@ -2080,12 +2051,13 @@ int uam_build_quads_t(uam_ctx* ctx, const UamRasterParams& rp, unsigned rs_q, si
     return UAM_OK;
 }
 
+// Makes the quad texels of the raster and rp's weights (unless the last ones still fit), then points rp at them: the row
+// stride becomes the quads', and the weights of an L = 2..3 raster, now inside the quads, become {1, 0, 0}.
 int uam_ensure_quads(uam_ctx* ctx, UamRasterParams* rp, cudaStream_t st) {
     const int W = rp->W, H = rp->H, lay = ctx->geo.layout, tf = ctx->geo.texel_floats;
     const int tiles_x = (W + 3) / 4, tiles_y = (H + 1) / 2;
     const unsigned rs_q = lay ? (unsigned)tiles_x * 8u : (unsigned)W;
     const unsigned blocks_x = (unsigned)(W + 31) / 32u, blocks_y = (unsigned)(H + 31) / 32u;
-    rp->row_stride2 = rs_q;
     rp->occ_blocks_x = blocks_x;
     const bool same_w = tf == 2 || (ctx->comb_w[0] == rp->w0 && ctx->comb_w[1] == rp->w1 && ctx->comb_w[2] == rp->w2);
     if (!(ctx->comb_valid && same_w)) {
@@ -2106,41 +2078,41 @@ int uam_ensure_quads(uam_ctx* ctx, UamRasterParams* rp, cudaStream_t st) {
     }
     rp->occ_bits = (const unsigned*)ctx->d_occ_bits + 4;
     rp->combined = ctx->comb_packed ? 2 : 1;
+    rp->row_stride = rs_q;
+    if (tf == 4) { rp->w0 = 1.0f; rp->w1 = 0.0f; rp->w2 = 0.0f; }
     return UAM_OK;
 }
 
-// slot: which scratch buffer of the ctx the binned pipeline may use (0 = caller-stream calls, 1.. = host pipeline stages).
-// best (nullable): also find the best candidate of the launch (fused into the last kernel of the binned pipeline; one more
-// small kernel behind the other scorers).
+// One launch of the scorer or of its gradient on the texels the call samples: the quad texels when
+// uam_raster_precompute made them for it (rp.combined = 1: + occupancy bit-plane, 2: sign-packed), the raster's own
+// otherwise.  slot: which scratch buffer of the ctx the binned pipeline may use (0 = caller-stream calls, 1.. = host
+// pipeline stages).  best (nullable, scorer only): also find the best candidate of the launch, which the binned pipeline
+// fuses into its last kernel and then reports in *best_done.
+template <bool GRAD>
+int uam_raster_dispatch(uam_ctx* ctx, const UamRasterParams& rp, const double* d_z, int64_t B, int N, float* d_cost,
+                        uint8_t* d_collide, long long* d_nsamp, double* d_grad, cudaStream_t st, int slot,
+                        const UamBestTail* best, bool* best_done) {
+    const int Wp = N + 2, lay = ctx->geo.layout;
+    const double2* z = reinterpret_cast<const double2*>(d_z);
+    double2* g = reinterpret_cast<double2*>(d_grad);
+    const void* tex = rp.combined ? ctx->d_tex_comb : ctx->d_tex;
+    const uint64_t key = rp.combined ? (ctx->comb_gen << 1) | 1u : ctx->raster_gen << 1;
+    auto launch = [&](auto form) {
+        constexpr int TF = decltype(form)::value;
+        return lay ? uam_raster_launch_t<TF, 1, GRAD>(ctx, tex, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, g, st, slot, best, best_done)
+                   : uam_raster_launch_t<TF, 0, GRAD>(ctx, tex, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, g, st, slot, best, best_done);
+    };
+    if (rp.combined == 2) return launch(std::integral_constant<int, 8>());
+    if (rp.combined) return launch(std::integral_constant<int, 1>());
+    if (ctx->geo.texel_floats == 2) return launch(std::integral_constant<int, 2>());
+    return launch(std::integral_constant<int, 4>());
+}
+
 int uam_raster_launch(uam_ctx* ctx, const double* d_z, int64_t B, int N, const UamRasterParams& rp, float* d_cost,
                       uint8_t* d_collide, long long* d_nsamp, cudaStream_t st, int slot, const UamBestTail* best = nullptr) {
-    const int Wp = N + 2;
-    const double2* z = reinterpret_cast<const double2*>(d_z);
-    const int tf = ctx->geo.texel_floats, lay = ctx->geo.layout;
-    const uint64_t key = ctx->raster_gen << 1;
-    bool best_done = false;
-    int rc;
     if (best && !d_cost) return uam_fail(ctx, UAM_ERR_INVALID, "the best-candidate key needs the cost output");
-    if (rp.combined) {
-        // large-batch integral mode on the quad texels (made by uam_raster_precompute)
-        UamRasterParams rc2 = rp;
-        if (tf == 4) { rc2.w0 = 1.0f; rc2.w1 = 0.0f; rc2.w2 = 0.0f; }     // the weights are inside the quads
-        rc2.row_stride = rp.row_stride2;
-        const uint64_t ckey = (ctx->comb_gen << 1) | 1u;
-        if (rp.combined == 2)
-            rc = lay ? uam_raster_launch_t<8, 1>(ctx, ctx->d_tex_comb, ckey, z, B, Wp, rc2, d_cost, d_collide, d_nsamp, st, slot, best, &best_done)
-                     : uam_raster_launch_t<8, 0>(ctx, ctx->d_tex_comb, ckey, z, B, Wp, rc2, d_cost, d_collide, d_nsamp, st, slot, best, &best_done);
-        else
-            rc = lay ? uam_raster_launch_t<1, 1>(ctx, ctx->d_tex_comb, ckey, z, B, Wp, rc2, d_cost, d_collide, d_nsamp, st, slot, best, &best_done)
-                     : uam_raster_launch_t<1, 0>(ctx, ctx->d_tex_comb, ckey, z, B, Wp, rc2, d_cost, d_collide, d_nsamp, st, slot, best, &best_done);
-    } else if (tf == 2) {
-        rc = lay ? uam_raster_launch_t<2, 1>(ctx, ctx->d_tex, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, best, &best_done)
-                 : uam_raster_launch_t<2, 0>(ctx, ctx->d_tex, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, best, &best_done);
-    } else {
-        rc = lay ? uam_raster_launch_t<4, 1>(ctx, ctx->d_tex, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, best, &best_done)
-                 : uam_raster_launch_t<4, 0>(ctx, ctx->d_tex, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, best, &best_done);
-    }
-    UAM_TRY(rc);
+    bool best_done = false;
+    UAM_TRY(uam_raster_dispatch<false>(ctx, rp, d_z, B, N, d_cost, d_collide, d_nsamp, nullptr, st, slot, best, &best_done));
     if (best && !best_done) UAM_TRY(uam_best_launch(ctx, d_cost, 0, B, *best, st));
     return UAM_OK;
 }
@@ -2150,49 +2122,23 @@ int uam_raster_launch(uam_ctx* ctx, const double* d_z, int64_t B, int N, const U
 // Once per API call, before any chunk is launched: make the quad texels if this call will use them.
 int uam_raster_precompute(uam_ctx* ctx, UamRasterParams* rp, int64_t B, int N, cudaStream_t st) {
     // large batches: integral mode through the binned pipelines, waypoint mode when the batch is worth the one-off build
-    const bool big_wp = rp->spc == 0.0 && (unsigned long long)B * (N + 2) >= 262144ull;
+    const bool big_wp = rp->spc == 0.0 && (unsigned long long)B * (N + 2) >= UAM_LARGE_BATCH_SEGMENTS;
     if (((rp->spc > 0.0 && rp->variant >= 2) || big_wp) && ctx->combine_layers && (unsigned long long)B * (N + 2) < 0xffffffffull) {
         UAM_TRY(uam_ensure_quads(ctx, rp, st));
     }
     return UAM_OK;
 }
 
-namespace {
-
-// The gradient forms of the kernels uam_raster_launch_t would run for the same call (variants 1 and 3 are refused by
-// the caller): waypoint kernel, warp-per-path integral kernel, or the binned pipeline.
-template <int TF, int LAYOUT>
-int uam_raster_grad_launch_t(uam_ctx* ctx, const void* texv, const double2* z, int64_t B, int Wp, const UamRasterParams& rp,
-                             float* d_cost, uint8_t* d_collide, double2* d_grad, cudaStream_t st) {
-    typedef typename UamTexel<TF>::T T;
-    const T* tex = (const T*)texv;
-    if (rp.spc == 0.0) {
-        const long long ctas = std::min<long long>((B + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA, (long long)ctx->sm_count * 16);
-        uam_k_score_raster_wp<TF, LAYOUT, true><<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, nullptr, d_grad);
-        UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_wp");
-        return UAM_OK;
-    }
-    if (rp.variant >= 2 && (unsigned long long)B * Wp < 0xffffffffull) {
-        bool unused = false;
-        return uam_raster_launch_binned<TF, LAYOUT>(ctx, texv, z, B, Wp, rp, d_cost, d_collide, nullptr, st, 0, nullptr, &unused, d_grad);
-    }
-    if constexpr (UamIsQuad<TF>::v) {
-        return uam_fail(ctx, UAM_ERR_STATE, "quad texels are not sampled by the warp-per-path integral kernels");
-    } else {
-        const size_t per_warp = uam_seg_table_bytes(Wp) + (size_t)Wp * sizeof(float4);
-        const size_t budget = 200 * 1024;
-        if (per_warp > budget) return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "N = %d waypoints per path is too many for integral mode", Wp - 2);
-        const int wpc = (int)std::max<size_t>(1, std::min<size_t>(UAM_WARPS_PER_CTA, budget / per_warp));
-        const size_t smem = per_warp * wpc;
-        const long long ctas = std::min<long long>((B + wpc - 1) / wpc, (long long)ctx->sm_count * 16);
-        if (smem > 48 * 1024) UAM_CUDA(ctx, cudaFuncSetAttribute(uam_k_score_raster_int<TF, LAYOUT, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        uam_k_score_raster_int<TF, LAYOUT, 0, true><<<(unsigned)ctas, wpc * 32, smem, st>>>(z, B, Wp, rp, tex, d_cost, d_collide, nullptr, d_grad);
-        UAM_CHECK_LAUNCH(ctx, "uam_k_score_raster_int");
-        return UAM_OK;
-    }
+int uam_raster_grad_supported(uam_ctx* ctx, const UamRasterParams& rp) {
+    if (rp.spc > 0.0 && (rp.variant == 1 || rp.variant == 3))
+        return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "integral variant %d has no gradient form (use -1, 0 or 2)", rp.variant);
+    return UAM_OK;
 }
 
-}  // namespace
+int uam_raster_grad_enqueue(uam_ctx* ctx, const UamRasterParams& rp, const double* d_z, int64_t B, int N, float* d_cost,
+                            uint8_t* d_collide, double* d_grad, cudaStream_t st) {
+    return uam_raster_dispatch<true>(ctx, rp, d_z, B, N, d_cost, d_collide, nullptr, d_grad, st, 0, nullptr, nullptr);
+}
 
 extern "C" int uam_grad_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
                                      double samples_per_cell, float* d_cost, uint8_t* d_collide, double* d_grad, void* stream) {
@@ -2201,34 +2147,11 @@ extern "C" int uam_grad_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B,
     UAM_TRY(uam_raster_prepare(ctx, B, N, h_p, n_p, flags, samples_per_cell, &rp));
     if (B == 0) return UAM_OK;
     if (!d_z || !d_grad) return uam_fail(ctx, UAM_ERR_INVALID, "paths or gradient pointer is NULL");
-    if (rp.spc > 0.0 && (rp.variant == 1 || rp.variant == 3))
-        return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "integral variant %d has no gradient form (use -1, 0 or 2)", rp.variant);
+    UAM_TRY(uam_raster_grad_supported(ctx, rp));
     UAM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = uam_pick_stream(ctx, stream);
     UAM_TRY(uam_raster_precompute(ctx, &rp, B, N, st));
     return uam_raster_grad_enqueue(ctx, rp, d_z, B, N, d_cost, d_collide, d_grad, st);
-}
-
-int uam_raster_grad_enqueue(uam_ctx* ctx, const UamRasterParams& rp, const double* d_z, int64_t B, int N, float* d_cost,
-                            uint8_t* d_collide, double* d_grad, cudaStream_t st) {
-    const int Wp = N + 2, lay = ctx->geo.layout;
-    const double2* z = reinterpret_cast<const double2*>(d_z);
-    double2* g = reinterpret_cast<double2*>(d_grad);
-    if (rp.combined) {
-        UamRasterParams rc2 = rp;          // as uam_raster_launch: the weights of an L = 2..3 raster are inside the quads
-        if (ctx->geo.texel_floats == 4) { rc2.w0 = 1.0f; rc2.w1 = 0.0f; rc2.w2 = 0.0f; }
-        rc2.row_stride = rp.row_stride2;
-        if (rp.combined == 2)
-            return lay ? uam_raster_grad_launch_t<8, 1>(ctx, ctx->d_tex_comb, z, B, Wp, rc2, d_cost, d_collide, g, st)
-                       : uam_raster_grad_launch_t<8, 0>(ctx, ctx->d_tex_comb, z, B, Wp, rc2, d_cost, d_collide, g, st);
-        return lay ? uam_raster_grad_launch_t<1, 1>(ctx, ctx->d_tex_comb, z, B, Wp, rc2, d_cost, d_collide, g, st)
-                   : uam_raster_grad_launch_t<1, 0>(ctx, ctx->d_tex_comb, z, B, Wp, rc2, d_cost, d_collide, g, st);
-    }
-    if (ctx->geo.texel_floats == 2)
-        return lay ? uam_raster_grad_launch_t<2, 1>(ctx, ctx->d_tex, z, B, Wp, rp, d_cost, d_collide, g, st)
-                   : uam_raster_grad_launch_t<2, 0>(ctx, ctx->d_tex, z, B, Wp, rp, d_cost, d_collide, g, st);
-    return lay ? uam_raster_grad_launch_t<4, 1>(ctx, ctx->d_tex, z, B, Wp, rp, d_cost, d_collide, g, st)
-               : uam_raster_grad_launch_t<4, 0>(ctx, ctx->d_tex, z, B, Wp, rp, d_cost, d_collide, g, st);
 }
 
 static int uam_score_paths_raster_impl(uam_ctx* ctx, const double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
@@ -2317,11 +2240,7 @@ static int uam_raster_submit_impl(uam_ctx* ctx, const double* h_z, const double*
     float* d_cost = (float*)ctx->d_stage_out[s];
     uint8_t* d_col = (uint8_t*)(d_cost + B);
     // the quad texels are shared by all slots: (re)built here, before anything of this submission is queued
-    {
-        const uint64_t gen0 = ctx->comb_gen;
-        UAM_TRY(uam_raster_precompute(ctx, &rp, B, N, st));
-        (void)gen0;
-    }
+    UAM_TRY(uam_raster_precompute(ctx, &rp, B, N, st));
     if (h_cand) {
         UAM_TRY(uam_reserve(ctx, &ctx->d_ring_cand[s], &ctx->ring_cand_bytes[s], (size_t)B * 5 * sizeof(double)));
         UAM_CUDA(ctx, cudaMemcpyAsync(ctx->d_ring_cand[s], h_cand, (size_t)B * 5 * sizeof(double), cudaMemcpyHostToDevice, st));
