@@ -264,6 +264,41 @@ int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int N, const d
                             double min_step_cells, float* d_cost, uint8_t* d_collide, int32_t* d_accepted,
                             void* stream);
 
+/* Swept check of whole path segments against the raster's occupancy, and each path's clearance.  The scorer above only
+ * looks at its samples; this call looks at every cell a segment crosses.  For every path of d_z (B, 2(N+2)) and every
+ * segment k = 0 .. N (z_k -> z_{k+1}):
+ *   1. pixel coordinates U = (x - x0)/dx - 0.5, V = (y - y0)/dy - 0.5 in fp64, in the scorer's order (round-to-nearest
+ *      divide, then subtract, no FMA): oracle.pixel_coords before its clamp.  Cell (i, j) has its centre at (U, V) = (j, i)
+ *      and its square is [j - 1/2, j + 1/2] x [i - 1/2, i + 1/2].
+ *   2. fixed point: Uq = rint(U 2^16), Vq = rint(V 2^16) (int64, ties to even).  A path with a non-finite coordinate or with
+ *      |U| or |V| >= 2^31 gets flags = UAM_SWEEP_INVALID and nothing else is evaluated for it: first hit = -1, d2min = -1.
+ *   3. a raster cell (0 <= i < H, 0 <= j < W) is touched by a segment iff the closed quantised segment meets the cell's
+ *      closed square dilated by one quantum: in fixed-point units the box [(2j-1) 2^15 - 1, (2j+1) 2^15 + 1] in u, likewise
+ *      in v.  Exact integer arithmetic (128-bit products of 48-bit differences): a zero-length segment touches the cells
+ *      around its point, a segment along a cell edge touches both sides, one through a grid vertex all four cells.
+ *   4. per path:
+ *      d_flags (uint8):         UAM_SWEEP_HIT: some segment touches an occupied cell;
+ *                               UAM_SWEEP_OUTSIDE: some waypoint lies outside the closed raster rectangle
+ *                               [-1/2, W-1/2] x [-1/2, H-1/2] (only raster cells are ever tested, the part outside is not
+ *                               judged); UAM_SWEEP_INVALID: see 2.
+ *      d_first_hit (int32, nullable): the lowest k whose segment touches an occupied cell, -1 if none.
+ *      d_d2min (int32, nullable):     min over all touched cells of min(d2, 65535), d2 = squared distance in cells from the
+ *                               cell's centre to the nearest occupied cell's centre (uam_edt's d_dist2: 0 on occupied
+ *                               cells); -1 when no raster cell is touched.  65535 means "at least 256 cells".  In map units
+ *                               the clearance is sqrt(d2min) |dx| when |dx| = |dy|.
+ * The one-quantum dilation covers the scorer's rounding (quantisation moves an endpoint by <= 2^-17 cell, the scorer's fp64
+ * samples lie within ~1e-11 cell of the segment, its nearest-cell choice on an fp32 fraction is off by <= 2^-24), so for a
+ * path inside the raster rectangle uam_score_paths_raster's collide flag (any samples_per_cell) implies UAM_SWEEP_HIT.
+ * Stream-ordered on `stream`, no host read-back; a path's outputs do not depend on the rest of the batch.  Uses the ctx's
+ * current raster: the occupancy bit-plane (flags, first hit) and, for d_d2min only, a uint16 field of min(d2, 65535) made
+ * with uam_edt (2 B per cell kept, ~26 B per cell of scratch while it is built) are built on the first call after each
+ * raster upload and kept; that first call may synchronise.  B = 0 is a no-op; N < 0 or a NULL d_z / d_flags give
+ * UAM_ERR_INVALID; no raster UAM_ERR_STATE; d_d2min on a raster over 23170 cells per side UAM_ERR_UNSUPPORTED (uam_edt's
+ * limit; flags and first hit work at any size). */
+enum { UAM_SWEEP_HIT = 1, UAM_SWEEP_OUTSIDE = 2, UAM_SWEEP_INVALID = 4 };
+int uam_sweep_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
+                           int32_t* d_d2min, void* stream);
+
 /* Scoring + best candidate in one call: as uam_score_paths_raster, and *d_key receives the best key (see uam_best) of the
  * batch -- of ALL ranks' batches when a peer group is attached (uam_peer_attach): the last kernel of the step finds the
  * local min, pushes it into every peer's symmetric block over NVLink and waits for theirs (no separate collective).

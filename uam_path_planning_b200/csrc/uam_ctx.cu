@@ -260,6 +260,7 @@ extern "C" int uam_ctx_destroy(uam_ctx* ctx) {
     cudaFree(ctx->d_tex_comb);
     cudaFree(ctx->d_occ_bits);
     cudaFree(ctx->d_refine_scratch);
+    cudaFree(ctx->d_sweep_d2);
     for (int i = 0; i < UAM_HOST_PIPE_DEPTH; ++i) {
         cudaFree(ctx->d_stage_in[i]);
         cudaFree(ctx->d_stage_out[i]);

@@ -187,7 +187,7 @@ struct uam_ctx {
     void* d_tex_comb = nullptr;
     size_t tex_comb_bytes = 0;
     bool comb_valid = false;
-    void* d_occ_bits = nullptr;
+    void* d_occ_bits = nullptr;         // 4 words (uam_build_quads_t's flag) + the bit-plane (uam_ensure_occ_bits)
     size_t occ_bits_bytes = 0;
     bool occ_bits_valid = false;
     bool comb_packed = false;           // quads carry the occupancy flags in their sign bits
@@ -213,6 +213,10 @@ struct uam_ctx {
     // raster refinement (uam_refine.cu): trial paths, both gradients and the per-path step state
     void* d_refine_scratch = nullptr;
     size_t refine_scratch_bytes = 0;
+    // swept path check (uam_sweep.cu): min(EDT d^2, 65535) per cell (H, W) uint16 of the raster of generation sweep_d2_gen
+    void* d_sweep_d2 = nullptr;
+    size_t sweep_d2_bytes = 0;
+    uint64_t sweep_d2_gen = 0;          // 0: none (raster_gen counts uploads from 1)
 };
 
 int uam_fail(uam_ctx* ctx, int code, const char* fmt, ...);
@@ -247,6 +251,17 @@ int uam_raster_grad_supported(uam_ctx* ctx, const UamRasterParams& rp);
 int uam_raster_precompute(uam_ctx* ctx, UamRasterParams* rp, int64_t B, int N, cudaStream_t st);
 int uam_raster_grad_enqueue(uam_ctx* ctx, const UamRasterParams& rp, const double* d_z, int64_t B, int N, float* d_cost,
                             uint8_t* d_collide, double* d_grad, cudaStream_t st);
+
+// Occupancy bit-plane of the current raster: one bit per cell, a 32-bit word = 8 x 4 cells, a 128-byte line = 4 x 8 words
+// = a 32 x 32-cell block (8192^2 cells = 8 MiB: L2-resident, mostly L1-resident along a path).  It sits at word 4 of
+// ctx->d_occ_bits.  uam_ensure_occ_bits builds it from the texels on first use after each raster upload and synchronises
+// `st` when it does, so every stream may read it afterwards (quad texels of the scorer, uam_sweep_paths_raster).
+int uam_ensure_occ_bits(uam_ctx* ctx, cudaStream_t st);
+inline unsigned uam_occ_words(int H, int W) { return (unsigned)((W + 31) / 32) * (unsigned)((H + 31) / 32) * 32u; }
+__host__ __device__ __forceinline__ unsigned uam_occ_word(unsigned i, unsigned j, unsigned blocks_x) {
+    return ((i >> 5) * blocks_x + (j >> 5)) * 32u + ((i >> 2) & 7u) * 4u + ((j >> 3) & 3u);
+}
+__host__ __device__ __forceinline__ unsigned uam_occ_bit(unsigned i, unsigned j) { return (i & 3u) * 8u + (j & 7u); }
 
 // NVTX range over the rest of the enclosing scope (host side; a no-op costing a few ns when no profiler is attached):
 // upload / bin / score / reduce / exchange phases show up by name on an Nsight Systems timeline
@@ -455,6 +470,12 @@ __device__ __forceinline__ unsigned long long uam_cta_min_key(unsigned long long
     if (threadIdx.x == 0)
         for (int i = 1; i < (int)((blockDim.x + 31) >> 5); ++i) k = s_k[i] < k ? s_k[i] : k;
     return k;
+}
+
+// pixel coordinate of a world coordinate: (x - x0)/dx - 1/2 with a true division (oracle: pixel_coords); the raster scorer's
+// and the swept check's
+__device__ __forceinline__ double uam_pix(double x, double x0, double dx) {
+    return __dsub_rn(__ddiv_rn(__dsub_rn(x, x0), dx), 0.5);
 }
 
 __device__ __forceinline__ float uam_warp_sum(float v) {

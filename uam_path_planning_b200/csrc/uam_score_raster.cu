@@ -66,11 +66,6 @@ __device__ __forceinline__ unsigned uam_quad_index(unsigned i, unsigned j, unsig
     return (i >> 1) * (rs - 4u) + ((i + j) << 1) - (j & 1u);
 }
 
-// pixel coordinate of a world coordinate: (x - x0)/dx - 1/2 with a true division (oracle: pixel_coords)
-__device__ __forceinline__ double uam_pix(double x, double x0, double dx) {
-    return __dsub_rn(__ddiv_rn(__dsub_rn(x, x0), dx), 0.5);
-}
-
 __device__ __forceinline__ double uam_norm2r(double dx, double dy) {
     return sqrt(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
 }
@@ -108,13 +103,6 @@ __device__ __forceinline__ void uam_cell_frac1_inside(double u, int& j0, float& 
     j0 = __double2loint(fu);
     f = (float)__dsub_rn(u, __dsub_rn(fu, 4503599627370496.0));
 }
-
-// Occupancy bit-plane of the quad mode: one bit per cell, a 32-bit word = 8 x 4 cells, a 128-byte line = 4 x 8 words
-// = a 32 x 32-cell block (8192^2 cells = 8 MiB: L2-resident, mostly L1-resident along a path).
-__host__ __device__ __forceinline__ unsigned uam_occ_word(unsigned i, unsigned j, unsigned blocks_x) {
-    return ((i >> 5) * blocks_x + (j >> 5)) * 32u + ((i >> 2) & 7u) * 4u + ((j >> 3) & 3u);
-}
-__host__ __device__ __forceinline__ unsigned uam_occ_bit(unsigned i, unsigned j) { return (i & 3u) * 8u + (j & 7u); }
 
 // A bilinear tap split into its load half and its arithmetic half, so that a loop can issue the loads of several
 // samples before it consumes the first one.
@@ -2024,8 +2012,7 @@ __global__ void uam_k_build_occ_bits(const typename UamTexel<TF>::T* __restrict_
 }
 
 template <int TF, int LAYOUT>
-int uam_build_quads_t(uam_ctx* ctx, const UamRasterParams& rp, unsigned rs_q, size_t n_out, unsigned blocks_x, unsigned n_words,
-                      cudaStream_t st) {
+int uam_build_quads_t(uam_ctx* ctx, const UamRasterParams& rp, unsigned rs_q, size_t n_out, cudaStream_t st) {
     typedef typename UamTexel<TF>::T T;
     // first choice: sign-packed quads (no second load per tap); the flag word sits in front of the bit-plane
     unsigned* bad = (unsigned*)ctx->d_occ_bits;
@@ -2039,12 +2026,7 @@ int uam_build_quads_t(uam_ctx* ctx, const UamRasterParams& rp, unsigned rs_q, si
     ctx->comb_packed = !h_bad && !ctx->no_sign_pack;
     if (ctx->comb_packed) return UAM_OK;
     // negative (or NaN) values somewhere: plain quads + occupancy bit-plane
-    if (!ctx->occ_bits_valid) {
-        uam_k_build_occ_bits<TF, LAYOUT><<<(n_words + 255) / 256, 256, 0, st>>>((const T*)ctx->d_tex, rp.H, rp.W, rp.row_stride, blocks_x, n_words,
-                                                                               (unsigned*)ctx->d_occ_bits + 4);
-        UAM_CHECK_LAUNCH(ctx, "uam_k_build_occ_bits");
-        ctx->occ_bits_valid = true;
-    }
+    UAM_TRY(uam_ensure_occ_bits(ctx, st));
     uam_k_build_quads<TF, LAYOUT, 0><<<ctx->sm_count * 8, 256, 0, st>>>((const T*)ctx->d_tex, rp.H, rp.W, rp.row_stride, rs_q, rp.w0, rp.w1, rp.w2,
                                                                          n_out, (float4*)ctx->d_tex_comb, bad);
     UAM_CHECK_LAUNCH(ctx, "uam_k_build_quads");
@@ -2057,20 +2039,16 @@ int uam_ensure_quads(uam_ctx* ctx, UamRasterParams* rp, cudaStream_t st) {
     const int W = rp->W, H = rp->H, lay = ctx->geo.layout, tf = ctx->geo.texel_floats;
     const int tiles_x = (W + 3) / 4, tiles_y = (H + 1) / 2;
     const unsigned rs_q = lay ? (unsigned)tiles_x * 8u : (unsigned)W;
-    const unsigned blocks_x = (unsigned)(W + 31) / 32u, blocks_y = (unsigned)(H + 31) / 32u;
-    rp->occ_blocks_x = blocks_x;
+    rp->occ_blocks_x = (unsigned)(W + 31) / 32u;
     const bool same_w = tf == 2 || (ctx->comb_w[0] == rp->w0 && ctx->comb_w[1] == rp->w1 && ctx->comb_w[2] == rp->w2);
     if (!(ctx->comb_valid && same_w)) {
         UAM_NVTX("uam.raster.build_quads");
         const size_t n_out = lay ? (size_t)tiles_x * tiles_y * 8 : (size_t)H * W;
-        const unsigned n_words = blocks_x * blocks_y * 32u;
         UAM_CUDA(ctx, cudaDeviceSynchronize());      // kernels on other streams may still read the old quads
         UAM_TRY(uam_reserve(ctx, &ctx->d_tex_comb, &ctx->tex_comb_bytes, n_out * sizeof(float4)));
-        UAM_TRY(uam_reserve(ctx, &ctx->d_occ_bits, &ctx->occ_bits_bytes, (size_t)(n_words + 4) * 4));
-        if (tf == 2) UAM_TRY(lay ? (uam_build_quads_t<2, 1>(ctx, *rp, rs_q, n_out, blocks_x, n_words, st))
-                                 : (uam_build_quads_t<2, 0>(ctx, *rp, rs_q, n_out, blocks_x, n_words, st)));
-        else UAM_TRY(lay ? (uam_build_quads_t<4, 1>(ctx, *rp, rs_q, n_out, blocks_x, n_words, st))
-                         : (uam_build_quads_t<4, 0>(ctx, *rp, rs_q, n_out, blocks_x, n_words, st)));
+        UAM_TRY(uam_reserve(ctx, &ctx->d_occ_bits, &ctx->occ_bits_bytes, (size_t)(uam_occ_words(H, W) + 4) * 4));
+        if (tf == 2) UAM_TRY(lay ? (uam_build_quads_t<2, 1>(ctx, *rp, rs_q, n_out, st)) : (uam_build_quads_t<2, 0>(ctx, *rp, rs_q, n_out, st)));
+        else UAM_TRY(lay ? (uam_build_quads_t<4, 1>(ctx, *rp, rs_q, n_out, st)) : (uam_build_quads_t<4, 0>(ctx, *rp, rs_q, n_out, st)));
         UAM_CUDA(ctx, cudaStreamSynchronize(st));    // every pipeline stream may use them from now on
         ctx->comb_valid = true;
         ctx->comb_w[0] = rp->w0; ctx->comb_w[1] = rp->w1; ctx->comb_w[2] = rp->w2;
@@ -2118,6 +2096,24 @@ int uam_raster_launch(uam_ctx* ctx, const double* d_z, int64_t B, int N, const U
 }
 
 }  // namespace
+
+int uam_ensure_occ_bits(uam_ctx* ctx, cudaStream_t st) {
+    if (ctx->occ_bits_valid) return UAM_OK;
+    const int H = ctx->geo.H, W = ctx->geo.W, lay = ctx->geo.layout, tf = ctx->geo.texel_floats;
+    const unsigned n_words = uam_occ_words(H, W), blocks_x = (unsigned)(W + 31) / 32u;
+    const unsigned rs = (unsigned)(lay ? ctx->geo.tiles_x * (tf == 4 ? 8 : 16) : W);    // the raster's own texels
+    UAM_TRY(uam_reserve(ctx, &ctx->d_occ_bits, &ctx->occ_bits_bytes, (size_t)(n_words + 4) * 4));
+    unsigned* bits = (unsigned*)ctx->d_occ_bits + 4;
+    const unsigned grid = (n_words + 255) / 256;
+    if (tf == 2 && lay) uam_k_build_occ_bits<2, 1><<<grid, 256, 0, st>>>((const float2*)ctx->d_tex, H, W, rs, blocks_x, n_words, bits);
+    else if (tf == 2) uam_k_build_occ_bits<2, 0><<<grid, 256, 0, st>>>((const float2*)ctx->d_tex, H, W, rs, blocks_x, n_words, bits);
+    else if (lay) uam_k_build_occ_bits<4, 1><<<grid, 256, 0, st>>>((const float4*)ctx->d_tex, H, W, rs, blocks_x, n_words, bits);
+    else uam_k_build_occ_bits<4, 0><<<grid, 256, 0, st>>>((const float4*)ctx->d_tex, H, W, rs, blocks_x, n_words, bits);
+    UAM_CHECK_LAUNCH(ctx, "uam_k_build_occ_bits");
+    UAM_CUDA(ctx, cudaStreamSynchronize(st));
+    ctx->occ_bits_valid = true;
+    return UAM_OK;
+}
 
 // Once per API call, before any chunk is launched: make the quad texels if this call will use them.
 int uam_raster_precompute(uam_ctx* ctx, UamRasterParams* rp, int64_t B, int N, cudaStream_t st) {

@@ -120,6 +120,28 @@ class RasterMap:
         return self.engine.refine_raster(Z, N, self.parameter_vector(weights, x_start), flags, samples_per_cell, iterations,
                                          step_cells, max_step_cells, min_step_cells)
 
+    def sweep_paths(self, Z, clearance: bool = True):
+        """Check every cell each segment of Z (B, 2(N+2)) float64 crosses against the occupancy -> (flags, first_hit,
+        d2min); numpy in -> numpy out, a CUDA tensor in -> CUDA tensors out.  score_paths only looks at its samples.
+
+        Segment k runs from z_k to z_{k+1} (k = 0 .. N).  In pixel coordinates U = (x - x0)/dx - 0.5, V = (y - y0)/dy - 0.5
+        (fp64, the scorer's), quantised to 2^-16 cell, a raster cell is touched by a segment iff the closed segment meets
+        the cell's closed square dilated by one quantum (exact integer test: a segment along a cell edge touches both
+        sides, one through a grid vertex all four cells, a zero-length one the cells around its point).
+          flags (uint8): 1 = some segment touches an occupied cell (HIT), 2 = some waypoint lies outside the raster
+                         rectangle [-1/2, W-1/2] x [-1/2, H-1/2] (only raster cells are judged), 4 = a coordinate is not
+                         finite or |U| or |V| >= 2^31 (INVALID: nothing else is evaluated, first_hit = d2min = -1);
+          first_hit (int32): the first segment that touches an occupied cell, -1 if none;
+          d2min (int32, None unless clearance): min over the touched cells of min(d2, 65535), d2 the squared distance in
+                         cells to the nearest occupied cell's centre (0 on an occupied cell, 65535 = 256 cells or more);
+                         -1 when no raster cell is touched.  The clearance in map units is sqrt(d2min) * |dx| when
+                         |dx| = |dy|.
+        For a path inside the raster rectangle, score_paths' collide flag (any samples_per_cell) implies HIT.  The first
+        call with clearance=True after a raster upload runs an EDT of the raster (include/uam_b200.h:
+        uam_sweep_paths_raster); rasters over 23170 cells per side support clearance=False only."""
+        N = Z.shape[1] // 2 - 2
+        return self.engine.sweep_raster(Z, N, True, clearance)
+
     def score_paths_best(self, Z, weights: Sequence[float], samples_per_cell: float = 0.0, length_smooth: bool = True,
                          x_start=None, global_offset: int = 0, out=None, key=None):
         """score_paths on a CUDA tensor + the best candidate's key (distributed.decode_key) in the same call; with a peer
