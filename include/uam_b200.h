@@ -264,6 +264,36 @@ int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int N, const d
                             double min_step_cells, float* d_cost, uint8_t* d_collide, int32_t* d_accepted,
                             void* stream);
 
+/* uam_refine_paths_raster with the swept check (uam_sweep_paths_raster, below) in its accept test, so that refinement
+ * never moves a path into an occupied cell between the scorer's samples, and, with min_d2 > 0, never closer than
+ * sqrt(min_d2) cells to an obstacle.  The rule is exactly uam_refine_paths_raster's (steps 1 - 4 above) with two
+ * additions:
+ *   - "evaluate Z" also runs the swept check on the whole batch: f = its flags (UAM_SWEEP_HIT | OUTSIDE | INVALID) and,
+ *     when the clearance is used (min_d2 > 0 or a non-NULL d_d2min), d2 = its d2min; these are uam_sweep_paths_raster's
+ *     bits;
+ *   - step 4 becomes: accept iff active and kt <= k and ct < c and (ft & ~f) == 0 and
+ *     (min_d2 == 0 or min(d2t, min_d2) >= min(d2, min_d2)) (signed int32: d2 = -1, no raster cell touched, is the
+ *     worst); on accept also f, d2 <- ft, d2t.
+ * So a trial never adds a swept flag the path did not have: a path inside the raster that sweeps clean stays clean,
+ * inside and valid.  A path that is already HIT may still be accepted into collide = 0 while it crosses an occupied
+ * cell: it gains no flag.  With min_d2 > 0 a path's clearance capped at min_d2, min(d2min, min_d2), never decreases: a path
+ * that starts at least sqrt(min_d2) cells from every occupied cell ends so too.  Every trial this call accepts,
+ * uam_refine_paths_raster would have accepted as well; when the swept conditions never reject a trial, the outputs
+ * are bit-identical to it.  On return d_cost / d_collide hold uam_score_paths_raster's bits for the returned paths, as
+ * there, and d_sweep_flags (uint8, required) / d_d2min (int32, nullable) uam_sweep_paths_raster's flags / d2min.
+ * min_d2 is in squared cells, the unit of d2min, in 0 .. 65535.  With d_d2min NULL and min_d2 > 0 the clearance is kept
+ * in scratch; with d_d2min NULL and min_d2 == 0 no clearance is computed.  Each trip adds one sweep launch of the trial
+ * batch after its gradient launch, on `stream`, no host read-back.  The occupancy bit-plane, the d^2 field (clearance
+ * only) and the quad texels are built first when missing (each may synchronise).  Scratch: that of
+ * uam_refine_paths_raster + 1 byte per path, + 4 with the clearance, + 4 more when d_d2min is NULL.  Errors: those of
+ * uam_refine_paths_raster in the same order (min_d2 out of range is UAM_ERR_INVALID with the step sizes, a NULL
+ * d_sweep_flags with the other pointers); then UAM_ERR_UNSUPPORTED for the clearance on a raster over 23170 cells per
+ * side or an N too large for the sweep's shared-memory table (N <= 3656), both before anything is built or reserved. */
+int uam_refine_paths_raster_swept(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
+                                  double samples_per_cell, int iterations, double step_cells, double max_step_cells,
+                                  double min_step_cells, int min_d2, float* d_cost, uint8_t* d_collide,
+                                  int32_t* d_accepted, uint8_t* d_sweep_flags, int32_t* d_d2min, void* stream);
+
 /* Swept check of whole path segments against the raster's occupancy, and each path's clearance.  The scorer above only
  * looks at its samples; this call looks at every cell a segment crosses.  For every path of d_z (B, 2(N+2)) and every
  * segment k = 0 .. N (z_k -> z_{k+1}):

@@ -55,6 +55,8 @@ SIGNATURES = {
     'uam_score_paths_raster_host': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _vp, _vp]),
     'uam_grad_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _vp, _vp, _vp, _vp]),
     'uam_refine_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _i, _d, _d, _d, _vp, _vp, _vp, _vp]),
+    'uam_refine_paths_raster_swept': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _i, _d, _d, _d, _i, _vp, _vp, _vp, _vp,
+                                           _vp, _vp]),
     'uam_sweep_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     'uam_eval_points': (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     'uam_eval_points_host': (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp]),

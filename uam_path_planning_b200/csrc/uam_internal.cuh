@@ -263,6 +263,16 @@ __host__ __device__ __forceinline__ unsigned uam_occ_word(unsigned i, unsigned j
 }
 __host__ __device__ __forceinline__ unsigned uam_occ_bit(unsigned i, unsigned j) { return (i & 3u) * 8u + (j & 7u); }
 
+// Swept check (uam_sweep.cu), in the steps of a call: uam_sweep_supported refuses an N whose segment table does not fit
+// in shared memory and, with the clearance, a raster beyond uam_edt's limit; uam_ensure_occ_bits and, with the
+// clearance, uam_sweep_ensure_d2 build the fields (both may synchronise: call them before enqueueing work that must
+// stay ordered); uam_sweep_enqueue then enqueues one uam_k_sweep_paths launch on `st`, without host synchronisation.
+// d_first_hit / d_d2min are nullable; d_d2min needs the d^2 field.
+int uam_sweep_supported(uam_ctx* ctx, int N, bool clearance);
+int uam_sweep_ensure_d2(uam_ctx* ctx, cudaStream_t st);
+int uam_sweep_enqueue(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
+                      int32_t* d_d2min, cudaStream_t st);
+
 // NVTX range over the rest of the enclosing scope (host side; a no-op costing a few ns when no profiler is attached):
 // upload / bin / score / reduce / exchange phases show up by name on an Nsight Systems timeline
 struct UamNvtxRange {

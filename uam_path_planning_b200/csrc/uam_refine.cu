@@ -7,6 +7,9 @@
 // evaluated and writes the next one.  The loop is stream-ordered: no host synchronisation or read-back per trip, and
 // every path is evaluated on every trip (a path's bits do not depend on the rest of the batch, and the kernel choice
 // stays the one of the call's B).
+//
+// uam_refine_paths_raster_swept adds one uam_k_sweep_paths launch of the trial batch per trip (uam_sweep_enqueue) and
+// the swept terms of the accept test (UAM_REFINE_SWEPT); everything else is the same loop.
 #include <algorithm>
 #include <cmath>
 
@@ -19,6 +22,7 @@ enum : int {
     UAM_REFINE_START = 1,      // tau = step_cells, accepted = 0 (first launch, after the gradient of Z)
     UAM_REFINE_ACCEPT = 2,     // take or drop the trial in zt, evaluated into (ct, kt, gt)
     UAM_REFINE_PROPOSE = 4,    // write the next trial into zt and whether it moved the path into active
+    UAM_REFINE_SWEPT = 8,      // the accept test also needs the trial's swept flags (ft) and clearance (d2t)
 };
 
 struct UamRefineState {
@@ -37,6 +41,13 @@ struct UamRefineState {
     int Wp;
     double h;                 // cell size: min(|dx|, |dy|)
     double step, max_step, min_step;
+    // UAM_REFINE_SWEPT: swept flags and clearance at z (the caller's outputs or scratch) and at zt; d2 / d2t are NULL
+    // when no clearance is computed, min_d2 > 0 only with them
+    uint8_t* f;
+    const uint8_t* ft;
+    int32_t* d2;
+    const int32_t* d2t;
+    int min_d2;
 };
 
 __device__ __forceinline__ double uam_warp_max(double v) {
@@ -64,12 +75,26 @@ __global__ void __launch_bounds__(UAM_CTA_THREADS) uam_k_refine_step(const UamRe
             kt = s.kt[b];
             take = was_active && kt <= s.k[b] && ct < c;
         }
+        uint8_t ft = 0;
+        int d2t = 0;
+        if (MODE & UAM_REFINE_SWEPT) {
+            ft = s.ft[b];
+            take = take && (ft & ~s.f[b]) == 0;
+            if (s.d2) {
+                d2t = s.d2t[b];
+                take = take && (s.min_d2 == 0 || min(d2t, s.min_d2) >= min(s.d2[b], s.min_d2));
+            }
+        }
         __syncwarp();                  // every lane has read the per-path scalars before lane 0 overwrites them
         if (MODE & UAM_REFINE_ACCEPT) {
             if (take) {
                 c = ct;
                 tau = fmin(2.0 * tau, s.max_step);
                 if (lane == 0) { s.c[b] = ct; s.k[b] = kt; s.accepted[b] += 1; }
+                if ((MODE & UAM_REFINE_SWEPT) && lane == 0) {
+                    s.f[b] = ft;
+                    if (s.d2) s.d2[b] = d2t;
+                }
             } else if (was_active) {
                 tau = 0.5 * tau;
             }
@@ -120,31 +145,40 @@ int uam_refine_step_launch(uam_ctx* ctx, const UamRefineState& s, cudaStream_t s
 
 }  // namespace
 
-extern "C" int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
-                                       double samples_per_cell, int iterations, double step_cells, double max_step_cells,
-                                       double min_step_cells, float* d_cost, uint8_t* d_collide, int32_t* d_accepted,
-                                       void* stream) {
+// Both entry points: swept = uam_refine_paths_raster_swept (min_d2, d_sweep_flags and d_d2min are only read then).
+static int uam_refine_run(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
+                          double samples_per_cell, int iterations, double step_cells, double max_step_cells,
+                          double min_step_cells, float* d_cost, uint8_t* d_collide, int32_t* d_accepted, bool swept,
+                          int min_d2, uint8_t* d_sweep_flags, int32_t* d_d2min, void* stream) {
     if (!ctx) return UAM_ERR_INVALID;
     if (iterations < 0) return uam_fail(ctx, UAM_ERR_INVALID, "iterations must be >= 0 (got %d)", iterations);
     if (!(std::isfinite(step_cells) && std::isfinite(max_step_cells) && std::isfinite(min_step_cells) && min_step_cells > 0.0 &&
           min_step_cells <= step_cells && step_cells <= max_step_cells))
         return uam_fail(ctx, UAM_ERR_INVALID, "step sizes must be finite with 0 < min <= step <= max (got %g, %g, %g)",
                         min_step_cells, step_cells, max_step_cells);
+    if (swept && (min_d2 < 0 || min_d2 > 65535)) return uam_fail(ctx, UAM_ERR_INVALID, "min_d2 must be in 0 .. 65535 (got %d)", min_d2);
     UamRasterParams rp;
     UAM_TRY(uam_raster_prepare(ctx, B, N, h_p, n_p, flags, samples_per_cell, &rp));
     if (B == 0) return UAM_OK;
     if (!d_z || !d_cost || !d_collide) return uam_fail(ctx, UAM_ERR_INVALID, "paths, cost or collide pointer is NULL");
+    if (swept && !d_sweep_flags) return uam_fail(ctx, UAM_ERR_INVALID, "sweep flags pointer is NULL");
     UAM_TRY(uam_raster_grad_supported(ctx, rp));
+    const bool clearance = swept && (min_d2 > 0 || d_d2min);
+    if (swept) UAM_TRY(uam_sweep_supported(ctx, N, clearance));
     UAM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = uam_pick_stream(ctx, stream);
-    UAM_NVTX("uam.raster.refine");
+    UAM_NVTX(swept ? "uam.raster.refine_swept" : "uam.raster.refine");
+    if (swept) UAM_TRY(uam_ensure_occ_bits(ctx, st));
+    if (clearance) UAM_TRY(uam_sweep_ensure_d2(ctx, st));
     UAM_TRY(uam_raster_precompute(ctx, &rp, B, N, st));
 
     // scratch: zt | g | gt (B x Wp double2 each) | tau (f64) | ct (f32) | accepted (i32, when the caller passes none) |
-    // kt (u8) | active (u8)
+    // [d2t (i32) | d2 (i32, when the caller passes none): clearance] | kt (u8) | active (u8) | [ft (u8): swept]
     const int Wp = N + 2;
     const size_t n = (size_t)B * Wp;
-    UAM_TRY(uam_reserve(ctx, &ctx->d_refine_scratch, &ctx->refine_scratch_bytes, 3 * n * sizeof(double2) + (size_t)B * 18));
+    const size_t swept_bytes = swept ? (size_t)B * (1 + (clearance ? 4 : 0) + (clearance && !d_d2min ? 4 : 0)) : 0;
+    UAM_TRY(uam_reserve(ctx, &ctx->d_refine_scratch, &ctx->refine_scratch_bytes,
+                        3 * n * sizeof(double2) + (size_t)B * 18 + swept_bytes));
     UamRefineState s;
     s.zt = (double2*)ctx->d_refine_scratch;
     s.g = s.zt + n;
@@ -154,9 +188,23 @@ extern "C" int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int
     float* ct = (float*)(s.tau + B);
     s.ct = ct;
     int32_t* acc_scratch = (int32_t*)(ct + B);
-    uint8_t* kt = (uint8_t*)(acc_scratch + B);
+    int32_t* i32_end = acc_scratch + B;
+    int32_t* d2t = nullptr;
+    s.d2 = nullptr;
+    if (clearance) {
+        d2t = i32_end;
+        i32_end += B;
+        s.d2 = d_d2min ? d_d2min : i32_end;
+        if (!d_d2min) i32_end += B;
+    }
+    s.d2t = d2t;
+    uint8_t* kt = (uint8_t*)i32_end;
     s.kt = kt;
     s.active = kt + B;
+    uint8_t* ft = swept ? kt + 2 * B : nullptr;
+    s.ft = ft;
+    s.f = d_sweep_flags;
+    s.min_d2 = min_d2;
     s.z = (double2*)d_z;
     s.c = d_cost;
     s.k = d_collide;
@@ -169,15 +217,40 @@ extern "C" int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int
     s.min_step = min_step_cells;
 
     UAM_TRY(uam_raster_grad_enqueue(ctx, rp, d_z, B, N, d_cost, d_collide, (double*)s.g, st));
+    if (swept) UAM_TRY(uam_sweep_enqueue(ctx, d_z, B, N, d_sweep_flags, nullptr, s.d2, st));
     if (iterations == 0) {
         if (d_accepted) UAM_CUDA(ctx, cudaMemsetAsync(d_accepted, 0, (size_t)B * sizeof(int32_t), st));
         return UAM_OK;
     }
     UAM_TRY(uam_refine_step_launch<UAM_REFINE_START | UAM_REFINE_PROPOSE>(ctx, s, st));
     for (int it = 0; it < iterations; ++it) {
+        const bool last = it + 1 == iterations;
         UAM_TRY(uam_raster_grad_enqueue(ctx, rp, (const double*)s.zt, B, N, ct, kt, (double*)gt, st));
-        if (it + 1 < iterations) UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_PROPOSE>(ctx, s, st));
-        else UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT>(ctx, s, st));
+        if (swept) {
+            UAM_TRY(uam_sweep_enqueue(ctx, (const double*)s.zt, B, N, ft, nullptr, d2t, st));
+            if (!last) UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_PROPOSE | UAM_REFINE_SWEPT>(ctx, s, st));
+            else UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_SWEPT>(ctx, s, st));
+        } else {
+            if (!last) UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_PROPOSE>(ctx, s, st));
+            else UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT>(ctx, s, st));
+        }
     }
     return UAM_OK;
+}
+
+extern "C" int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
+                                       double samples_per_cell, int iterations, double step_cells, double max_step_cells,
+                                       double min_step_cells, float* d_cost, uint8_t* d_collide, int32_t* d_accepted,
+                                       void* stream) {
+    return uam_refine_run(ctx, d_z, B, N, h_p, n_p, flags, samples_per_cell, iterations, step_cells, max_step_cells,
+                          min_step_cells, d_cost, d_collide, d_accepted, false, 0, nullptr, nullptr, stream);
+}
+
+extern "C" int uam_refine_paths_raster_swept(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p,
+                                             int flags, double samples_per_cell, int iterations, double step_cells,
+                                             double max_step_cells, double min_step_cells, int min_d2, float* d_cost,
+                                             uint8_t* d_collide, int32_t* d_accepted, uint8_t* d_sweep_flags,
+                                             int32_t* d_d2min, void* stream) {
+    return uam_refine_run(ctx, d_z, B, N, h_p, n_p, flags, samples_per_cell, iterations, step_cells, max_step_cells,
+                          min_step_cells, d_cost, d_collide, d_accepted, true, min_d2, d_sweep_flags, d_d2min, stream);
 }

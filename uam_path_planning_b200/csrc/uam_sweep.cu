@@ -217,6 +217,8 @@ __global__ void uam_k_clip_d2(const int* __restrict__ d2, size_t n, unsigned sho
         out[o] = (unsigned short)min(d2[o], UAM_SWEEP_D2_CLIP);
 }
 
+}  // namespace
+
 // min(EDT d^2, 65535) of the current raster, built once per upload.  The occupancy bytes and the int32 d^2 (5 B per cell)
 // and uam_edt's own scratch (what this build adds to ctx->d_scratch) are freed again; the field itself is 2 B per cell.
 int uam_sweep_ensure_d2(uam_ctx* ctx, cudaStream_t st) {
@@ -253,30 +255,23 @@ int uam_sweep_ensure_d2(uam_ctx* ctx, cudaStream_t st) {
     return rc;
 }
 
-}  // namespace
-
-extern "C" int uam_sweep_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
-                                      int32_t* d_d2min, void* stream) {
-    if (!ctx) return UAM_ERR_INVALID;
-    if (B < 0 || N < 0) return uam_fail(ctx, UAM_ERR_INVALID, "need B >= 0 and N >= 0 (got B=%lld N=%d)", (long long)B, N);
-    if (B == 0) return UAM_OK;
-    if (!d_z || !d_flags) return uam_fail(ctx, UAM_ERR_INVALID, "paths or flags pointer is NULL");
-    if (!ctx->has_raster) return uam_fail(ctx, UAM_ERR_STATE, "no raster: call uam_map_set_raster first");
-    if (d_d2min && (ctx->geo.H > 23170 || ctx->geo.W > 23170))
+int uam_sweep_supported(uam_ctx* ctx, int N, bool clearance) {
+    if (clearance && (ctx->geo.H > 23170 || ctx->geo.W > 23170))
         return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "clearance needs a raster of at most 23170 cells per side (uam_edt's limit)");
     const size_t per_warp = uam_sweep_table_bytes((int)std::min<long long>((long long)N + 1, 1 << 24));
     if (per_warp > UAM_SWEEP_SMEM_BUDGET) return uam_fail(ctx, UAM_ERR_UNSUPPORTED, "N = %d waypoints per path is too many", N);
-    UAM_NVTX("uam.raster.sweep");
-    UAM_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = uam_pick_stream(ctx, stream);
-    UAM_TRY(uam_ensure_occ_bits(ctx, st));
-    if (d_d2min) UAM_TRY(uam_sweep_ensure_d2(ctx, st));
+    return UAM_OK;
+}
+
+int uam_sweep_enqueue(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
+                      int32_t* d_d2min, cudaStream_t st) {
     UamSweepArgs g;
     g.x0 = ctx->geo.x0; g.dx = ctx->geo.dx; g.y0 = ctx->geo.y0; g.dy = ctx->geo.dy;
     g.H = ctx->geo.H; g.W = ctx->geo.W;
     g.occ_bits = (const unsigned*)ctx->d_occ_bits + 4;
     g.blocks_x = (unsigned)(g.W + 31) / 32u;
     g.d2 = d_d2min ? (const unsigned short*)ctx->d_sweep_d2 : nullptr;
+    const size_t per_warp = uam_sweep_table_bytes(N + 1);
     const int wpc = (int)std::max<size_t>(1, std::min<size_t>(UAM_WARPS_PER_CTA, UAM_SWEEP_SMEM_BUDGET / per_warp));
     const size_t smem = per_warp * wpc;
     const long long ctas = std::min<long long>((B + wpc - 1) / wpc, (long long)ctx->sm_count * 16);
@@ -285,4 +280,20 @@ extern "C" int uam_sweep_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B
                                                               d_first_hit, d_d2min);
     UAM_CHECK_LAUNCH(ctx, "uam_k_sweep_paths");
     return UAM_OK;
+}
+
+extern "C" int uam_sweep_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
+                                      int32_t* d_d2min, void* stream) {
+    if (!ctx) return UAM_ERR_INVALID;
+    if (B < 0 || N < 0) return uam_fail(ctx, UAM_ERR_INVALID, "need B >= 0 and N >= 0 (got B=%lld N=%d)", (long long)B, N);
+    if (B == 0) return UAM_OK;
+    if (!d_z || !d_flags) return uam_fail(ctx, UAM_ERR_INVALID, "paths or flags pointer is NULL");
+    if (!ctx->has_raster) return uam_fail(ctx, UAM_ERR_STATE, "no raster: call uam_map_set_raster first");
+    UAM_TRY(uam_sweep_supported(ctx, N, d_d2min != nullptr));
+    UAM_NVTX("uam.raster.sweep");
+    UAM_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = uam_pick_stream(ctx, stream);
+    UAM_TRY(uam_ensure_occ_bits(ctx, st));
+    if (d_d2min) UAM_TRY(uam_sweep_ensure_d2(ctx, st));
+    return uam_sweep_enqueue(ctx, d_z, B, N, d_flags, d_first_hit, d_d2min, st);
 }

@@ -120,6 +120,25 @@ class RasterMap:
         return self.engine.refine_raster(Z, N, self.parameter_vector(weights, x_start), flags, samples_per_cell, iterations,
                                          step_cells, max_step_cells, min_step_cells)
 
+    def refine_paths_swept(self, Z, weights: Sequence[float], samples_per_cell: float = 0.0, iterations: int = 20,
+                           length_smooth: bool = True, x_start=None, step_cells: float = 1.0, max_step_cells: float = 64.0,
+                           min_step_cells: float = 1.0 / 256, min_d2: int = 0):
+        """refine_paths with the swept check (sweep_paths) in the accept test -> (Z_out, cost, collide, accepted,
+        sweep_flags, d2min).
+
+        A trial is kept only if refine_paths would keep it, it adds no sweep flag the path did not have (HIT, OUTSIDE,
+        INVALID), and, with min_d2 > 0, min(d2min, min_d2) does not drop.  So a path that sweeps clean inside the raster
+        stays clean between the samples as well, and one that starts at least sqrt(min_d2) cells from every occupied cell
+        ends so too.  min_d2 is an integer in squared cells (sweep_paths' d2min unit), 0 .. 65535: min_d2 = 2 keeps a
+        diagonal neighbour of an obstacle allowed, min_d2 = 4 asks for 2 cells.  cost / collide are score_paths(Z_out)'s
+        bits, sweep_flags / d2min sweep_paths(Z_out)'s; d2min is None when min_d2 == 0.  When the swept conditions never
+        reject a trial the result is bit-identical to refine_paths.  include/uam_b200.h (uam_refine_paths_raster_swept)
+        has the exact rule.  numpy in -> numpy out; a CUDA tensor in -> new CUDA tensors out (Z itself is not modified)."""
+        N = Z.shape[1] // 2 - 2
+        flags = (_lib.UAM_LENGTH_SMOOTH if length_smooth else 0) | (_lib.UAM_OWN_START if x_start is None else 0)
+        return self.engine.refine_raster_swept(Z, N, self.parameter_vector(weights, x_start), flags, samples_per_cell,
+                                               iterations, step_cells, max_step_cells, min_step_cells, min_d2)
+
     def sweep_paths(self, Z, clearance: bool = True):
         """Check every cell each segment of Z (B, 2(N+2)) float64 crosses against the occupancy -> (flags, first_hit,
         d2min); numpy in -> numpy out, a CUDA tensor in -> CUDA tensors out.  score_paths only looks at its samples.
