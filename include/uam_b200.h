@@ -329,6 +329,49 @@ enum { UAM_SWEEP_HIT = 1, UAM_SWEEP_OUTSIDE = 2, UAM_SWEEP_INVALID = 4 };
 int uam_sweep_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
                            int32_t* d_d2min, void* stream);
 
+/* Swept check of whole path segments against the analytic hard obstacles (the shapes Map.collides tests, uploaded with
+ * uam_map_set_shapes; region shapes are not tested).  uam_score_paths_analytic's collide flag, like map.py:41-43, looks at
+ * the N + 2 waypoints only; this call asks whether any segment enters an obstacle between them.
+ * Definition.  For every path of d_z (B, 2(N+2)) float64, segment k = 0 .. N from z_k to z_{k+1}, z(t) = z_k + t (z_{k+1}
+ * - z_k), and hard obstacle o (obstacle order = insertion order = device order): let h_i^R be the formula of record i of
+ * o (uam_h_exact: lines and boxes are affine in (x, y), an ellipse is a convex quadratic) in exact real arithmetic on the
+ * record's doubles, and K_o = { x : h_i^R(x) <= 1e-14 for every i of o } (`contains`, quadratic_obstacle.py:89-94, in
+ * exact arithmetic).  The segment meets K_o when some t in [0, 1] has z(t) in K_o.  The device decides HIT(k, o) in fp64:
+ *   G1 (never misses): if the real segment meets K_o, then HIT(k, o);
+ *   G2 (agrees with the waypoint check): if the fp64 `contains` is true at z_k or z_{k+1} (uam_psi's `inside`, the bits of
+ *      Map.collides and of uam_score_paths_analytic's collide flag), then HIT(k, o); so for every path that is not
+ *      INVALID, the analytic scorer's collide flag implies UAM_SWEEP_HIT;
+ *   G3 (bounded false alarm): if HIT(k, o), the real segment meets K_o^eta = { x : h_i^R(x) <= 1e-14 + eta_i for every i },
+ *      with A = z_k, B = z_{k+1}, u = 2^-53 and
+ *        line  (rec {0, Ax', Ay', dx', dy', sgn}):  eta_i = 2^-46 (M_i(A) + M_i(B)) + 2^-990,
+ *                                                   M_i(x, y) = |sgn| (|dy'| (|x| + |Ax'|) + |dx'| (|y| + |Ay'|));
+ *        box   (rec {2, axis, sign, c, r}):         eta_i = 2^-46 (M_i(A) + M_i(B)) + 2^-990,  M_i = |x_axis| + |c| + |r|;
+ *        ellipse (rec {1, cx, cy, r1, r2}):         eta_i = 2^-44 (2 + S) + 2^-94 S^2 + 2^-990,
+ *                                                   S = (|Ax - cx| + |Bx - Ax|) / |r1| + (|Ay - cy| + |By - Ay|) / |r2|,
+ *                                                   for S <= 2^40 (a segment within 2^40 radii of the ellipse);
+ *      M_i bounds the fp64 evaluation error of the formula, 3.01 u M_i,, which eta_i exceeds 16-fold, as G2 needs; S is
+ *      the segment's extent in the ellipse's scaled coordinates (DESIGN.md 9g derives both);
+ *   G4 (deterministic): the outputs are those of the numpy restatement in tests/analytic_sweep_reference.py, bit for bit,
+ *      in the same fp64 operation order; a path's outputs depend on that path and the map only, not on the rest of the
+ *      batch nor on UAM_OPT_SHAPE_GRID.
+ * Per path:
+ *   d_flags (uint8):                UAM_SWEEP_HIT: HIT(k, o) for some k and o; UAM_SWEEP_INVALID: a coordinate is not
+ *                                   finite or |coordinate| >= 1e100 (uam_psi's bound), nothing else is evaluated for the
+ *                                   path (first hit and first obstacle -1); UAM_SWEEP_OUTSIDE is never set.
+ *   d_first_hit (int32, nullable):  the lowest k with a hit, -1 if none;
+ *   d_first_obstacle (int32, nullable): the smallest o with HIT(first_hit, o), -1 if none.
+ * Cell lists: a G x G grid (G = 32 .. 256) over the obstacles' bounding box lists per cell the obstacles that may meet the
+ * cell at tolerance 1e-14; a segment tests only the obstacles listed in the cells it crosses.  They are built on the
+ * first call after each uam_map_set_shapes (that call synchronises) and kept; with UAM_OPT_SHAPE_GRID = 0, or fewer than 4
+ * obstacles, every segment tests every obstacle.  Stream-ordered on `stream` otherwise, no host read-back.
+ * Errors, in this order: B < 0, N < 0 or N > 2^28 UAM_ERR_INVALID; then B = 0 is a no-op; a NULL d_z / d_flags
+ * UAM_ERR_INVALID; no shapes uploaded UAM_ERR_STATE;
+ * then, before anything is launched, UAM_ERR_UNSUPPORTED for an obstacle record with a field that is not finite or beyond
+ * 1e100 in magnitude, an ellipse radius below 1e-50 in magnitude (0 included), or an obstacle with two ellipse records:
+ * the error bounds above do not hold for them.  A map without obstacles gives flags 0 (INVALID rows excepted) and -1. */
+int uam_sweep_paths_analytic(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
+                             int32_t* d_first_obstacle, void* stream);
+
 /* Scoring + best candidate in one call: as uam_score_paths_raster, and *d_key receives the best key (see uam_best) of the
  * batch -- of ALL ranks' batches when a peer group is attached (uam_peer_attach): the last kernel of the step finds the
  * local min, pushes it into every peer's symmetric block over NVLink and waits for theirs (no separate collective).

@@ -25,7 +25,7 @@ UAM_OWN_START = 1 << 4
 
 UAM_EDGE_LINE, UAM_EDGE_ELLIPSE, UAM_EDGE_BOX = 0, 1, 2
 
-# uam_sweep_paths_raster flag bits
+# flag bits of uam_sweep_paths_raster / uam_sweep_paths_analytic
 UAM_SWEEP_HIT, UAM_SWEEP_OUTSIDE, UAM_SWEEP_INVALID = 1, 2, 4
 
 _vp = C.c_void_p
@@ -58,6 +58,7 @@ SIGNATURES = {
     'uam_refine_paths_raster_swept': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _i, _d, _d, _d, _i, _vp, _vp, _vp, _vp,
                                            _vp, _vp]),
     'uam_sweep_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
+    'uam_sweep_paths_analytic': (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     'uam_eval_points': (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     'uam_eval_points_host': (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp]),
     'uam_eval_inequalities_host': (_i, [_vp, _vp, _i, _vp, _i64, _vp]),

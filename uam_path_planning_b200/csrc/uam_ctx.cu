@@ -250,6 +250,8 @@ extern "C" int uam_ctx_destroy(uam_ctx* ctx) {
     cudaFree(ctx->d_psic);
     cudaFree(ctx->d_grid_start);
     cudaFree(ctx->d_grid_items);
+    cudaFree(ctx->d_obs_grid);
+    cudaFree(ctx->d_obs_items);
     cudaFree(ctx->d_tex);
     cudaFree(ctx->d_scratch);
     cudaFree(ctx->d_cull_scratch);
@@ -399,6 +401,7 @@ extern "C" int uam_map_set_shapes(uam_ctx* ctx, const double* h_edges, int n_edg
     ctx->n_regions = n_regions;
     ctx->n_obs = n_obs;
     ctx->has_shapes = true;
+    ctx->shapes_gen++;
     ctx->edges_finite = finite;
     ctx->psic_valid = false;
     return UAM_OK;

@@ -51,6 +51,18 @@ struct UamShapeGrid {
     const int* items;
 };
 
+// Cell lists over the hard obstacles for the swept analytic check (uam_sweep_analytic.cu): cell (cy, cx) of a G x G grid
+// lists, in ascending obstacle order, every obstacle no single record of which is > 1e-14 (with the margin of
+// uam_edge_excludes_tile) on the cell's box widened by 1/1000 of a cell; the boxes of the border cells reach out to
+// +-ext.  Only segments whose four coordinates are all within [-qmax, qmax] use the lists (see the bound in the .cu).
+struct UamObsGrid {
+    double gx0, gy0, inv_cw, inv_ch;
+    double qmax;
+    int G;
+    const int* start;     // G * G + 1 offsets into items
+    const int* items;
+};
+
 struct UamRasterGeo {
     double x0, dx, y0, dy;
     int H, W, L;
@@ -217,6 +229,16 @@ struct uam_ctx {
     void* d_sweep_d2 = nullptr;
     size_t sweep_d2_bytes = 0;
     uint64_t sweep_d2_gen = 0;          // 0: none (raster_gen counts uploads from 1)
+    // swept check against the analytic obstacles (uam_sweep_analytic.cu): the obstacles' records checked on the host and
+    // their cell lists, both for the shape table of generation obs_gen (shapes_gen counts uploads from 1)
+    uint64_t shapes_gen = 0;
+    uint64_t obs_gen = 0;
+    int obs_rc = UAM_OK;                // UAM_ERR_UNSUPPORTED when the records break the sweep's error bounds
+    std::string obs_err;
+    UamObsGrid obs_grid = {};           // G == 0: no lists (fewer than 4 obstacles, or the bounds do not allow them)
+    int* d_obs_grid = nullptr;          // G * G + 1 offsets (+ G * G counts while they are built)
+    int* d_obs_items = nullptr;
+    size_t obs_grid_bytes = 0, obs_items_bytes = 0;
 };
 
 int uam_fail(uam_ctx* ctx, int code, const char* fmt, ...);
@@ -226,6 +248,8 @@ int uam_reserve_pinned(uam_ctx* ctx, void** ptr, size_t* cur, size_t need);
 int uam_make_params(uam_ctx* ctx, const double* h_p, int n_p, int flags, UamParams* out);
 int uam_ensure_shape_norm(uam_ctx* ctx, const UamParams& prm, cudaStream_t st, bool want_grid = true);
 int uam_build_shape_grid(uam_ctx* ctx, double e, int flags, cudaStream_t st);
+// the shape grid's exclusive prefix sum: start[0..n] of counts[0..n) (one CTA on `st`)
+int uam_shape_grid_scan(uam_ctx* ctx, const int* counts, int n, int* start, cudaStream_t st);
 // the grid to use for a call with these parameters (G == 0 when culling would not be exact for them)
 UamShapeGrid uam_pick_shape_grid(const uam_ctx* ctx, const UamParams& prm);
 cudaStream_t uam_pick_stream(uam_ctx* ctx, void* stream);

@@ -144,6 +144,12 @@ int uam_build_shape_grid(uam_ctx* ctx, double e, int flags, cudaStream_t st) {
     return UAM_OK;
 }
 
+int uam_shape_grid_scan(uam_ctx* ctx, const int* counts, int n, int* start, cudaStream_t st) {
+    uam_k_shape_grid_scan<<<1, 1024, 0, st>>>(counts, n, start);
+    UAM_CHECK_LAUNCH(ctx, "uam_k_shape_grid_scan");
+    return UAM_OK;
+}
+
 UamShapeGrid uam_pick_shape_grid(const uam_ctx* ctx, const UamParams& prm) {
     UamShapeGrid none{};
     // (the grid was built for these flags: uam_ensure_shape_norm rebuilds it whenever e or the smooth flags change)

@@ -331,6 +331,31 @@ class Engine:
             return tuple(None if t is None else t.cpu().numpy() for t in (flags, first, d2min))
         return flags, first, d2min
 
+    def sweep_analytic(self, Z, N: int, want_first_hit: bool = True, want_first_obstacle: bool = True):
+        """Z (B, 2(N+2)) float64 -> (flags u8 (B,), first_hit i32 (B,) | None, first_obstacle i32 (B,) | None) of
+        uam_sweep_paths_analytic: every segment checked against the analytic hard obstacles; numpy in -> numpy out, CUDA
+        tensor in -> CUDA tensors out."""
+        import torch
+        N = int(N)
+        host = not _is_tensor(Z)
+        if host:
+            Z = _f64c(Z)
+            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
+                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
+            Z = torch.from_numpy(Z).to(f'cuda:{self.device}')
+        assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+        st = self._tensor_args(Z)
+        B = Z.shape[0]
+        flags = torch.empty(B, dtype=torch.uint8, device=Z.device)
+        first = torch.empty(B, dtype=torch.int32, device=Z.device) if want_first_hit else None
+        obst = torch.empty(B, dtype=torch.int32, device=Z.device) if want_first_obstacle else None
+        self._check(self._lib.uam_sweep_paths_analytic(self._h, C.c_void_p(Z.data_ptr()), B, N, C.c_void_p(flags.data_ptr()),
+                                                       C.c_void_p(first.data_ptr()) if want_first_hit else None,
+                                                       C.c_void_p(obst.data_ptr()) if want_first_obstacle else None, st))
+        if host:
+            return tuple(None if t is None else t.cpu().numpy() for t in (flags, first, obst))
+        return flags, first, obst
+
     def score_raster_best(self, Z, N: int, p, flags: int, samples_per_cell: float, global_offset: int = 0, out=None, key=None):
         """score_raster on a CUDA tensor + the best key of the batch -- of every rank's batch when a peer group is attached
         (attach_peers): the exchange over NVLink peer memory rides in the last kernel of the step.

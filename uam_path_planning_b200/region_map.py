@@ -88,6 +88,20 @@ class Map:
         out = self.engine().eval_points(x.reshape(-1, 2), p, 0, want=('collide',))['collide'].astype(bool)
         return bool(out[0]) if x.ndim == 1 else out
 
+    def sweep_paths(self, Z):
+        """Swept check of every segment of the paths Z (B, 2(N+2)) against the hard obstacles -> (flags u8 (B,), first_hit
+        i32 (B,), first_obstacle i32 (B,)); N comes from Z's width, numpy in -> numpy out, CUDA tensor in -> CUDA tensors
+        out (uam_sweep_paths_analytic, include/uam_b200.h).  flags has UAM_SWEEP_HIT when some segment hits an obstacle and
+        UAM_SWEEP_INVALID for a row with a coordinate that is not finite or >= 1e100 in magnitude; first_hit is the lowest
+        hitting segment and first_obstacle the smallest obstacle index it hits (order of ``obstacles``), -1 if none.
+        G1: a segment that meets an obstacle in exact arithmetic is always reported.
+        G2: a waypoint that ``collides`` reports makes both of its segments hit, so the analytic scorer's collide flag
+        implies HIT.
+        G3: a reported segment comes within a few ulps of the obstacle: it meets the obstacle's inequalities relaxed by a
+        bound eta_i of the record's and the endpoints' magnitudes (about 1e-12 km on the reference's maps)."""
+        N = int(Z.shape[1]) // 2 - 2
+        return self.engine().sweep_analytic(Z, N, True, True)
+
     def intersection(self, x0, direction):
         # map.py:19-39 calls QuadraticObstacle.intersection, which is commented out in the reference
         raise AttributeError("'QuadraticObstacle' object has no attribute 'intersection'")
