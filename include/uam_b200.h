@@ -372,6 +372,52 @@ int uam_sweep_paths_raster(uam_ctx* ctx, const double* d_z, int64_t B, int N, ui
 int uam_sweep_paths_analytic(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
                              int32_t* d_first_obstacle, void* stream);
 
+/* Clearance of whole path segments from the analytic hard obstacles: how far each path stays from the obstacles, and
+ * which segment and obstacle come closest.  Paths, segments and obstacle order as in uam_sweep_paths_analytic.
+ * The set P_o of obstacle o, by the form of its records (the forms polygon(), square() and ball() make):
+ *   polygon: >= 3 line records; P_o is the convex hull of their origins (Ax, Ay).  Checked on the host: each direction
+ *            ends at the next origin, |A_i + d_i - A_{i+1}| <= 2^-50 (|A_i| + |A_{i+1}|) per component, cyclically, and
+ *            every origin but the record's own two lies strictly inside it (fp64 h < 0): a strictly convex polygon in
+ *            hull order with inward signs;
+ *   box:     exactly 4 box records, one per (axis, sign); P_o is the rectangle [c- - r-, c+ + r+] per axis (fp64), not empty;
+ *   ellipse: exactly one ellipse record; P_o is the filled ellipse (a disc when |r1| == |r2|, measured in closed form).
+ * Any other obstacle (for example line records with an ellipse record) gives UAM_ERR_UNSUPPORTED naming it, before
+ * anything is launched; uam_sweep_paths_analytic does not look at forms.
+ * The distance of segment k and obstacle o: D(k, o) = 0 iff HIT(k, o) (the sweep's own decision); otherwise the fp64
+ * distance from the segment to P_o, at least 2^-1022:
+ *   polygon, box: the minimum of the point-to-segment distances of each vertex to the segment and of A and B to each edge;
+ *   disc:         (distance from the centre to the segment) - r;
+ *   ellipse:      the minimum of the point-to-ellipse distances of A and B (Eberly's bisection, run until its midpoint
+ *                 repeats an end) and of the distances from the segment to the two boundary points whose normal is
+ *                 perpendicular to it, each counted when its foot on the segment's line falls in [0, 1].
+ * Per path: d_clearance (float64, nullable) = min(cap, min over k, o of D(k, o)); d_nearest_segment / d_nearest_obstacle
+ * (int32, nullable): the pair that attains it, the smallest k and then the smallest o, both -1 when the clearance equals
+ * cap (nothing lies within cap); d_flags (uint8, required): UAM_SWEEP_HIT and UAM_SWEEP_INVALID as the sweep sets them.
+ * An INVALID row gets clearance NaN and -1.  So clearance >= m is the keep-out check of a margin m <= cap.
+ *   D1 (agrees with the sweep): d_flags equals uam_sweep_paths_analytic's flags bit for bit; a HIT path has clearance 0,
+ *      nearest segment = first hit and nearest obstacle = first obstacle; a path neither HIT nor INVALID has clearance > 0.
+ *   D2 (error bound): for a pair that is not HIT, |D(k, o) - dist(segment k, P_o)| <= delta, with A, B the segment's ends,
+ *      D the exact distance, u = 2^-53, M the largest coordinate magnitude of A, B and the obstacle (polygon: its
+ *      vertices; box: its rectangle's bounds; disc and ellipse: |cx| + e0, |cy| + e0, e0 >= e1 the semi-axes):
+ *        polygon, box, disc: delta = 2^-48 M + 4 u D + 2^-1000;
+ *        ellipse:            delta = 2^-40 (e0 / e1) M + 4 u D + 2^-1000.
+ *      For a HIT pair the segment meets K_o^eta (G3), whose points lie within eps of P_o: box eps = sum over the two
+ *      axes of max_i (1e-14 + eta_i); ellipse eps = e0 (1e-14 + eta) / 2; polygon eps = max_i (1e-14 + eta_i) /
+ *      (|sgn_i| |d_i|) / cos(phi / 2), phi the largest exterior angle (DESIGN.md 9h).
+ *   D3 (deterministic): the outputs are those of the numpy restatement in tests/analytic_clearance_reference.py, bit for
+ *      bit; a path's outputs depend on that path and the map only, not on the rest of the batch nor on
+ *      UAM_OPT_SHAPE_GRID, and on cap only through the min with cap.
+ * Cell lists: the sweep's cells, listing also every obstacle whose box lies within cap (1 + 2^-40) of the cell (plus a
+ * margin above delta).  They are built on the first call after each uam_map_set_shapes or change of cap (that call
+ * synchronises) and kept; with UAM_OPT_SHAPE_GRID = 0, where the sweep has no lists, or where the lists would hold over
+ * 3/4 of all (cell, obstacle) pairs, every segment tests every obstacle.  Stream-ordered on `stream` otherwise.
+ * Errors, in this order: B < 0, N < 0, N > 2^28, or cap not in (0, 1e100] UAM_ERR_INVALID; then B = 0 is a no-op; a NULL
+ * d_z / d_flags UAM_ERR_INVALID; no shapes UAM_ERR_STATE; the sweep's record checks, then the form checks above,
+ * UAM_ERR_UNSUPPORTED.  A map without obstacles gives clearance = cap and -1 (INVALID rows excepted). */
+int uam_clearance_paths_analytic(uam_ctx* ctx, const double* d_z, int64_t B, int N, double cap, uint8_t* d_flags,
+                                 double* d_clearance, int32_t* d_nearest_segment, int32_t* d_nearest_obstacle,
+                                 void* stream);
+
 /* Scoring + best candidate in one call: as uam_score_paths_raster, and *d_key receives the best key (see uam_best) of the
  * batch -- of ALL ranks' batches when a peer group is attached (uam_peer_attach): the last kernel of the step finds the
  * local min, pushes it into every peer's symmetric block over NVLink and waits for theirs (no separate collective).

@@ -59,6 +59,7 @@ SIGNATURES = {
                                            _vp, _vp]),
     'uam_sweep_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     'uam_sweep_paths_analytic': (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
+    'uam_clearance_paths_analytic': (_i, [_vp, _vp, _i64, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     'uam_eval_points': (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     'uam_eval_points_host': (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp]),
     'uam_eval_inequalities_host': (_i, [_vp, _vp, _i, _vp, _i64, _vp]),

@@ -252,6 +252,9 @@ extern "C" int uam_ctx_destroy(uam_ctx* ctx) {
     cudaFree(ctx->d_grid_items);
     cudaFree(ctx->d_obs_grid);
     cudaFree(ctx->d_obs_items);
+    cudaFree(ctx->d_obs_geom);
+    cudaFree(ctx->d_clr_grid);
+    cudaFree(ctx->d_clr_items);
     cudaFree(ctx->d_tex);
     cudaFree(ctx->d_scratch);
     cudaFree(ctx->d_cull_scratch);

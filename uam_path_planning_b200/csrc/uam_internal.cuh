@@ -63,6 +63,16 @@ struct UamObsGrid {
     const int* items;
 };
 
+// Form of a hard obstacle for the clearance (uam_clearance_paths_analytic), decided on the host from its records
+enum { UAM_FORM_POLYGON = 0, UAM_FORM_ELLIPSE = 1, UAM_FORM_BOX = 2, UAM_FORM_DISC = 3 };
+struct UamObsGeom {
+    double x0, x1, y0, y1;        // box: the rectangle [x0, x1] x [y0, y1] (fp64 c - r, c + r of its records)
+    double bx0, bx1, by0, by1;    // a box that contains the obstacle (P_o), rounded outward
+    double rho;                   // the factor of the distance's error bound: 1, or e0 / e1 for an ellipse (DESIGN.md 9h)
+    int form;
+    int pad;
+};
+
 struct UamRasterGeo {
     double x0, dx, y0, dy;
     int H, W, L;
@@ -239,6 +249,20 @@ struct uam_ctx {
     int* d_obs_grid = nullptr;          // G * G + 1 offsets (+ G * G counts while they are built)
     int* d_obs_items = nullptr;
     size_t obs_grid_bytes = 0, obs_items_bytes = 0;
+    // clearance (same file): the obstacles' forms and boxes, checked with the records above, and cell lists dilated by
+    // the cap of generation clr_gen (clr_cap)
+    int clr_rc = UAM_OK;                // UAM_ERR_UNSUPPORTED when an obstacle is none of the forms the clearance measures
+    std::string clr_err;
+    UamObsGeom* d_obs_geom = nullptr;
+    size_t obs_geom_bytes = 0;
+    std::vector<UamObsGeom> h_obs_geom;
+    double obs_cw = 0.0, obs_ch = 0.0, obs_ext = 0.0;   // the sweep grid's cell sides and border reach
+    uint64_t clr_gen = 0;
+    double clr_cap = 0.0;
+    UamObsGrid clr_grid = {};           // G == 0: every segment tests every obstacle
+    int* d_clr_grid = nullptr;
+    int* d_clr_items = nullptr;
+    size_t clr_grid_bytes = 0, clr_items_bytes = 0;
 };
 
 int uam_fail(uam_ctx* ctx, int code, const char* fmt, ...);

@@ -356,6 +356,32 @@ class Engine:
             return tuple(None if t is None else t.cpu().numpy() for t in (flags, first, obst))
         return flags, first, obst
 
+    def clearance_analytic(self, Z, N: int, cap: float, want_nearest: bool = True):
+        """Z (B, 2(N+2)) float64 -> (flags u8 (B,), clearance f64 (B,), nearest_segment i32 (B,) | None, nearest_obstacle
+        i32 (B,) | None) of uam_clearance_paths_analytic: each path's distance from the analytic hard obstacles, capped at
+        cap; numpy in -> numpy out, CUDA tensor in -> CUDA tensors out."""
+        import torch
+        N = int(N)
+        host = not _is_tensor(Z)
+        if host:
+            Z = _f64c(Z)
+            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
+                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
+            Z = torch.from_numpy(Z).to(f'cuda:{self.device}')
+        assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+        st = self._tensor_args(Z)
+        B = Z.shape[0]
+        flags = torch.empty(B, dtype=torch.uint8, device=Z.device)
+        clear = torch.empty(B, dtype=torch.float64, device=Z.device)
+        seg = torch.empty(B, dtype=torch.int32, device=Z.device) if want_nearest else None
+        obst = torch.empty(B, dtype=torch.int32, device=Z.device) if want_nearest else None
+        ptr = (lambda t: None if t is None else C.c_void_p(t.data_ptr()))
+        self._check(self._lib.uam_clearance_paths_analytic(self._h, ptr(Z), B, N, float(cap), ptr(flags), ptr(clear), ptr(seg),
+                                                           ptr(obst), st))
+        if host:
+            return tuple(None if t is None else t.cpu().numpy() for t in (flags, clear, seg, obst))
+        return flags, clear, seg, obst
+
     def score_raster_best(self, Z, N: int, p, flags: int, samples_per_cell: float, global_offset: int = 0, out=None, key=None):
         """score_raster on a CUDA tensor + the best key of the batch -- of every rank's batch when a peer group is attached
         (attach_peers): the exchange over NVLink peer memory rides in the last kernel of the step.

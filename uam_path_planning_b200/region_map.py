@@ -102,6 +102,23 @@ class Map:
         N = int(Z.shape[1]) // 2 - 2
         return self.engine().sweep_analytic(Z, N, True, True)
 
+    def path_clearance(self, Z, cap):
+        """How far each path of Z (B, 2(N+2)) stays from the hard obstacles, up to cap -> (flags u8 (B,), clearance f64
+        (B,), nearest_segment i32 (B,), nearest_obstacle i32 (B,)); N comes from Z's width, numpy in -> numpy out, CUDA
+        tensor in -> CUDA tensors out (uam_clearance_paths_analytic, include/uam_b200.h).  clearance is min(cap, the
+        distance from the path's segments to the obstacles), and the nearest pair is the segment and obstacle that
+        attain it (smallest segment, then smallest obstacle), -1 when nothing lies within cap.  So ``clearance >= m`` is
+        the keep-out check of a margin m <= cap.  Obstacles must be polygons, boxes or ellipses, as polygon(), square()
+        and ball() make them; other record combinations raise.
+        D1: flags are ``sweep_paths``'s flags bit for bit; a path that hits has clearance 0 and its nearest pair is the
+        sweep's first hit; any other valid path has clearance > 0.  INVALID rows get NaN and -1.
+        D2: a non-hitting segment's distance is exact up to a rounding bound of a few ulps of the coordinates' magnitude
+        (more for elongated ellipses: it scales with their axis ratio).
+        D3: the results are deterministic, bit for bit: they do not depend on the rest of the batch, on the cell lists,
+        or on cap other than through the min with cap."""
+        N = int(Z.shape[1]) // 2 - 2
+        return self.engine().clearance_analytic(Z, N, cap, True)
+
     def intersection(self, x0, direction):
         # map.py:19-39 calls QuadraticObstacle.intersection, which is commented out in the reference
         raise AttributeError("'QuadraticObstacle' object has no attribute 'intersection'")
