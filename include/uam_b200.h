@@ -294,6 +294,41 @@ int uam_refine_paths_raster_swept(uam_ctx* ctx, double* d_z, int64_t B, int N, c
                                   double min_step_cells, int min_d2, float* d_cost, uint8_t* d_collide,
                                   int32_t* d_accepted, uint8_t* d_sweep_flags, int32_t* d_d2min, void* stream);
 
+/* uam_refine_paths_raster with the analytic check (uam_sweep_paths_analytic and uam_clearance_paths_analytic, below) in
+ * its accept test, so that refinement never moves a path into a no-fly shape, between the raster's cell centres as
+ * well, and, with margin > 0, never closer than margin (map units, km) to one.  The shapes are those of the last
+ * uam_map_set_shapes.  The rule is exactly uam_refine_paths_raster's (steps 1 - 4 above) with two additions:
+ *   - "evaluate Z" also computes, for the whole batch, f = the flags of uam_sweep_paths_analytic (UAM_SWEEP_HIT |
+ *     INVALID) and, with margin > 0, cl = the clearance of uam_clearance_paths_analytic at cap = margin; these are those
+ *     calls' bits;
+ *   - step 4 becomes: accept iff active and kt <= k and ct < c and (ft & ~f) == 0 and (margin == 0 or clt >= cl) (fp64;
+ *     a NaN compares false and rejects); on accept also f, cl <- ft, clt.
+ *   K1 (no new hit): a trial never adds HIT or INVALID: a path that sweeps clean against the shapes stays clean, with
+ *      G1's "never misses" carried over;
+ *   K2 (keep-out): with margin > 0, min(clearance, margin) never drops: a path that starts at least margin from every
+ *      obstacle (up to the clearance's delta, D2) ends so, and one that starts closer never gets closer;
+ *   K3 (refines no further than the plain call): every trial this call accepts, uam_refine_paths_raster would have
+ *      accepted as well; when the new terms never reject a trial (for example a map without obstacles, or with
+ *      obstacles far from every path), the outputs are bit-identical to it;
+ *   K4 (outputs): on return d_cost / d_collide hold uam_score_paths_raster's bits for the returned paths, as there;
+ *      d_sweep_flags (uint8, required) uam_sweep_paths_analytic's flags; d_clearance (float64, nullable, only with
+ *      margin > 0) uam_clearance_paths_analytic's clearance at cap = margin.
+ * A path that is already HIT may still be accepted into collide = 0 while it cuts a shape: that trial adds no flag.  With
+ * margin > 0 a path whose clearance is NaN (INVALID) takes no trial.  margin is in [0, 1e100]; margin = 0 uses the sweep
+ * only.  Each trip adds one launch of the analytic sweep (margin = 0) or of the analytic clearance (margin > 0) of the
+ * trial batch after its gradient launch, on `stream`, no host read-back.  The record checks and the sweep's cell lists,
+ * the clearance's lists for cap = margin (both cached: per upload, and per upload and cap) and the quad texels are built
+ * first when missing (each may synchronise).  Scratch: that of uam_refine_paths_raster + 1 byte per path, + 8 with
+ * margin > 0, + 8 more when d_clearance is NULL.  Errors, in this order: those of uam_refine_paths_raster in the same
+ * order (margin out of range or N > 2^28 is UAM_ERR_INVALID with the step sizes; a NULL d_sweep_flags, or a non-NULL
+ * d_clearance with margin = 0, UAM_ERR_INVALID with the other pointers); no shapes uploaded UAM_ERR_STATE; the sweep's
+ * record checks, then with margin > 0 the clearance's form checks, UAM_ERR_UNSUPPORTED; all before any quad build or
+ * scratch reservation. */
+int uam_refine_paths_raster_keepout(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
+                                    double samples_per_cell, int iterations, double step_cells, double max_step_cells,
+                                    double min_step_cells, double margin, float* d_cost, uint8_t* d_collide,
+                                    int32_t* d_accepted, uint8_t* d_sweep_flags, double* d_clearance, void* stream);
+
 /* Swept check of whole path segments against the raster's occupancy, and each path's clearance.  The scorer above only
  * looks at its samples; this call looks at every cell a segment crosses.  For every path of d_z (B, 2(N+2)) and every
  * segment k = 0 .. N (z_k -> z_{k+1}):

@@ -57,6 +57,8 @@ SIGNATURES = {
     'uam_refine_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _i, _d, _d, _d, _vp, _vp, _vp, _vp]),
     'uam_refine_paths_raster_swept': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _i, _d, _d, _d, _i, _vp, _vp, _vp, _vp,
                                            _vp, _vp]),
+    'uam_refine_paths_raster_keepout': (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _d, _i, _d, _d, _d, _d, _vp, _vp, _vp,
+                                             _vp, _vp, _vp]),
     'uam_sweep_paths_raster': (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     'uam_sweep_paths_analytic': (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     'uam_clearance_paths_analytic': (_i, [_vp, _vp, _i64, _i, _d, _vp, _vp, _vp, _vp, _vp]),

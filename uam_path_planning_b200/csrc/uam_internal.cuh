@@ -321,6 +321,22 @@ int uam_sweep_ensure_d2(uam_ctx* ctx, cudaStream_t st);
 int uam_sweep_enqueue(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
                       int32_t* d_d2min, cudaStream_t st);
 
+// Analytic sweep and clearance (uam_sweep_analytic.cu), in the steps of a call once the shapes are known to be uploaded:
+// uam_ensure_obs_tables checks the obstacles' records and forms and builds the sweep's cell lists on the first call
+// after each upload; uam_obs_supported then returns the record checks' verdict and, with the clearance, the form
+// checks' (UAM_ERR_UNSUPPORTED naming the obstacle); uam_ensure_clr_lists builds the clearance's lists for `cap` when
+// they are missing (shape_grid option on).  Both builds synchronise the device when they run: call them before
+// enqueueing work that must stay ordered.  uam_sweep_analytic_enqueue / uam_clearance_analytic_enqueue then enqueue one
+// launch on `st`, without host synchronisation; the clearance's needs uam_ensure_clr_lists for the same cap first.
+int uam_ensure_obs_tables(uam_ctx* ctx, cudaStream_t st);
+int uam_obs_supported(uam_ctx* ctx, bool clearance);
+int uam_ensure_clr_lists(uam_ctx* ctx, double cap, cudaStream_t st);
+int uam_sweep_analytic_enqueue(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
+                               int32_t* d_first_obstacle, cudaStream_t st);
+int uam_clearance_analytic_enqueue(uam_ctx* ctx, const double* d_z, int64_t B, int N, double cap, uint8_t* d_flags,
+                                   double* d_clearance, int32_t* d_nearest_segment, int32_t* d_nearest_obstacle,
+                                   cudaStream_t st);
+
 // NVTX range over the rest of the enclosing scope (host side; a no-op costing a few ns when no profiler is attached):
 // upload / bin / score / reduce / exchange phases show up by name on an Nsight Systems timeline
 struct UamNvtxRange {

@@ -10,6 +10,9 @@
 //
 // uam_refine_paths_raster_swept adds one uam_k_sweep_paths launch of the trial batch per trip (uam_sweep_enqueue) and
 // the swept terms of the accept test (UAM_REFINE_SWEPT); everything else is the same loop.
+// uam_refine_paths_raster_keepout adds one launch of the analytic sweep, or with a margin of the analytic clearance, of
+// the trial batch per trip (uam_sweep_analytic_enqueue / uam_clearance_analytic_enqueue) and its terms of the accept
+// test (UAM_REFINE_KEEPOUT).
 #include <algorithm>
 #include <cmath>
 
@@ -23,6 +26,7 @@ enum : int {
     UAM_REFINE_ACCEPT = 2,     // take or drop the trial in zt, evaluated into (ct, kt, gt)
     UAM_REFINE_PROPOSE = 4,    // write the next trial into zt and whether it moved the path into active
     UAM_REFINE_SWEPT = 8,      // the accept test also needs the trial's swept flags (ft) and clearance (d2t)
+    UAM_REFINE_KEEPOUT = 16,   // ... the trial's analytic sweep flags (ft) and clearance (clt)
 };
 
 struct UamRefineState {
@@ -48,6 +52,10 @@ struct UamRefineState {
     int32_t* d2;
     const int32_t* d2t;
     int min_d2;
+    // UAM_REFINE_KEEPOUT: f / ft hold the analytic sweep's flags; the analytic clearance capped at the margin at z (the
+    // caller's output or scratch) and at zt, both NULL with margin 0
+    double* cl;
+    const double* clt;
 };
 
 __device__ __forceinline__ double uam_warp_max(double v) {
@@ -85,6 +93,15 @@ __global__ void __launch_bounds__(UAM_CTA_THREADS) uam_k_refine_step(const UamRe
                 take = take && (s.min_d2 == 0 || min(d2t, s.min_d2) >= min(s.d2[b], s.min_d2));
             }
         }
+        double clt = 0.0;
+        if (MODE & UAM_REFINE_KEEPOUT) {
+            ft = s.ft[b];
+            take = take && (ft & ~s.f[b]) == 0;
+            if (s.cl) {
+                clt = s.clt[b];
+                take = take && clt >= s.cl[b];     // a NaN rejects
+            }
+        }
         __syncwarp();                  // every lane has read the per-path scalars before lane 0 overwrites them
         if (MODE & UAM_REFINE_ACCEPT) {
             if (take) {
@@ -94,6 +111,10 @@ __global__ void __launch_bounds__(UAM_CTA_THREADS) uam_k_refine_step(const UamRe
                 if ((MODE & UAM_REFINE_SWEPT) && lane == 0) {
                     s.f[b] = ft;
                     if (s.d2) s.d2[b] = d2t;
+                }
+                if ((MODE & UAM_REFINE_KEEPOUT) && lane == 0) {
+                    s.f[b] = ft;
+                    if (s.cl) s.cl[b] = clt;
                 }
             } else if (was_active) {
                 tau = 0.5 * tau;
@@ -145,11 +166,21 @@ int uam_refine_step_launch(uam_ctx* ctx, const UamRefineState& s, cudaStream_t s
 
 }  // namespace
 
-// Both entry points: swept = uam_refine_paths_raster_swept (min_d2, d_sweep_flags and d_d2min are only read then).
+// the analytic check of the keep-out refinement on a batch: the sweep's flags, or with margin > 0 the clearance's flags
+// and clearance capped at the margin
+static int uam_keepout_enqueue(uam_ctx* ctx, const double* d_z, int64_t B, int N, double margin, uint8_t* d_flags,
+                               double* d_clearance, cudaStream_t st) {
+    if (margin > 0.0) return uam_clearance_analytic_enqueue(ctx, d_z, B, N, margin, d_flags, d_clearance, nullptr, nullptr, st);
+    return uam_sweep_analytic_enqueue(ctx, d_z, B, N, d_flags, nullptr, nullptr, st);
+}
+
+// All entry points: swept = uam_refine_paths_raster_swept (min_d2, d_sweep_flags and d_d2min are only read then),
+// keepout = uam_refine_paths_raster_keepout (margin, d_sweep_flags and d_clearance are only read then).
 static int uam_refine_run(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p, int flags,
                           double samples_per_cell, int iterations, double step_cells, double max_step_cells,
                           double min_step_cells, float* d_cost, uint8_t* d_collide, int32_t* d_accepted, bool swept,
-                          int min_d2, uint8_t* d_sweep_flags, int32_t* d_d2min, void* stream) {
+                          int min_d2, uint8_t* d_sweep_flags, int32_t* d_d2min, bool keepout, double margin,
+                          double* d_clearance, void* stream) {
     if (!ctx) return UAM_ERR_INVALID;
     if (iterations < 0) return uam_fail(ctx, UAM_ERR_INVALID, "iterations must be >= 0 (got %d)", iterations);
     if (!(std::isfinite(step_cells) && std::isfinite(max_step_cells) && std::isfinite(min_step_cells) && min_step_cells > 0.0 &&
@@ -157,35 +188,59 @@ static int uam_refine_run(uam_ctx* ctx, double* d_z, int64_t B, int N, const dou
         return uam_fail(ctx, UAM_ERR_INVALID, "step sizes must be finite with 0 < min <= step <= max (got %g, %g, %g)",
                         min_step_cells, step_cells, max_step_cells);
     if (swept && (min_d2 < 0 || min_d2 > 65535)) return uam_fail(ctx, UAM_ERR_INVALID, "min_d2 must be in 0 .. 65535 (got %d)", min_d2);
+    if (keepout && !(margin >= 0.0 && margin <= 1e100))
+        return uam_fail(ctx, UAM_ERR_INVALID, "margin must be in [0, 1e100] (got %g)", margin);
+    if (keepout && N > (1 << 28)) return uam_fail(ctx, UAM_ERR_INVALID, "need N <= 2^28 for the analytic check (got %d)", N);
     UamRasterParams rp;
     UAM_TRY(uam_raster_prepare(ctx, B, N, h_p, n_p, flags, samples_per_cell, &rp));
     if (B == 0) return UAM_OK;
     if (!d_z || !d_cost || !d_collide) return uam_fail(ctx, UAM_ERR_INVALID, "paths, cost or collide pointer is NULL");
-    if (swept && !d_sweep_flags) return uam_fail(ctx, UAM_ERR_INVALID, "sweep flags pointer is NULL");
+    if ((swept || keepout) && !d_sweep_flags) return uam_fail(ctx, UAM_ERR_INVALID, "sweep flags pointer is NULL");
+    if (keepout && d_clearance && margin == 0.0)
+        return uam_fail(ctx, UAM_ERR_INVALID, "a clearance pointer needs margin > 0 (the clearance is capped at the margin)");
     UAM_TRY(uam_raster_grad_supported(ctx, rp));
     const bool clearance = swept && (min_d2 > 0 || d_d2min);
     if (swept) UAM_TRY(uam_sweep_supported(ctx, N, clearance));
+    const bool keepout_cl = keepout && margin > 0.0;
+    if (keepout && !ctx->has_shapes) return uam_fail(ctx, UAM_ERR_STATE, "no shapes: call uam_map_set_shapes first");
     UAM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = uam_pick_stream(ctx, stream);
-    UAM_NVTX(swept ? "uam.raster.refine_swept" : "uam.raster.refine");
+    UAM_NVTX(swept ? "uam.raster.refine_swept" : keepout ? "uam.raster.refine_keepout" : "uam.raster.refine");
+    if (keepout) {
+        UAM_TRY(uam_ensure_obs_tables(ctx, st));
+        UAM_TRY(uam_obs_supported(ctx, keepout_cl));
+        if (keepout_cl) UAM_TRY(uam_ensure_clr_lists(ctx, margin, st));
+    }
     if (swept) UAM_TRY(uam_ensure_occ_bits(ctx, st));
     if (clearance) UAM_TRY(uam_sweep_ensure_d2(ctx, st));
     UAM_TRY(uam_raster_precompute(ctx, &rp, B, N, st));
 
-    // scratch: zt | g | gt (B x Wp double2 each) | tau (f64) | ct (f32) | accepted (i32, when the caller passes none) |
-    // [d2t (i32) | d2 (i32, when the caller passes none): clearance] | kt (u8) | active (u8) | [ft (u8): swept]
+    // scratch: zt | g | gt (B x Wp double2 each) | tau (f64) | [clt (f64) | cl (f64, when the caller passes none):
+    // keep-out with a margin] | ct (f32) | accepted (i32, when the caller passes none) | [d2t (i32) | d2 (i32, when the
+    // caller passes none): clearance] | kt (u8) | active (u8) | [ft (u8): swept or keep-out]
     const int Wp = N + 2;
     const size_t n = (size_t)B * Wp;
     const size_t swept_bytes = swept ? (size_t)B * (1 + (clearance ? 4 : 0) + (clearance && !d_d2min ? 4 : 0)) : 0;
+    const size_t keepout_bytes = keepout ? (size_t)B * (1 + (keepout_cl ? 8 : 0) + (keepout_cl && !d_clearance ? 8 : 0)) : 0;
     UAM_TRY(uam_reserve(ctx, &ctx->d_refine_scratch, &ctx->refine_scratch_bytes,
-                        3 * n * sizeof(double2) + (size_t)B * 18 + swept_bytes));
+                        3 * n * sizeof(double2) + (size_t)B * 18 + swept_bytes + keepout_bytes));
     UamRefineState s;
     s.zt = (double2*)ctx->d_refine_scratch;
     s.g = s.zt + n;
     double2* gt = s.g + n;
     s.gt = gt;
     s.tau = (double*)(gt + n);
-    float* ct = (float*)(s.tau + B);
+    double* f64_end = s.tau + B;
+    double* clt = nullptr;
+    s.cl = nullptr;
+    if (keepout_cl) {
+        clt = f64_end;
+        f64_end += B;
+        s.cl = d_clearance ? d_clearance : f64_end;
+        if (!d_clearance) f64_end += B;
+    }
+    s.clt = clt;
+    float* ct = (float*)f64_end;
     s.ct = ct;
     int32_t* acc_scratch = (int32_t*)(ct + B);
     int32_t* i32_end = acc_scratch + B;
@@ -201,7 +256,7 @@ static int uam_refine_run(uam_ctx* ctx, double* d_z, int64_t B, int N, const dou
     uint8_t* kt = (uint8_t*)i32_end;
     s.kt = kt;
     s.active = kt + B;
-    uint8_t* ft = swept ? kt + 2 * B : nullptr;
+    uint8_t* ft = swept || keepout ? kt + 2 * B : nullptr;
     s.ft = ft;
     s.f = d_sweep_flags;
     s.min_d2 = min_d2;
@@ -218,6 +273,7 @@ static int uam_refine_run(uam_ctx* ctx, double* d_z, int64_t B, int N, const dou
 
     UAM_TRY(uam_raster_grad_enqueue(ctx, rp, d_z, B, N, d_cost, d_collide, (double*)s.g, st));
     if (swept) UAM_TRY(uam_sweep_enqueue(ctx, d_z, B, N, d_sweep_flags, nullptr, s.d2, st));
+    if (keepout) UAM_TRY(uam_keepout_enqueue(ctx, d_z, B, N, margin, d_sweep_flags, s.cl, st));
     if (iterations == 0) {
         if (d_accepted) UAM_CUDA(ctx, cudaMemsetAsync(d_accepted, 0, (size_t)B * sizeof(int32_t), st));
         return UAM_OK;
@@ -230,6 +286,10 @@ static int uam_refine_run(uam_ctx* ctx, double* d_z, int64_t B, int N, const dou
             UAM_TRY(uam_sweep_enqueue(ctx, (const double*)s.zt, B, N, ft, nullptr, d2t, st));
             if (!last) UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_PROPOSE | UAM_REFINE_SWEPT>(ctx, s, st));
             else UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_SWEPT>(ctx, s, st));
+        } else if (keepout) {
+            UAM_TRY(uam_keepout_enqueue(ctx, (const double*)s.zt, B, N, margin, ft, clt, st));
+            if (!last) UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_PROPOSE | UAM_REFINE_KEEPOUT>(ctx, s, st));
+            else UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_KEEPOUT>(ctx, s, st));
         } else {
             if (!last) UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT | UAM_REFINE_PROPOSE>(ctx, s, st));
             else UAM_TRY(uam_refine_step_launch<UAM_REFINE_ACCEPT>(ctx, s, st));
@@ -243,7 +303,8 @@ extern "C" int uam_refine_paths_raster(uam_ctx* ctx, double* d_z, int64_t B, int
                                        double min_step_cells, float* d_cost, uint8_t* d_collide, int32_t* d_accepted,
                                        void* stream) {
     return uam_refine_run(ctx, d_z, B, N, h_p, n_p, flags, samples_per_cell, iterations, step_cells, max_step_cells,
-                          min_step_cells, d_cost, d_collide, d_accepted, false, 0, nullptr, nullptr, stream);
+                          min_step_cells, d_cost, d_collide, d_accepted, false, 0, nullptr, nullptr, false, 0.0, nullptr,
+                          stream);
 }
 
 extern "C" int uam_refine_paths_raster_swept(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p,
@@ -252,5 +313,16 @@ extern "C" int uam_refine_paths_raster_swept(uam_ctx* ctx, double* d_z, int64_t 
                                              uint8_t* d_collide, int32_t* d_accepted, uint8_t* d_sweep_flags,
                                              int32_t* d_d2min, void* stream) {
     return uam_refine_run(ctx, d_z, B, N, h_p, n_p, flags, samples_per_cell, iterations, step_cells, max_step_cells,
-                          min_step_cells, d_cost, d_collide, d_accepted, true, min_d2, d_sweep_flags, d_d2min, stream);
+                          min_step_cells, d_cost, d_collide, d_accepted, true, min_d2, d_sweep_flags, d_d2min, false, 0.0,
+                          nullptr, stream);
+}
+
+extern "C" int uam_refine_paths_raster_keepout(uam_ctx* ctx, double* d_z, int64_t B, int N, const double* h_p, int n_p,
+                                               int flags, double samples_per_cell, int iterations, double step_cells,
+                                               double max_step_cells, double min_step_cells, double margin, float* d_cost,
+                                               uint8_t* d_collide, int32_t* d_accepted, uint8_t* d_sweep_flags,
+                                               double* d_clearance, void* stream) {
+    return uam_refine_run(ctx, d_z, B, N, h_p, n_p, flags, samples_per_cell, iterations, step_cells, max_step_cells,
+                          min_step_cells, d_cost, d_collide, d_accepted, false, 0, d_sweep_flags, nullptr, true, margin,
+                          d_clearance, stream);
 }

@@ -589,11 +589,15 @@ int uam_obs_forms(const std::vector<UamShape>& shapes, const std::vector<UamEdge
     return UAM_OK;
 }
 
+}  // namespace
+
 // On the first call after each upload: copy the obstacles' records back, check them, and (shape_grid option on, at
-// least 4 obstacles) build the lists.  Synchronises `st`.
+// least 4 obstacles) build the lists.  Synchronises the device first (a call on another stream may still read the old
+// lists), then `st`.
 int uam_ensure_obs_tables(uam_ctx* ctx, cudaStream_t st) {
     if (ctx->obs_gen == ctx->shapes_gen) return UAM_OK;
     UAM_NVTX("uam.analytic.sweep.build_lists");
+    UAM_CUDA(ctx, cudaDeviceSynchronize());
     const int n_obs = ctx->n_obs;
     std::vector<UamShape> shapes(n_obs);
     std::vector<UamEdge> recs;
@@ -706,9 +710,12 @@ int uam_ensure_obs_tables(uam_ctx* ctx, cudaStream_t st) {
 // cells, every obstacle the sweep lists there and every obstacle whose box lies within dil_o = cap (1 + 2^-40) +
 // 2^-36 rho_o (qmax + |box|) of the cell (the second term exceeds the distance's error bound delta, DESIGN.md 9h).  No
 // lists (every segment tests every obstacle) where the sweep has none or where they would hold over 3/4 of all pairs.
+// Nothing is built with the shape_grid option off.  Synchronises the device first (a clearance call on another stream
+// may still read the old lists), then `st`.
 int uam_ensure_clr_lists(uam_ctx* ctx, double cap, cudaStream_t st) {
-    if (ctx->clr_gen == ctx->shapes_gen && ctx->clr_cap == cap) return UAM_OK;
+    if (!ctx->shape_grid_opt || (ctx->clr_gen == ctx->shapes_gen && ctx->clr_cap == cap)) return UAM_OK;
     UAM_NVTX("uam.analytic.clearance.build_lists");
+    UAM_CUDA(ctx, cudaDeviceSynchronize());
     ctx->clr_grid = UamObsGrid{};
     ctx->clr_gen = ctx->shapes_gen;
     ctx->clr_cap = cap;
@@ -749,7 +756,34 @@ int uam_ensure_clr_lists(uam_ctx* ctx, double cap, cudaStream_t st) {
     return UAM_OK;
 }
 
-}  // namespace
+int uam_obs_supported(uam_ctx* ctx, bool clearance) {
+    if (ctx->obs_rc != UAM_OK) return uam_fail(ctx, ctx->obs_rc, "%s", ctx->obs_err.c_str());
+    if (clearance && ctx->clr_rc != UAM_OK) return uam_fail(ctx, ctx->clr_rc, "%s", ctx->clr_err.c_str());
+    return UAM_OK;
+}
+
+int uam_sweep_analytic_enqueue(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags, int32_t* d_first_hit,
+                               int32_t* d_first_obstacle, cudaStream_t st) {
+    const UamObsGrid og = ctx->shape_grid_opt ? ctx->obs_grid : UamObsGrid{};
+    const long long ctas = std::min<long long>((B + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA, (long long)ctx->sm_count * 16);
+    uam_k_sweep_analytic<<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(reinterpret_cast<const double2*>(d_z), B, N + 2,
+                                                                     ctx->d_edges, ctx->d_shapes, ctx->n_obs, og, d_flags,
+                                                                     d_first_hit, d_first_obstacle);
+    UAM_CHECK_LAUNCH(ctx, "uam_k_sweep_analytic");
+    return UAM_OK;
+}
+
+int uam_clearance_analytic_enqueue(uam_ctx* ctx, const double* d_z, int64_t B, int N, double cap, uint8_t* d_flags,
+                                   double* d_clearance, int32_t* d_nearest_segment, int32_t* d_nearest_obstacle,
+                                   cudaStream_t st) {
+    const UamObsGrid og = ctx->shape_grid_opt ? ctx->clr_grid : UamObsGrid{};
+    const long long ctas = std::min<long long>((B + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA, (long long)ctx->sm_count * 16);
+    uam_k_clearance_analytic<<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(
+        reinterpret_cast<const double2*>(d_z), B, N + 2, ctx->d_edges, ctx->d_shapes, ctx->d_obs_geom, ctx->n_obs, og, cap,
+        d_flags, d_clearance, d_nearest_segment, d_nearest_obstacle);
+    UAM_CHECK_LAUNCH(ctx, "uam_k_clearance_analytic");
+    return UAM_OK;
+}
 
 extern "C" int uam_sweep_paths_analytic(uam_ctx* ctx, const double* d_z, int64_t B, int N, uint8_t* d_flags,
                                         int32_t* d_first_hit, int32_t* d_first_obstacle, void* stream) {
@@ -762,18 +796,9 @@ extern "C" int uam_sweep_paths_analytic(uam_ctx* ctx, const double* d_z, int64_t
     UAM_NVTX("uam.analytic.sweep");
     UAM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = uam_pick_stream(ctx, stream);
-    if (ctx->obs_gen != ctx->shapes_gen) {
-        UAM_CUDA(ctx, cudaDeviceSynchronize());      // a sweep on another stream may still read the old lists
-        UAM_TRY(uam_ensure_obs_tables(ctx, st));
-    }
-    if (ctx->obs_rc != UAM_OK) return uam_fail(ctx, ctx->obs_rc, "%s", ctx->obs_err.c_str());
-    const UamObsGrid og = ctx->shape_grid_opt ? ctx->obs_grid : UamObsGrid{};
-    const long long ctas = std::min<long long>((B + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA, (long long)ctx->sm_count * 16);
-    uam_k_sweep_analytic<<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(reinterpret_cast<const double2*>(d_z), B, N + 2,
-                                                                     ctx->d_edges, ctx->d_shapes, ctx->n_obs, og, d_flags,
-                                                                     d_first_hit, d_first_obstacle);
-    UAM_CHECK_LAUNCH(ctx, "uam_k_sweep_analytic");
-    return UAM_OK;
+    UAM_TRY(uam_ensure_obs_tables(ctx, st));
+    UAM_TRY(uam_obs_supported(ctx, false));
+    return uam_sweep_analytic_enqueue(ctx, d_z, B, N, d_flags, d_first_hit, d_first_obstacle, st);
 }
 
 extern "C" int uam_clearance_paths_analytic(uam_ctx* ctx, const double* d_z, int64_t B, int N, double cap, uint8_t* d_flags,
@@ -789,24 +814,9 @@ extern "C" int uam_clearance_paths_analytic(uam_ctx* ctx, const double* d_z, int
     UAM_NVTX("uam.analytic.clearance");
     UAM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = uam_pick_stream(ctx, stream);
-    if (ctx->obs_gen != ctx->shapes_gen) {
-        UAM_CUDA(ctx, cudaDeviceSynchronize());      // a sweep on another stream may still read the old lists
-        UAM_TRY(uam_ensure_obs_tables(ctx, st));
-    }
-    if (ctx->obs_rc != UAM_OK) return uam_fail(ctx, ctx->obs_rc, "%s", ctx->obs_err.c_str());
-    if (ctx->clr_rc != UAM_OK) return uam_fail(ctx, ctx->clr_rc, "%s", ctx->clr_err.c_str());
-    UamObsGrid og{};
-    if (ctx->shape_grid_opt) {
-        if (ctx->clr_gen != ctx->shapes_gen || ctx->clr_cap != cap) {
-            UAM_CUDA(ctx, cudaDeviceSynchronize());  // a clearance call on another stream may still read the old lists
-            UAM_TRY(uam_ensure_clr_lists(ctx, cap, st));
-        }
-        og = ctx->clr_grid;
-    }
-    const long long ctas = std::min<long long>((B + UAM_WARPS_PER_CTA - 1) / UAM_WARPS_PER_CTA, (long long)ctx->sm_count * 16);
-    uam_k_clearance_analytic<<<(unsigned)ctas, UAM_CTA_THREADS, 0, st>>>(
-        reinterpret_cast<const double2*>(d_z), B, N + 2, ctx->d_edges, ctx->d_shapes, ctx->d_obs_geom, ctx->n_obs, og, cap,
-        d_flags, d_clearance, d_nearest_segment, d_nearest_obstacle);
-    UAM_CHECK_LAUNCH(ctx, "uam_k_clearance_analytic");
-    return UAM_OK;
+    UAM_TRY(uam_ensure_obs_tables(ctx, st));
+    UAM_TRY(uam_obs_supported(ctx, true));
+    UAM_TRY(uam_ensure_clr_lists(ctx, cap, st));
+    return uam_clearance_analytic_enqueue(ctx, d_z, B, N, cap, d_flags, d_clearance, d_nearest_segment, d_nearest_obstacle,
+                                          st);
 }

@@ -306,6 +306,44 @@ class Engine:
             return tuple(None if t is None else t.cpu().numpy() for t in out)
         return out
 
+    def refine_raster_keepout(self, Z, N: int, p, flags: int, samples_per_cell: float, iterations: int,
+                              step_cells: float, max_step_cells: float, min_step_cells: float, margin: float = 0.0,
+                              want_clearance: bool = False):
+        """Z (B, 2(N+2)) float64 -> (Z_out f64, cost f32 (B,), collide u8 (B,), accepted i32 (B,), sweep flags u8 (B,),
+        clearance f64 (B,) | None) of uam_refine_paths_raster_keepout; clearance (capped at margin) is returned when
+        want_clearance, which needs margin > 0.  numpy in -> numpy out, CUDA tensor in -> new CUDA tensors out (Z is not
+        modified)."""
+        import torch
+        p = _f64c(p)
+        N = int(N)
+        margin = float(margin)
+        host = not _is_tensor(Z)
+        if host:
+            Z = _f64c(Z)
+            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
+                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
+            Zo = torch.from_numpy(Z).to(f'cuda:{self.device}')
+        else:
+            assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+            self._tensor_args(Z)
+            Zo = Z.clone()
+        st = self._tensor_args(Zo)
+        B = Zo.shape[0]
+        cost = torch.empty(B, dtype=torch.float32, device=Zo.device)
+        col = torch.empty(B, dtype=torch.uint8, device=Zo.device)
+        acc = torch.empty(B, dtype=torch.int32, device=Zo.device)
+        sflags = torch.empty(B, dtype=torch.uint8, device=Zo.device)
+        clear = torch.empty(B, dtype=torch.float64, device=Zo.device) if want_clearance else None
+        self._check(self._lib.uam_refine_paths_raster_keepout(
+            self._h, C.c_void_p(Zo.data_ptr()), B, N, _np_ptr(p), p.size, flags, float(samples_per_cell), int(iterations),
+            float(step_cells), float(max_step_cells), float(min_step_cells), margin, C.c_void_p(cost.data_ptr()),
+            C.c_void_p(col.data_ptr()), C.c_void_p(acc.data_ptr()), C.c_void_p(sflags.data_ptr()),
+            None if clear is None else C.c_void_p(clear.data_ptr()), st))
+        out = (Zo, cost, col, acc, sflags, clear)
+        if host:
+            return tuple(None if t is None else t.cpu().numpy() for t in out)
+        return out
+
     def sweep_raster(self, Z, N: int, want_first_hit: bool = True, want_d2min: bool = True):
         """Z (B, 2(N+2)) float64 -> (flags u8 (B,), first_hit i32 (B,) | None, d2min i32 (B,) | None) of
         uam_sweep_paths_raster: every cell each segment crosses checked against the raster's occupancy; numpy in -> numpy

@@ -48,7 +48,9 @@ class RasterMap:
     @classmethod
     def from_map(cls, m: RegionMap, H: int, W: int, geo, enlargement: float = 0.0, device: Optional[int] = None,
                  clearance: bool = False, options: Optional[dict] = None) -> 'RasterMap':
-        """Rasterise the map's regions and obstacles at the cell centres (map rebuild, config 4)."""
+        """Rasterise the map's regions and obstacles at the cell centres (map rebuild, config 4).  The map's shapes are
+        uploaded to the raster's engine as well, for refine_paths_keepout: that upload is a snapshot of the map, so after
+        changing the map's obstacles call set_obstacles(m) again."""
         rm = cls(H, W, geo, device, options)
         eng = rm.engine
         eng.set_shapes(m.obstacles, m._region_lists())
@@ -62,13 +64,21 @@ class RasterMap:
     @classmethod
     def from_arrays(cls, layers, geo, occupancy=None, device: Optional[int] = None,
                     options: Optional[dict] = None) -> 'RasterMap':
-        """Adopt existing rasters (numpy or CUDA tensors)."""
+        """Adopt existing rasters (numpy or CUDA tensors).  No shapes are uploaded: set_obstacles gives
+        refine_paths_keepout the no-fly shapes to check against."""
         L, H, W = layers.shape
         rm = cls(H, W, geo, device, options)
         rm.engine.set_raster(layers, rm.geo, occupancy)
         if _is_tensor(layers):
             rm.layers, rm.occupancy = layers, occupancy
         return rm
+
+    def set_obstacles(self, m: RegionMap):
+        """Upload the hard obstacles of the map m (m.obstacles, no regions) to the raster's engine, for
+        refine_paths_keepout: for example the footprint rectangles mapgen.dem_rectangles made from the DEM whose mask is
+        this raster's occupancy.  The upload is a snapshot: after changing m's obstacles, call it again.  It changes no
+        raster output (score_paths, cost_gradient, refine_paths, refine_paths_swept, sweep_paths)."""
+        self.engine.set_shapes(m.obstacles, [])
 
     # ---- score ---------------------------------------------------------------------------------------------
     def parameter_vector(self, weights: Sequence[float], x_start=None) -> np.ndarray:
@@ -138,6 +148,29 @@ class RasterMap:
         flags = (_lib.UAM_LENGTH_SMOOTH if length_smooth else 0) | (_lib.UAM_OWN_START if x_start is None else 0)
         return self.engine.refine_raster_swept(Z, N, self.parameter_vector(weights, x_start), flags, samples_per_cell,
                                                iterations, step_cells, max_step_cells, min_step_cells, min_d2)
+
+    def refine_paths_keepout(self, Z, weights: Sequence[float], samples_per_cell: float = 0.0, iterations: int = 20,
+                             length_smooth: bool = True, x_start=None, step_cells: float = 1.0, max_step_cells: float = 64.0,
+                             min_step_cells: float = 1.0 / 256, margin: float = 0.0):
+        """refine_paths with the analytic check against the no-fly shapes (Map.sweep_paths, Map.path_clearance) in the
+        accept test -> (Z_out, cost, collide, accepted, sweep_flags, clearance).
+
+        The shapes are the hard obstacles uploaded last to this raster's engine (from_map, set_obstacles).  A trial is
+        kept only if refine_paths would keep it, it adds no analytic sweep flag the path did not have (HIT, INVALID),
+        and, with margin > 0, its clearance capped at margin does not drop (fp64; a NaN rejects).  So a path that sweeps
+        clean against the shapes stays clean, between the raster's cell centres as well, and one that starts at least
+        margin from every obstacle ends so too (up to the clearance's rounding bound); one that starts closer never gets
+        closer.  margin is in map units (km), 0 .. 1e100; margin = 0 uses the sweep only.  cost / collide are
+        score_paths(Z_out)'s bits, sweep_flags Map.sweep_paths(Z_out)'s flags, clearance Map.path_clearance(Z_out,
+        margin)'s clearance; clearance is None when margin == 0.  A path that is already HIT may still drop to
+        collide = 0 while it cuts a shape, since that trial adds no flag.  When the analytic terms never reject a trial
+        the result is bit-identical to refine_paths.  include/uam_b200.h (uam_refine_paths_raster_keepout) has the exact
+        rule.  numpy in -> numpy out; a CUDA tensor in -> new CUDA tensors out (Z itself is not modified)."""
+        N = Z.shape[1] // 2 - 2
+        flags = (_lib.UAM_LENGTH_SMOOTH if length_smooth else 0) | (_lib.UAM_OWN_START if x_start is None else 0)
+        return self.engine.refine_raster_keepout(Z, N, self.parameter_vector(weights, x_start), flags, samples_per_cell,
+                                                 iterations, step_cells, max_step_cells, min_step_cells, margin,
+                                                 float(margin) > 0.0)
 
     def sweep_paths(self, Z, clearance: bool = True):
         """Check every cell each segment of Z (B, 2(N+2)) float64 crosses against the occupancy -> (flags, first_hit,
