@@ -216,6 +216,26 @@ class Engine:
                                                           float(samples_per_cell), _np_ptr(cost), _np_ptr(col)))
         return cost, col
 
+    def _paths_on_device(self, Z, N: int, clone: bool = False):
+        """(Z as a float64 (B, 2(N+2)) tensor on this engine's device, whether Z came from the host): a host array is
+        converted, checked and copied over; a tensor is checked, and with clone checked and then cloned."""
+        import torch
+        if not _is_tensor(Z):
+            Z = _f64c(Z)
+            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
+                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
+            return torch.from_numpy(Z).to(f'cuda:{self.device}'), True
+        assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+        if clone:
+            self._tensor_args(Z)
+            Z = Z.clone()
+        return Z, False
+
+    @staticmethod
+    def _outputs(outs, host: bool):
+        """outs as numpy arrays when the input came from the host, as they are otherwise; None stays None"""
+        return tuple(None if t is None else t.cpu().numpy() for t in outs) if host else tuple(outs)
+
     def grad_raster(self, Z, N: int, p, flags: int, samples_per_cell: float = 0.0):
         """Z (B, 2(N+2)) float64 -> (cost f32 (B,), collide u8 (B,), grad f64 (B, 2(N+2))) of the raster cost
         (uam_grad_paths_raster: cost / collide are score_raster's bits); numpy in -> numpy out, CUDA tensor in -> CUDA
@@ -223,13 +243,7 @@ class Engine:
         import torch
         p = _f64c(p)
         N = int(N)
-        host = not _is_tensor(Z)
-        if host:
-            Z = _f64c(Z)
-            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
-                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
-            Z = torch.from_numpy(Z).to(f'cuda:{self.device}')
-        assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+        Z, host = self._paths_on_device(Z, N)
         st = self._tensor_args(Z)
         B = Z.shape[0]
         cost = torch.empty(B, dtype=torch.float32, device=Z.device)
@@ -238,37 +252,31 @@ class Engine:
         self._check(self._lib.uam_grad_paths_raster(self._h, C.c_void_p(Z.data_ptr()), B, N, _np_ptr(p), p.size, flags,
                                                     float(samples_per_cell), C.c_void_p(cost.data_ptr()),
                                                     C.c_void_p(col.data_ptr()), C.c_void_p(grad.data_ptr()), st))
-        return (cost.cpu().numpy(), col.cpu().numpy(), grad.cpu().numpy()) if host else (cost, col, grad)
+        return self._outputs((cost, col, grad), host)
+
+    def _refine(self, entry, Z, N: int, p: np.ndarray, flags: int, samples_per_cell: float, iterations: int,
+                step_cells: float, max_step_cells: float, min_step_cells: float, extra_args=(), extra_outs=()):
+        """The refine_raster* calls: entry is the C entry point, extra_args its arguments after min_step_cells,
+        extra_outs the dtypes (None: a NULL pointer) of its (B,) outputs after accepted -> (Z_out, cost, collide,
+        accepted, *extra outputs)."""
+        import torch
+        Zo, host = self._paths_on_device(Z, N, clone=True)
+        st = self._tensor_args(Zo)
+        B = Zo.shape[0]
+        outs = [torch.empty(B, dtype=d, device=Zo.device) for d in (torch.float32, torch.uint8, torch.int32)]
+        outs += [None if d is None else torch.empty(B, dtype=d, device=Zo.device) for d in extra_outs]
+        self._check(entry(self._h, C.c_void_p(Zo.data_ptr()), B, N, _np_ptr(p), p.size, flags, float(samples_per_cell),
+                          int(iterations), float(step_cells), float(max_step_cells), float(min_step_cells), *extra_args,
+                          *[None if t is None else C.c_void_p(t.data_ptr()) for t in outs], st))
+        return self._outputs((Zo, *outs), host)
 
     def refine_raster(self, Z, N: int, p, flags: int, samples_per_cell: float, iterations: int, step_cells: float,
                       max_step_cells: float, min_step_cells: float):
         """Z (B, 2(N+2)) float64 -> (Z_out f64, cost f32 (B,), collide u8 (B,), accepted i32 (B,)) of
         uam_refine_paths_raster; numpy in -> numpy out, CUDA tensor in -> new CUDA tensors out (Z is not modified)."""
-        import torch
-        p = _f64c(p)
-        N = int(N)
-        host = not _is_tensor(Z)
-        if host:
-            Z = _f64c(Z)
-            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
-                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
-            Zo = torch.from_numpy(Z).to(f'cuda:{self.device}')
-        else:
-            assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
-            self._tensor_args(Z)
-            Zo = Z.clone()
-        st = self._tensor_args(Zo)
-        B = Zo.shape[0]
-        cost = torch.empty(B, dtype=torch.float32, device=Zo.device)
-        col = torch.empty(B, dtype=torch.uint8, device=Zo.device)
-        acc = torch.empty(B, dtype=torch.int32, device=Zo.device)
-        self._check(self._lib.uam_refine_paths_raster(
-            self._h, C.c_void_p(Zo.data_ptr()), B, N, _np_ptr(p), p.size, flags, float(samples_per_cell), int(iterations),
-            float(step_cells), float(max_step_cells), float(min_step_cells), C.c_void_p(cost.data_ptr()),
-            C.c_void_p(col.data_ptr()), C.c_void_p(acc.data_ptr()), st))
-        if host:
-            return Zo.cpu().numpy(), cost.cpu().numpy(), col.cpu().numpy(), acc.cpu().numpy()
-        return Zo, cost, col, acc
+        p, N = _f64c(p), int(N)
+        return self._refine(self._lib.uam_refine_paths_raster, Z, N, p, flags, samples_per_cell, iterations, step_cells,
+                            max_step_cells, min_step_cells)
 
     def refine_raster_swept(self, Z, N: int, p, flags: int, samples_per_cell: float, iterations: int, step_cells: float,
                             max_step_cells: float, min_step_cells: float, min_d2: int = 0, want_d2min: bool = False):
@@ -276,35 +284,10 @@ class Engine:
         d2min i32 (B,) | None) of uam_refine_paths_raster_swept; d2min is returned when want_d2min or min_d2 > 0.
         numpy in -> numpy out, CUDA tensor in -> new CUDA tensors out (Z is not modified)."""
         import torch
-        p = _f64c(p)
-        N = int(N)
-        min_d2 = operator.index(min_d2)
-        host = not _is_tensor(Z)
-        if host:
-            Z = _f64c(Z)
-            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
-                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
-            Zo = torch.from_numpy(Z).to(f'cuda:{self.device}')
-        else:
-            assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
-            self._tensor_args(Z)
-            Zo = Z.clone()
-        st = self._tensor_args(Zo)
-        B = Zo.shape[0]
-        cost = torch.empty(B, dtype=torch.float32, device=Zo.device)
-        col = torch.empty(B, dtype=torch.uint8, device=Zo.device)
-        acc = torch.empty(B, dtype=torch.int32, device=Zo.device)
-        sflags = torch.empty(B, dtype=torch.uint8, device=Zo.device)
-        d2min = torch.empty(B, dtype=torch.int32, device=Zo.device) if want_d2min or min_d2 > 0 else None
-        self._check(self._lib.uam_refine_paths_raster_swept(
-            self._h, C.c_void_p(Zo.data_ptr()), B, N, _np_ptr(p), p.size, flags, float(samples_per_cell), int(iterations),
-            float(step_cells), float(max_step_cells), float(min_step_cells), min_d2, C.c_void_p(cost.data_ptr()),
-            C.c_void_p(col.data_ptr()), C.c_void_p(acc.data_ptr()), C.c_void_p(sflags.data_ptr()),
-            None if d2min is None else C.c_void_p(d2min.data_ptr()), st))
-        out = (Zo, cost, col, acc, sflags, d2min)
-        if host:
-            return tuple(None if t is None else t.cpu().numpy() for t in out)
-        return out
+        p, N, min_d2 = _f64c(p), int(N), operator.index(min_d2)
+        return self._refine(self._lib.uam_refine_paths_raster_swept, Z, N, p, flags, samples_per_cell, iterations,
+                            step_cells, max_step_cells, min_step_cells, (min_d2,),
+                            (torch.uint8, torch.int32 if want_d2min or min_d2 > 0 else None))
 
     def refine_raster_keepout(self, Z, N: int, p, flags: int, samples_per_cell: float, iterations: int,
                               step_cells: float, max_step_cells: float, min_step_cells: float, margin: float = 0.0,
@@ -314,35 +297,10 @@ class Engine:
         want_clearance, which needs margin > 0.  numpy in -> numpy out, CUDA tensor in -> new CUDA tensors out (Z is not
         modified)."""
         import torch
-        p = _f64c(p)
-        N = int(N)
-        margin = float(margin)
-        host = not _is_tensor(Z)
-        if host:
-            Z = _f64c(Z)
-            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
-                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
-            Zo = torch.from_numpy(Z).to(f'cuda:{self.device}')
-        else:
-            assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
-            self._tensor_args(Z)
-            Zo = Z.clone()
-        st = self._tensor_args(Zo)
-        B = Zo.shape[0]
-        cost = torch.empty(B, dtype=torch.float32, device=Zo.device)
-        col = torch.empty(B, dtype=torch.uint8, device=Zo.device)
-        acc = torch.empty(B, dtype=torch.int32, device=Zo.device)
-        sflags = torch.empty(B, dtype=torch.uint8, device=Zo.device)
-        clear = torch.empty(B, dtype=torch.float64, device=Zo.device) if want_clearance else None
-        self._check(self._lib.uam_refine_paths_raster_keepout(
-            self._h, C.c_void_p(Zo.data_ptr()), B, N, _np_ptr(p), p.size, flags, float(samples_per_cell), int(iterations),
-            float(step_cells), float(max_step_cells), float(min_step_cells), margin, C.c_void_p(cost.data_ptr()),
-            C.c_void_p(col.data_ptr()), C.c_void_p(acc.data_ptr()), C.c_void_p(sflags.data_ptr()),
-            None if clear is None else C.c_void_p(clear.data_ptr()), st))
-        out = (Zo, cost, col, acc, sflags, clear)
-        if host:
-            return tuple(None if t is None else t.cpu().numpy() for t in out)
-        return out
+        p, N, margin = _f64c(p), int(N), float(margin)
+        return self._refine(self._lib.uam_refine_paths_raster_keepout, Z, N, p, flags, samples_per_cell, iterations,
+                            step_cells, max_step_cells, min_step_cells, (margin,),
+                            (torch.uint8, torch.float64 if want_clearance else None))
 
     def sweep_raster(self, Z, N: int, want_first_hit: bool = True, want_d2min: bool = True):
         """Z (B, 2(N+2)) float64 -> (flags u8 (B,), first_hit i32 (B,) | None, d2min i32 (B,) | None) of
@@ -350,13 +308,7 @@ class Engine:
         out, CUDA tensor in -> CUDA tensors out."""
         import torch
         N = int(N)
-        host = not _is_tensor(Z)
-        if host:
-            Z = _f64c(Z)
-            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
-                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
-            Z = torch.from_numpy(Z).to(f'cuda:{self.device}')
-        assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+        Z, host = self._paths_on_device(Z, N)
         st = self._tensor_args(Z)
         B = Z.shape[0]
         flags = torch.empty(B, dtype=torch.uint8, device=Z.device)
@@ -365,9 +317,7 @@ class Engine:
         self._check(self._lib.uam_sweep_paths_raster(self._h, C.c_void_p(Z.data_ptr()), B, N, C.c_void_p(flags.data_ptr()),
                                                      C.c_void_p(first.data_ptr()) if want_first_hit else None,
                                                      C.c_void_p(d2min.data_ptr()) if want_d2min else None, st))
-        if host:
-            return tuple(None if t is None else t.cpu().numpy() for t in (flags, first, d2min))
-        return flags, first, d2min
+        return self._outputs((flags, first, d2min), host)
 
     def sweep_analytic(self, Z, N: int, want_first_hit: bool = True, want_first_obstacle: bool = True):
         """Z (B, 2(N+2)) float64 -> (flags u8 (B,), first_hit i32 (B,) | None, first_obstacle i32 (B,) | None) of
@@ -375,13 +325,7 @@ class Engine:
         tensor in -> CUDA tensors out."""
         import torch
         N = int(N)
-        host = not _is_tensor(Z)
-        if host:
-            Z = _f64c(Z)
-            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
-                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
-            Z = torch.from_numpy(Z).to(f'cuda:{self.device}')
-        assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+        Z, host = self._paths_on_device(Z, N)
         st = self._tensor_args(Z)
         B = Z.shape[0]
         flags = torch.empty(B, dtype=torch.uint8, device=Z.device)
@@ -390,9 +334,7 @@ class Engine:
         self._check(self._lib.uam_sweep_paths_analytic(self._h, C.c_void_p(Z.data_ptr()), B, N, C.c_void_p(flags.data_ptr()),
                                                        C.c_void_p(first.data_ptr()) if want_first_hit else None,
                                                        C.c_void_p(obst.data_ptr()) if want_first_obstacle else None, st))
-        if host:
-            return tuple(None if t is None else t.cpu().numpy() for t in (flags, first, obst))
-        return flags, first, obst
+        return self._outputs((flags, first, obst), host)
 
     def clearance_analytic(self, Z, N: int, cap: float, want_nearest: bool = True):
         """Z (B, 2(N+2)) float64 -> (flags u8 (B,), clearance f64 (B,), nearest_segment i32 (B,) | None, nearest_obstacle
@@ -400,13 +342,7 @@ class Engine:
         cap; numpy in -> numpy out, CUDA tensor in -> CUDA tensors out."""
         import torch
         N = int(N)
-        host = not _is_tensor(Z)
-        if host:
-            Z = _f64c(Z)
-            if Z.ndim != 2 or Z.shape[1] != 2 * (N + 2):
-                raise ValueError(f'paths must be (B, {2 * (N + 2)}) for N = {N}, got {Z.shape}')
-            Z = torch.from_numpy(Z).to(f'cuda:{self.device}')
-        assert Z.dtype == torch.float64 and Z.dim() == 2 and Z.shape[1] == 2 * (N + 2)
+        Z, host = self._paths_on_device(Z, N)
         st = self._tensor_args(Z)
         B = Z.shape[0]
         flags = torch.empty(B, dtype=torch.uint8, device=Z.device)
@@ -416,9 +352,7 @@ class Engine:
         ptr = (lambda t: None if t is None else C.c_void_p(t.data_ptr()))
         self._check(self._lib.uam_clearance_paths_analytic(self._h, ptr(Z), B, N, float(cap), ptr(flags), ptr(clear), ptr(seg),
                                                            ptr(obst), st))
-        if host:
-            return tuple(None if t is None else t.cpu().numpy() for t in (flags, clear, seg, obst))
-        return flags, clear, seg, obst
+        return self._outputs((flags, clear, seg, obst), host)
 
     def score_raster_best(self, Z, N: int, p, flags: int, samples_per_cell: float, global_offset: int = 0, out=None, key=None):
         """score_raster on a CUDA tensor + the best key of the batch -- of every rank's batch when a peer group is attached
