@@ -93,12 +93,15 @@ enum {
                                          CUDA events on the caller's stream (resets the statistics) */
     UAM_OPT_GRID_DELTA = 6,           /* grid search: width of the distance window relaxed per round (0 = automatic: the cost
                                          of crossing one 32-cell tile at the mean cell cost); ordering only, same results */
-    UAM_OPT_COMBINE_LAYERS = 5,       /* 1 (default): large-batch integral mode samples "quad texels": the layers are folded
-                                         into ONE layer sum_l w_l * layer_l (the penalty is linear in the layers) and every
-                                         cell stores its 2 x 2 bilinear footprint as one float4, so a tap is one 16-byte
-                                         load; occupancy flags ride in the sign bits when all values are >= 0, else in a
-                                         bit-plane.  Rebuilt when the weights or the raster change.  2: as 1 but always the
-                                         bit-plane form.  0: always sample every layer texel by texel */
+    UAM_OPT_COMBINE_LAYERS = 5,       /* 1 (default): large-batch integral mode (and waypoint mode) samples the layers folded
+                                         into ONE layer sum_l w_l * layer_l (the penalty is linear in the layers).  First
+                                         choice is the "gather layer": 4 bytes per cell in a 2-D CUDA array, occupancy in
+                                         the sign bits, a tap is one tex2Dgather of the 2 x 2 bilinear footprint.  Integral
+                                         variant 3, rasters beyond the device's gather limits and folded values < 0 use
+                                         "quad texels" instead: every cell stores its footprint as one float4, a tap is one
+                                         16-byte load; occupancy flags ride in the sign bits when all values are >= 0, else
+                                         in a bit-plane.  Rebuilt when the weights or the raster change.  2: always the
+                                         quad texels with the bit-plane.  0: always sample every layer texel by texel */
     UAM_OPT_HOST_CHUNKS = 7,          /* uam_score_paths_raster_host: chunks per call flowing through the copy / score
                                          pipeline (0 = default 4) */
     UAM_OPT_HOST_TAPER = 8,           /* ... chunk sizes change linearly from the first to the last chunk: t > 0 the last chunk

@@ -96,6 +96,8 @@ extern "C" int uam_ctx_create(int device, uam_ctx** out) {
     ctx->device = device;
     if (cudaSetDevice(device) != cudaSuccess) { delete ctx; return UAM_ERR_CUDA; }
     cudaDeviceGetAttribute(&ctx->sm_count, cudaDevAttrMultiProcessorCount, device);
+    cudaDeviceGetAttribute(&ctx->gather_max_w, cudaDevAttrMaxTexture2DGatherWidth, device);
+    cudaDeviceGetAttribute(&ctx->gather_max_h, cudaDevAttrMaxTexture2DGatherHeight, device);
     if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) { delete ctx; return UAM_ERR_CUDA; }
     for (int i = 0; i < UAM_HOST_PIPE_DEPTH; ++i) {
         if (cudaStreamCreateWithFlags(&ctx->pipe_stream[i], cudaStreamNonBlocking) != cudaSuccess ||
@@ -263,6 +265,8 @@ extern "C" int uam_ctx_destroy(uam_ctx* ctx) {
     for (int i = 0; i <= UAM_HOST_PIPE_DEPTH; ++i) cudaFree(ctx->d_piece_scratch[i]);
     cudaFree(ctx->d_tiles);
     cudaFree(ctx->d_tex_comb);
+    if (ctx->gather_tex) cudaDestroyTextureObject(ctx->gather_tex);
+    cudaFreeArray(ctx->gather_arr);
     cudaFree(ctx->d_occ_bits);
     cudaFree(ctx->d_refine_scratch);
     cudaFree(ctx->d_sweep_d2);

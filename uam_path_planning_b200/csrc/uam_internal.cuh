@@ -93,9 +93,11 @@ struct UamRasterParams {
     float w0, w1, w2;     // combined with L = 2..3: {1, 0, 0}, the weights are inside the quads
     int flags;
     int variant;          // integral-mode kernel, decided once per API call from the call's whole batch
-    int combined;         // score on the quad texels (ctx->d_tex_comb): 1 = + bit-plane, 2 = sign-packed
+    int combined;         // score on the weight-folded layer: 1 = quad texels (ctx->d_tex_comb) + bit-plane, 2 = sign-packed
+                          // quad texels, 3 = sign-packed gather layer (gather_tex)
     const unsigned* occ_bits;   // quad mode: occupancy bit-plane (uam_occ_word / uam_occ_bit)
     unsigned occ_blocks_x;      // 32 x 32-cell blocks per block-row of the bit-plane
+    unsigned long long gather_tex;   // combined == 3: texture object of ctx->gather_arr
 };
 
 // ---- best-candidate exchange between the ranks of one box (uam_best.cu) -------------------------------------------
@@ -213,6 +215,14 @@ struct uam_ctx {
     size_t occ_bits_bytes = 0;
     bool occ_bits_valid = false;
     bool comb_packed = false;           // quads carry the occupancy flags in their sign bits
+    // gather layer: the folded layer, 4 bytes per cell (sign bit = occupancy), in a 2-D CUDA array read by tex2Dgather;
+    // made instead of the quads when the raster fits gather_max_w x gather_max_h and the folded values are >= 0
+    cudaArray_t gather_arr = nullptr;
+    cudaTextureObject_t gather_tex = 0;
+    int gather_w = 0, gather_h = 0;     // dimensions of gather_arr
+    int gather_max_w = 0, gather_max_h = 0;   // cudaDevAttrMaxTexture2DGatherWidth / Height of the device
+    bool comb_gather = false;           // the valid folded form is the gather layer (else the quads)
+    bool comb_want_gather = false;      // ... and it was built for a call that asked for the gather layer
     int no_sign_pack = 0;               // UAM_NO_SIGN_PACK=1 forces the bit-plane form (tests)
     float comb_w[3] = {};
     uint64_t comb_gen = 0, raster_gen = 0;

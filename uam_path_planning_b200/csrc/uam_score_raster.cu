@@ -36,7 +36,11 @@ template <> struct UamTexel<2> { typedef float2 T; };
 template <> struct UamTexel<4> { typedef float4 T; };
 template <> struct UamTexel<1> { typedef float4 T; };      // quad mode: the 2 x 2 bilinear footprint of a cell in one texel
 template <> struct UamTexel<8> { typedef float4 T; };      // quad mode, occupancy flags in the sign bits (values >= 0)
-template <int TF> struct UamIsQuad { static const bool v = (TF == 1 || TF == 8); };
+template <> struct UamTexel<16> { typedef unsigned T; };   // gather layer: the kernels read rp.gather_tex, not the pointer
+// forms that sample the weight-folded layer with one load per tap (quads or the gather layer)
+template <int TF> struct UamIsFolded { static const bool v = (TF == 1 || TF == 8 || TF == 16); };
+// forms whose values are >= 0 and carry the occupancy flags in their sign bits
+template <int TF> struct UamSignPacked { static const bool v = (TF == 8 || TF == 16); };
 
 // Texel address = uam_tex_row(i) + uam_tex_col(j)  (both layouts are separable).
 // LAYOUT 0: row-major (H, W).  LAYOUT 1: tiled so that one 128-byte line is a compact 2-D block and every 32-byte
@@ -126,6 +130,18 @@ struct UamTap<8> {
     float fx, fy;
 };
 
+// gather layer: one tex2Dgather (TLD4) returns the bits of the four corner values, sign-packed like TF 8's, in the gather
+// order (i0+1,j0) (i0+1,j0+1) (i0,j0+1) (i0,j0) -- TF 8's q.x, q.y, q.z, q.w are g.w, g.z, g.x, g.y
+template <>
+struct UamTap<16> {
+    uint4 g;
+    float fx, fy;
+};
+
+// unnormalised texture coordinate c + 1 (0 <= c < 2^23 - 1) as 2^23 + c + 1 assembled as bits, minus 2^23: a LOP3 and an
+// FADD instead of the conversion unit.  Gathering at (j0 + 1, i0 + 1) returns exactly texels j0..j0+1 x i0..i0+1.
+__device__ __forceinline__ float uam_tex_coord(int c) { return __int_as_float(0x4B000000 | (c + 1)) - 8388608.0f; }
+
 template <int TF, int LAYOUT, bool CLAMP = true>
 __device__ __forceinline__ void uam_tap_load(const typename UamTexel<TF>::T* __restrict__ tex, const UamRasterParams& rp,
                                              double u, double v, UamTap<TF>& t) {
@@ -137,7 +153,9 @@ __device__ __forceinline__ void uam_tap_load(const typename UamTexel<TF>::T* __r
         uam_cell_frac1_inside(u, j0, t.fx);
         uam_cell_frac1_inside(v, i0, t.fy);
     }
-    if constexpr (TF == 8) {
+    if constexpr (TF == 16) {
+        t.g = tex2Dgather<uint4>(rp.gather_tex, uam_tex_coord(j0), uam_tex_coord(i0), 0);
+    } else if constexpr (TF == 8) {
         t.q = __ldg(tex + uam_quad_index<LAYOUT>(i0, j0, rp.row_stride));
     } else if constexpr (TF == 1) {
         t.q = __ldg(tex + uam_quad_index<LAYOUT>(i0, j0, rp.row_stride));
@@ -156,7 +174,13 @@ __device__ __forceinline__ void uam_tap_load(const typename UamTexel<TF>::T* __r
 
 template <int TF>
 __device__ __forceinline__ void uam_tap_eval(const UamRasterParams& rp, const UamTap<TF>& t, float& pen, bool& occ) {
-    if constexpr (TF == 8) {
+    if constexpr (TF == 16) {
+        pen = rp.w0 * uam_lerp2(fabsf(__uint_as_float(t.g.w)), fabsf(__uint_as_float(t.g.z)), fabsf(__uint_as_float(t.g.x)),
+                                fabsf(__uint_as_float(t.g.y)), t.fx, t.fy);
+        const bool right = t.fx >= 0.5f, down = t.fy >= 0.5f;
+        const unsigned o = down ? (right ? t.g.y : t.g.x) : (right ? t.g.z : t.g.w);
+        occ = (int)o < 0;
+    } else if constexpr (TF == 8) {
         pen = rp.w0 * uam_lerp2(fabsf(t.q.x), fabsf(t.q.y), fabsf(t.q.z), fabsf(t.q.w), t.fx, t.fy);
         const bool right = t.fx >= 0.5f, down = t.fy >= 0.5f;
         const float o = down ? (right ? t.q.w : t.q.z) : (right ? t.q.y : t.q.x);
@@ -190,7 +214,11 @@ __device__ __forceinline__ void uam_lerp2_grad(float t00, float t01, float t10, 
 template <int TF>
 __device__ __forceinline__ void uam_tap_grad(const UamRasterParams& rp, const UamTap<TF>& t, float& pen, bool& occ, float& du, float& dv) {
     uam_tap_eval<TF>(rp, t, pen, occ);
-    if constexpr (TF == 8) {
+    if constexpr (TF == 16) {
+        uam_lerp2_grad(fabsf(__uint_as_float(t.g.w)), fabsf(__uint_as_float(t.g.z)), fabsf(__uint_as_float(t.g.x)),
+                       fabsf(__uint_as_float(t.g.y)), t.fx, t.fy, du, dv);
+        du *= rp.w0; dv *= rp.w0;
+    } else if constexpr (TF == 8) {
         uam_lerp2_grad(fabsf(t.q.x), fabsf(t.q.y), fabsf(t.q.z), fabsf(t.q.w), t.fx, t.fy, du, dv);
         du *= rp.w0; dv *= rp.w0;
     } else if constexpr (TF == 1) {
@@ -906,6 +934,7 @@ struct __align__(16) UamGroupRec {
 template <int TF> struct UamTapsPerTrip { static const int N = 2; };
 template <> struct UamTapsPerTrip<1> { static const int N = 4; };
 template <> struct UamTapsPerTrip<8> { static const int N = 4; };
+template <> struct UamTapsPerTrip<16> { static const int N = 4; };
 
 // GRAD: four more 32 x 33 partial matrices behind the group's shared memory, for the per-record sums of dP/du, s dP/du,
 // dP/dv and s dP/dv (s = the sample's number in its record); flushed and reduced exactly like the penalty partials.
@@ -1150,7 +1179,7 @@ __device__ __forceinline__ void uam_group_score(const UamRasterParams& rp, const
 // on the C3 shard (B200 at 1000 W) the kernel takes 1.455 ms at 3 CTAs, 1.531 ms at 4 and 1.604 ms at 2
 // (profiles/r03_ab_group_occupancy.txt).
 template <int TF, int LAYOUT, bool GRAD = false>
-__global__ void __launch_bounds__(UAM_CTA_THREADS, GRAD ? 1 : (UamIsQuad<TF>::v ? 3 : 4))
+__global__ void __launch_bounds__(UAM_CTA_THREADS, GRAD ? 1 : (UamIsFolded<TF>::v ? 3 : 4))
 uam_k_score_groups(unsigned long long n_seg, int Wp, UamRasterParams rp, const typename UamTexel<TF>::T* __restrict__ tex,
                    const double2* __restrict__ z, const unsigned* __restrict__ sorted_id, float* __restrict__ part_pen,
                    uint8_t* __restrict__ part_col, unsigned* __restrict__ next_group, float4* __restrict__ part_grad) {
@@ -1183,9 +1212,9 @@ uam_k_score_groups(unsigned long long n_seg, int Wp, UamRasterParams rp, const t
             if (have) part_grad[r.id] = uam_seg_grad(gmine, r.IS);
         }
         if (have) {
-            if (TF == 8 && rp.w0 >= 0.0f) {
-                // sign-packed quads with a weight >= 0: every tap is >= 0, so the partial is >= 0 (or NaN) and its sign bit is
-                // free to carry the collision flag (-0.0f = "0, occupied"): one scattered 4-byte store per segment instead of
+            if (UamSignPacked<TF>::v && rp.w0 >= 0.0f) {
+                // sign-packed quads or gather layer with a weight >= 0: every tap is >= 0, so the partial is >= 0 (or NaN) and
+                // its sign bit is free to carry the collision flag (-0.0f = "0, occupied"): one scattered 4-byte store per segment instead of
                 // 4 + 1 bytes (uam_k_reduce_paths<., 1> reads it back)
                 part_pen[r.id] = __uint_as_float((__float_as_uint(mine * r.IS) & 0x7fffffffu) | (col ? 0x80000000u : 0u));
             } else {
@@ -1198,7 +1227,7 @@ uam_k_score_groups(unsigned long long n_seg, int Wp, UamRasterParams rp, const t
 
 // one warp per path: fixed-order sum of the per-segment partials + the length term
 // BEST: the launch also finds the best candidate (and exchanges it with the peer ranks): uam_best_tail_cta
-// PACKED: the collision flag is the sign bit of the partial (uam_k_score_groups<8>), part_col is not read.
+// PACKED: the collision flag is the sign bit of the partial (uam_k_score_groups<8> / <16>), part_col is not read.
 // len_path: the paths' length terms from uam_k_bin_hist (the waypoints are then read only when nsamp is asked for).
 // GRAD: also grad: waypoint j = segment j's start share + segment j-1's end share (part_grad, fp32, in that order) + the
 // fp64 length part.
@@ -1681,7 +1710,7 @@ __global__ void uam_k_build_tiles(const typename UamTexel<TF>::T* __restrict__ t
         const unsigned i = (tile / (unsigned)tg.tiles_x) * UAM_TS + li, j = (tile % (unsigned)tg.tiles_x) * UAM_TS + lj;
         T v;
         if (i < (unsigned)rp.H && j < (unsigned)rp.W) {
-            v = tex[uam_tex_row<(UamIsQuad<TF>::v ? 4 : TF), LAYOUT>(i, rp.row_stride) + uam_tex_col<(UamIsQuad<TF>::v ? 4 : TF), LAYOUT>(j)];
+            v = tex[uam_tex_row<(UamIsFolded<TF>::v ? 4 : TF), LAYOUT>(i, rp.row_stride) + uam_tex_col<(UamIsFolded<TF>::v ? 4 : TF), LAYOUT>(j)];
         } else {
             if constexpr (TF == 2) v = make_float2(0.0f, 0.0f); else v = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         }
@@ -1798,7 +1827,7 @@ int uam_raster_launch_binned(uam_ctx* ctx, const void* texv, const double2* z, i
     }
     const long long rctas = std::min<long long>((B + 4 * UAM_WARPS_PER_CTA - 1) / (4 * UAM_WARPS_PER_CTA), (long long)ctx->sm_count * 16);   // 4 paths per warp and trip
     UAM_NVTX("uam.raster.reduce+best");
-    const bool packed = TF == 8 && rp.w0 >= 0.0f;       // the condition uam_k_score_groups tests
+    const bool packed = UamSignPacked<TF>::v && rp.w0 >= 0.0f;       // the condition uam_k_score_groups tests
     const UamBestTail tl = best ? *best : UamBestTail{};
     const auto reduce = d_grad ? (packed ? uam_k_reduce_paths<0, 1, true> : uam_k_reduce_paths<0, 0, true>)
                       : best   ? (packed ? uam_k_reduce_paths<1, 1> : uam_k_reduce_paths<1, 0>)
@@ -1913,7 +1942,7 @@ int uam_raster_launch_t(uam_ctx* ctx, const void* texv, uint64_t tex_key, const 
         return UAM_OK;
     }
     if (rp.variant >= 2 && (unsigned long long)B * Wp < 0xffffffffull) {
-        if constexpr (!GRAD) {
+        if constexpr (!GRAD && TF != 16) {
             if (rp.variant == 3 && (rp.W + UAM_TS - 1) / UAM_TS + (rp.H + UAM_TS - 1) / UAM_TS < 65535) {
                 bool fell_back = false;
                 UAM_TRY((uam_raster_launch_tiles<TF, LAYOUT>(ctx, texv, tex_key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, &fell_back)));
@@ -1922,8 +1951,8 @@ int uam_raster_launch_t(uam_ctx* ctx, const void* texv, uint64_t tex_key, const 
         }
         return uam_raster_launch_binned<TF, LAYOUT>(ctx, texv, z, B, Wp, rp, d_cost, d_collide, d_nsamp, st, slot, best, best_done, d_grad);
     }
-    if constexpr (UamIsQuad<TF>::v) {
-        return uam_fail(ctx, UAM_ERR_STATE, "quad texels are not sampled by the warp-per-path integral kernels");
+    if constexpr (UamIsFolded<TF>::v) {
+        return uam_fail(ctx, UAM_ERR_STATE, "the folded layer is not sampled by the warp-per-path integral kernels");
     } else {
         const size_t per_warp = uam_seg_table_bytes(Wp) + (GRAD ? (size_t)Wp * sizeof(float4) : 0);
         const size_t budget = 200 * 1024;
@@ -1956,6 +1985,21 @@ int uam_raster_launch_t(uam_ctx* ctx, const void* texv, uint64_t tex_key, const 
 // Built per (raster, weights) and kept until either changes.
 // PACK = 1: store occupied cells' values negated (sign bit = occupancy flag; needs every value >= 0: a negative or NaN
 // value raises *bad and the caller rebuilds with PACK = 0 + the bit-plane).
+// The folded value of cell (i, j) of the raster's texels (quads and gather layer alike).
+template <int TF, int LAYOUT, int PACK>
+__device__ __forceinline__ float uam_fold_value(const typename UamTexel<TF>::T* __restrict__ tex, int i, int j, unsigned rs_src,
+                                                float w0, float w1, float w2, bool& neg) {
+    const typename UamTexel<TF>::T t = tex[uam_tex_row<TF, LAYOUT>(i, rs_src) + uam_tex_col<TF, LAYOUT>(j)];
+    float c, o;
+    if constexpr (TF == 2) { c = t.x; o = t.y; } else { c = w0 * t.x + w1 * t.y + w2 * t.z; o = t.w; }
+    if constexpr (PACK) {
+        neg = neg || !(c >= 0.0f);
+        c = fabsf(c);                    // -0.0 -> +0.0
+        if (o != 0.0f) c = -c;
+    }
+    return c;
+}
+
 template <int TF, int LAYOUT, int PACK>
 __global__ void uam_k_build_quads(const typename UamTexel<TF>::T* __restrict__ tex, int H, int W, unsigned rs_src, unsigned rs_q,
                                   float w0, float w1, float w2, size_t n_out, float4* __restrict__ quad, unsigned* __restrict__ bad) {
@@ -1963,15 +2007,7 @@ __global__ void uam_k_build_quads(const typename UamTexel<TF>::T* __restrict__ t
     bool neg = false;
     auto value = [&](int i, int j) -> float {
         if (i >= H || j >= W) return 0.0f;
-        const typename UamTexel<TF>::T t = tex[uam_tex_row<TF, LAYOUT>(i, rs_src) + uam_tex_col<TF, LAYOUT>(j)];
-        float c, o;
-        if constexpr (TF == 2) { c = t.x; o = t.y; } else { c = w0 * t.x + w1 * t.y + w2 * t.z; o = t.w; }
-        if constexpr (PACK) {
-            neg = neg || !(c >= 0.0f);
-            c = fabsf(c);                    // -0.0 -> +0.0
-            if (o != 0.0f) c = -c;
-        }
-        return c;
+        return uam_fold_value<TF, LAYOUT, PACK>(tex, i, j, rs_src, w0, w1, w2, neg);
     };
     for (size_t o = (size_t)blockIdx.x * blockDim.x + threadIdx.x; o < n_out; o += stride) {
         int i, j;                     // o -> cell of the float4 layout (one thread per output texel, coalesced stores)
@@ -1988,6 +2024,20 @@ __global__ void uam_k_build_quads(const typename UamTexel<TF>::T* __restrict__ t
         quad[o] = make_float4(value(i, j), value(i, j + 1), value(i + 1, j), value(i + 1, j + 1));
     }
     if (PACK && neg) atomicOr(bad, 1u);
+}
+
+// Gather layer, staged row-major (H, W) in `out` for the copy into the CUDA array: the bits of the sign-packed folded
+// value of every cell, the value the four sign-packed quads that share the cell hold.  A negative or NaN value raises *bad.
+template <int TF, int LAYOUT>
+__global__ void uam_k_build_gather(const typename UamTexel<TF>::T* __restrict__ tex, int H, int W, unsigned rs_src, float w0,
+                                   float w1, float w2, unsigned* __restrict__ out, unsigned* __restrict__ bad) {
+    const unsigned n = (unsigned)H * (unsigned)W, stride = gridDim.x * blockDim.x;     // (< 2^32: uam_map_set_raster)
+    bool neg = false;
+    for (unsigned o = blockIdx.x * blockDim.x + threadIdx.x; o < n; o += stride) {
+        const int i = (int)(o / (unsigned)W), j = (int)(o - (unsigned)i * (unsigned)W);
+        out[o] = __float_as_uint(uam_fold_value<TF, LAYOUT, 1>(tex, i, j, rs_src, w0, w1, w2, neg));
+    }
+    if (neg) atomicOr(bad, 1u);
 }
 
 // one thread per 32-bit word (8 x 4 cells) of the occupancy bit-plane
@@ -2033,36 +2083,104 @@ int uam_build_quads_t(uam_ctx* ctx, const UamRasterParams& rp, unsigned rs_q, si
     return UAM_OK;
 }
 
-// Makes the quad texels of the raster and rp's weights (unless the last ones still fit), then points rp at them: the row
-// stride becomes the quads', and the weights of an L = 2..3 raster, now inside the quads, become {1, 0, 0}.
+// Gather layer of the raster and rp's weights: folds the layer into ctx->d_tex_comb (staging) and copies it into
+// ctx->gather_arr, (re)made when the raster's dimensions change.  *ok = false when a folded value is negative or NaN (the
+// sign bits cannot carry the occupancy flags; the caller makes the bit-plane quads instead).
+template <int TF, int LAYOUT>
+int uam_build_gather_t(uam_ctx* ctx, const UamRasterParams& rp, cudaStream_t st, bool* ok) {
+    typedef typename UamTexel<TF>::T T;
+    const int H = rp.H, W = rp.W;
+    if (ctx->gather_arr && (ctx->gather_w != W || ctx->gather_h != H)) {
+        UAM_CUDA(ctx, cudaDestroyTextureObject(ctx->gather_tex));
+        UAM_CUDA(ctx, cudaFreeArray(ctx->gather_arr));
+        ctx->gather_tex = 0;
+        ctx->gather_arr = nullptr;
+    }
+    if (!ctx->gather_arr) {
+        const cudaChannelFormatDesc desc = cudaCreateChannelDesc<unsigned>();    // integer texels come back bit for bit
+        UAM_CUDA(ctx, cudaMallocArray(&ctx->gather_arr, &desc, (size_t)W, (size_t)H, cudaArrayTextureGather));
+        cudaResourceDesc rd = {};
+        rd.resType = cudaResourceTypeArray;
+        rd.res.array.array = ctx->gather_arr;
+        cudaTextureDesc td = {};
+        td.addressMode[0] = td.addressMode[1] = cudaAddressModeClamp;
+        td.filterMode = cudaFilterModePoint;
+        td.readMode = cudaReadModeElementType;
+        td.normalizedCoords = 0;
+        const cudaError_t e = cudaCreateTextureObject(&ctx->gather_tex, &rd, &td, nullptr);
+        if (e != cudaSuccess) {
+            cudaFreeArray(ctx->gather_arr);
+            ctx->gather_arr = nullptr;
+            ctx->gather_tex = 0;
+            return uam_cuda_fail(ctx, e, "cudaCreateTextureObject (gather layer)");
+        }
+        ctx->gather_w = W;
+        ctx->gather_h = H;
+    }
+    const size_t row = (size_t)W * 4;
+    UAM_TRY(uam_reserve(ctx, &ctx->d_tex_comb, &ctx->tex_comb_bytes, row * H));
+    unsigned* bad = (unsigned*)ctx->d_occ_bits;
+    UAM_CUDA(ctx, cudaMemsetAsync(bad, 0, 4, st));
+    uam_k_build_gather<TF, LAYOUT><<<ctx->sm_count * 8, 256, 0, st>>>((const T*)ctx->d_tex, H, W, rp.row_stride, rp.w0, rp.w1, rp.w2,
+                                                                       (unsigned*)ctx->d_tex_comb, bad);
+    UAM_CHECK_LAUNCH(ctx, "uam_k_build_gather");
+    UAM_CUDA(ctx, cudaMemcpy2DToArrayAsync(ctx->gather_arr, 0, 0, ctx->d_tex_comb, row, row, H, cudaMemcpyDeviceToDevice, st));
+    unsigned h_bad = 0;
+    UAM_CUDA(ctx, cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, st));
+    UAM_CUDA(ctx, cudaStreamSynchronize(st));
+    *ok = !h_bad;
+    return UAM_OK;
+}
+
+// Makes the weight-folded layer of the raster and rp's weights (unless the last one still fits), then points rp at it.
+// First choice is the gather layer; the quads are made instead for the tile-staged variant 3 (it copies quads into
+// shared memory), for rasters beyond the device's gather limits, when combine_layers = 2 asks for the bit-plane form,
+// and when a folded value is negative or NaN.  With quads the row stride becomes the quads'.  Either way the weights of
+// an L = 2..3 raster, now inside the folded layer, become {1, 0, 0}.
 int uam_ensure_quads(uam_ctx* ctx, UamRasterParams* rp, cudaStream_t st) {
     const int W = rp->W, H = rp->H, lay = ctx->geo.layout, tf = ctx->geo.texel_floats;
     const int tiles_x = (W + 3) / 4, tiles_y = (H + 1) / 2;
     const unsigned rs_q = lay ? (unsigned)tiles_x * 8u : (unsigned)W;
     rp->occ_blocks_x = (unsigned)(W + 31) / 32u;
+    const bool want_gather = !ctx->no_sign_pack && !(rp->spc > 0.0 && rp->variant == 3) && W <= ctx->gather_max_w &&
+                             H <= ctx->gather_max_h;
     const bool same_w = tf == 2 || (ctx->comb_w[0] == rp->w0 && ctx->comb_w[1] == rp->w1 && ctx->comb_w[2] == rp->w2);
-    if (!(ctx->comb_valid && same_w)) {
+    if (!(ctx->comb_valid && same_w && ctx->comb_want_gather == want_gather)) {
         UAM_NVTX("uam.raster.build_quads");
-        const size_t n_out = lay ? (size_t)tiles_x * tiles_y * 8 : (size_t)H * W;
-        UAM_CUDA(ctx, cudaDeviceSynchronize());      // kernels on other streams may still read the old quads
-        UAM_TRY(uam_reserve(ctx, &ctx->d_tex_comb, &ctx->tex_comb_bytes, n_out * sizeof(float4)));
+        UAM_CUDA(ctx, cudaDeviceSynchronize());      // kernels on other streams may still read the old layer
         UAM_TRY(uam_reserve(ctx, &ctx->d_occ_bits, &ctx->occ_bits_bytes, (size_t)(uam_occ_words(H, W) + 4) * 4));
-        if (tf == 2) UAM_TRY(lay ? (uam_build_quads_t<2, 1>(ctx, *rp, rs_q, n_out, st)) : (uam_build_quads_t<2, 0>(ctx, *rp, rs_q, n_out, st)));
-        else UAM_TRY(lay ? (uam_build_quads_t<4, 1>(ctx, *rp, rs_q, n_out, st)) : (uam_build_quads_t<4, 0>(ctx, *rp, rs_q, n_out, st)));
-        UAM_CUDA(ctx, cudaStreamSynchronize(st));    // every pipeline stream may use them from now on
+        bool gather = false;
+        if (want_gather) {
+            if (tf == 2) UAM_TRY(lay ? (uam_build_gather_t<2, 1>(ctx, *rp, st, &gather)) : (uam_build_gather_t<2, 0>(ctx, *rp, st, &gather)));
+            else UAM_TRY(lay ? (uam_build_gather_t<4, 1>(ctx, *rp, st, &gather)) : (uam_build_gather_t<4, 0>(ctx, *rp, st, &gather)));
+        }
+        if (!gather) {
+            const size_t n_out = lay ? (size_t)tiles_x * tiles_y * 8 : (size_t)H * W;
+            UAM_TRY(uam_reserve(ctx, &ctx->d_tex_comb, &ctx->tex_comb_bytes, n_out * sizeof(float4)));
+            if (tf == 2) UAM_TRY(lay ? (uam_build_quads_t<2, 1>(ctx, *rp, rs_q, n_out, st)) : (uam_build_quads_t<2, 0>(ctx, *rp, rs_q, n_out, st)));
+            else UAM_TRY(lay ? (uam_build_quads_t<4, 1>(ctx, *rp, rs_q, n_out, st)) : (uam_build_quads_t<4, 0>(ctx, *rp, rs_q, n_out, st)));
+        }
+        UAM_CUDA(ctx, cudaStreamSynchronize(st));    // every pipeline stream may use it from now on
         ctx->comb_valid = true;
+        ctx->comb_gather = gather;
+        ctx->comb_want_gather = want_gather;
         ctx->comb_w[0] = rp->w0; ctx->comb_w[1] = rp->w1; ctx->comb_w[2] = rp->w2;
         ctx->comb_gen += 1;
     }
-    rp->occ_bits = (const unsigned*)ctx->d_occ_bits + 4;
-    rp->combined = ctx->comb_packed ? 2 : 1;
-    rp->row_stride = rs_q;
+    if (ctx->comb_gather) {
+        rp->combined = 3;
+        rp->gather_tex = ctx->gather_tex;
+    } else {
+        rp->occ_bits = (const unsigned*)ctx->d_occ_bits + 4;
+        rp->combined = ctx->comb_packed ? 2 : 1;
+        rp->row_stride = rs_q;
+    }
     if (tf == 4) { rp->w0 = 1.0f; rp->w1 = 0.0f; rp->w2 = 0.0f; }
     return UAM_OK;
 }
 
 // One launch of the scorer or of its gradient on the texels the call samples: the quad texels when
-// uam_raster_precompute made them for it (rp.combined = 1: + occupancy bit-plane, 2: sign-packed), the raster's own
+// uam_raster_precompute made them for it (rp.combined = 1: + occupancy bit-plane, 2: sign-packed, 3: the gather layer), the raster's own
 // otherwise.  slot: which scratch buffer of the ctx the binned pipeline may use (0 = caller-stream calls, 1.. = host
 // pipeline stages).  best (nullable, scorer only): also find the best candidate of the launch, which the binned pipeline
 // fuses into its last kernel and then reports in *best_done.
@@ -2080,6 +2198,7 @@ int uam_raster_dispatch(uam_ctx* ctx, const UamRasterParams& rp, const double* d
         return lay ? uam_raster_launch_t<TF, 1, GRAD>(ctx, tex, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, g, st, slot, best, best_done)
                    : uam_raster_launch_t<TF, 0, GRAD>(ctx, tex, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, g, st, slot, best, best_done);
     };
+    if (rp.combined == 3) return uam_raster_launch_t<16, 0, GRAD>(ctx, nullptr, key, z, B, Wp, rp, d_cost, d_collide, d_nsamp, g, st, slot, best, best_done);
     if (rp.combined == 2) return launch(std::integral_constant<int, 8>());
     if (rp.combined) return launch(std::integral_constant<int, 1>());
     if (ctx->geo.texel_floats == 2) return launch(std::integral_constant<int, 2>());
